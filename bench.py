@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --steps K --warmup W     # the CPU arm (oracle port) on host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...     # one rank per GPU (games shard, no collective)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs (rank 0)
 
 A "step" is one lockstep ply of self-play for every game of the rank: one batched MCTS of
 ``--sims`` iterations over ``--games`` concurrent trees (select -> gather -> net -> expand/backup,
@@ -55,7 +56,14 @@ def parse():
                     help="skip extra.iteration (BASELINE configs[4]: self-play + replay all-gather + training + weight "
                          "broadcast; the only part of the bench that moves bytes over NCCL)")
     ap.add_argument("--iteration-plies", type=int, default=70, help="lockstep plies of extra.iteration (a game lasts ~60)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm's timed steps")
+    return args
 
 
 # ------------------------------------------------------------------------------------------- clocks
@@ -294,6 +302,8 @@ def run_b200(args):
     launches = sp.total_launches() - l0
     sp.mcts.check_errors()
     tstats = sp.mcts.stats()  # d and b of the last search
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, sp, args.dump_outputs)  # before region 2, whose searches replace the trees
 
     # ---- timed region 2: end to end through the host-facing search API (e2e) ---------------------
     # per step: roots in pinned host memory -> H2D -> n_sims-iteration search -> pi + move -> D2H
@@ -457,6 +467,36 @@ def run_b200(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(torch, sp, out_dir, budget=64 << 20):
+    """What a caller of the timed step (BatchedSelfPlay.play_move) has after its last call, one row per game, as float32
+    DIR/<name>.npy: the root statistics of that move's search (root_visits, root_pi = the visit distribution recorded for
+    training, root_q), the move played (action, 64 = pass) and the position the game stands at afterwards (board: +1 the
+    side to move, -1 its opponent, cell = row * 8 + col; player; ply).  Rows beyond `budget` bytes: a fixed, seeded
+    sample of the games, their indices in rows.npy.  counters.npy (float64): the self-play counters of BatchedSelfPlay.stats."""
+    import numpy as np
+
+    B = sp.n_games
+    counts, pi, q = sp.mcts.root_policy()
+    bits = torch.arange(64, device=sp.me.device)
+
+    def cells(b):
+        return ((b[:B, None] >> bits) & 1).float()
+
+    out = {"root_visits": counts[:B].float(), "root_pi": pi[:B], "root_q": q[:B], "action": sp.last_action[:B].float(),
+           "board": cells(sp.me) - cells(sp.opp), "player": sp.player[:B].float(), "ply": sp.ply[:B].float()}
+    out = {k: v.cpu().numpy().astype(np.float32) for k, v in out.items()}
+    row_bytes = sum(v[0].nbytes for v in out.values()) + 8  # + its index in rows.npy
+    room = budget - 4096  # .npy headers and counters.npy
+    if B * row_bytes > room:
+        rows = np.sort(np.random.default_rng(0).choice(B, room // row_bytes, replace=False))
+        out = {k: v[rows] for k, v in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    out["counters"] = sp.counters.cpu().numpy().astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def iteration_block(args, rank, world):

@@ -214,3 +214,34 @@ def test_training_step_reduces_loss_on_selfplay_records():
     for _ in range(30):
         last = train.train_step(model, opt, planes, pi, z)
     assert last["loss"] < first["loss"]
+
+
+def test_bench_dump_outputs_repeat_and_describe_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: two runs with the same arguments write identical arrays; pi is the root visit
+    distribution, and past the sampled opening plies (temp_plies 8 < warm-up 2 + 8 timed steps) the move played is the
+    most visited root action"""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        p = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--games", "256", "--sims", "64", "--steps", "8",
+                            "--warmup", "2", "--no-extra", "--no-iteration", "--no-cpu-baseline", "--scale-games", "0",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 8
+        runs.append({f[:-4]: np.load(out / f) for f in sorted(os.listdir(out))})
+    a, b = runs
+    assert sorted(a) == ["action", "board", "counters", "player", "ply", "root_pi", "root_q", "root_visits"]
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k], equal_nan=True), k
+    n = a["root_visits"]
+    assert n.shape == (256, 65) and a["board"].shape == (256, 64)
+    np.testing.assert_allclose(a["root_pi"], n / n.sum(1, keepdims=True), rtol=1e-6)
+    late = a["ply"] >= 9  # searched at ply 8 or later (a game that ended restarts at ply 0)
+    assert late.sum() > 200 and np.array_equal(a["action"][late], n[late].argmax(1).astype(np.float32))
+    assert (a["board"][:, [27, 28, 35, 36]] != 0).all() and a["counters"][1] == 10 * 256  # centre cells; plies played

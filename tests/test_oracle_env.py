@@ -2,14 +2,13 @@
 
 tests/golden/reversi_env.npz and ttt_env.npz were produced by oracle/make_golden.py running the
 LIVE reference (reversi_board.py / tic_tac_toe_board.py); ttt_env.npz also carries the
-reference's only golden file, tic_tac_toe_data.csv.  When /root/reference is present the oracle is
-additionally checked against the live classes on fresh random boards.
+reference's only golden file, tic_tac_toe_data.csv.  The oracle is checked against them through its batched
+wire-format functions and through its board classes.
 """
 import numpy as np
 import pytest
 
 from oracle import pyoracle as po
-from oracle import ref_shim
 
 
 @pytest.mark.parametrize("size", [4, 6, 8])
@@ -94,36 +93,50 @@ def test_ttt_csv_golden(golden_ttt):
     assert follows >= 180 - 20 - 20  # 20 games: every in-game transition must follow the rule
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="live reference not present")
-def test_oracle_vs_live_reference_random_boards():
-    RB = ref_shim.reversi_board_cls()
+def _bits(mask):
+    return [k for k in range(64) if (int(mask) >> k) & 1]
+
+
+def test_oracle_vs_live_reference_random_boards(golden_env):
+    """The board class (generate_possible_moves, make_move, is_game_over, get_score) against the answers of the
+    reference's ReversiBoard recorded in reversi_env.npz, on a seeded sample of 150 boards per size; the order of
+    generate_possible_moves against the move the reference episodes picked from its list (moves[len(moves) // 2])."""
+    g = golden_env
     rng = np.random.default_rng(123)
     for size in (4, 6, 8):
-        for _ in range(150):
-            pe = rng.uniform(0.05, 0.9)
-            u = rng.random((size, size))
-            g = np.where(u < pe, 0, np.where(rng.random((size, size)) < 0.5, 1, -1))
-            rb = RB(size=size)
-            rb.board = g.copy()
+        me, opp = g[f"s{size}_me"], g[f"s{size}_opp"]
+        succ_idx, bad_idx = g[f"s{size}_succ_idx"], g[f"s{size}_bad_idx"]
+        for i in np.sort(rng.choice(len(me), 150, replace=False)):
             ob = po.OracleReversiBoard(size=size)
-            ob.board = g.copy()
-            for p in (1, -1):
-                assert rb.generate_possible_moves(p) == ob.generate_possible_moves(p)
-                for (r, c) in rb.generate_possible_moves(p)[:4]:
-                    assert np.array_equal(rb.make_move(r, c, p).board, ob.make_move(r, c, p).board)
-            assert rb.is_game_over() == ob.is_game_over()
-            assert rb.get_score() == ob.get_score()
+            ob.board = po.wire_to_grid(me[i], opp[i], size)
+            for p, key in ((1, "mask"), (-1, "mask_opp")):
+                assert [r * 8 + c for r, c in ob.generate_possible_moves(p)] == _bits(g[f"s{size}_{key}"][i])
+            for j in np.flatnonzero(succ_idx == i):
+                a = int(g[f"s{size}_succ_act"][j])
+                nb = ob.make_move(a >> 3, a & 7, 1)
+                assert po.grid_to_wire(nb.board, -1) == (int(g[f"s{size}_succ_me"][j]), int(g[f"s{size}_succ_opp"][j]))
+            for j in np.flatnonzero(bad_idx == i):
+                a = int(g[f"s{size}_bad_act"][j])
+                with pytest.raises(ValueError, match="Invalid move"):
+                    ob.make_move(a >> 3, a & 7, 1)
+            assert ob.is_game_over() == bool(g[f"s{size}_over"][i])
+            assert ob.get_score() == (int(g[f"s{size}_winner"][i]), (int(g[f"s{size}_cnt_me"][i]), int(g[f"s{size}_cnt_opp"][i])))
+        for m, o, a in zip(g[f"ep{size}_me"], g[f"ep{size}_opp"], g[f"ep{size}_action"]):
+            ob = po.OracleReversiBoard(size=size)
+            ob.board = po.wire_to_grid(m, o, size)
+            moves = ob.generate_possible_moves(1)
+            assert (moves[len(moves) // 2] if moves else None) == (None if a == 64 else (a >> 3, a & 7))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="live reference not present")
-def test_ttt_oracle_vs_live_reference():
-    TB = ref_shim.ttt_board_cls()
-    rng = np.random.default_rng(5)
-    for _ in range(300):
-        g = rng.integers(-1, 2, size=(3, 3))
-        rb, ob = TB(g), po.OracleTicTacToeBoard(g)
-        assert rb.is_game_over() == ob.is_game_over()
-        assert rb.generate_possible_moves() == ob.generate_possible_moves()
+def test_ttt_oracle_vs_live_reference(golden_ttt):
+    """The board class (is_game_over, generate_possible_moves) against the answers of the reference's TicTacToeBoard
+    recorded in ttt_env.npz, on all 3^9 grids."""
+    g = golden_ttt
+    for x, o, mask, over, winner in zip(g["x"], g["o"], g["mask"], g["over"], g["winner"]):
+        grid = np.array([1 if (x >> k) & 1 else -1 if (o >> k) & 1 else 0 for k in range(9)], np.int64).reshape(3, 3)
+        ob = po.OracleTicTacToeBoard(grid)
+        assert ob.is_game_over() == (bool(over), None if winner == 2 else int(winner))
+        assert [r * 3 + c for r, c in ob.generate_possible_moves()] == _bits(mask)
 
 
 def test_board_generators_are_seeded():
