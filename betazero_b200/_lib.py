@@ -45,11 +45,26 @@ class BzSelfplayState(C.Structure):
     ]
 
 
+class BzMatchState(C.Structure):
+    """Mirror of ``bz_match_state`` (include/betazero_b200.h)."""
+
+    _fields_ = [
+        ("n_games", C.c_int32), ("board_size", C.c_int32), ("opening_plies", C.c_int32), ("n_trees", C.c_int32),
+        ("seed", C.c_uint64), ("first_pair_id", C.c_int64),
+        ("me", ptr), ("opp", ptr), ("player", ptr), ("ply", ptr), ("result", ptr), ("count_x", ptr), ("count_o", ptr),
+        ("moves", ptr), ("tree_of_game", ptr),
+        ("game_of_tree", ptr), ("root_me", ptr), ("root_opp", ptr), ("pair_net", ptr),
+        ("counters", ptr),
+    ]
+    N_SCALARS = 6
+
+
 # name -> argtypes; every function returns int.  Must list EVERY symbol of include/betazero_b200.h
 # (tests/test_abi.py cross-checks this table against the header).
 _I64, _INT, _U64, _F = C.c_int64, C.c_int, C.c_uint64, C.c_float
 _PP = C.POINTER(BzTreePools)
 _SP = C.POINTER(BzSelfplayState)
+_MP = C.POINTER(BzMatchState)
 SIGNATURES = {
     "bz_abi_version": [],
     "bz_error_string": [_INT],
@@ -69,6 +84,7 @@ SIGNATURES = {
     "bz_mcts_expand_backup": [_PP, ptr, ptr, ptr],
     "bz_mcts_step": [_PP, ptr, ptr, ptr],
     "bz_mcts_search_fused": [_PP, ptr, ptr, _INT, ptr],
+    "bz_mcts_search_fused_two_nets": [_PP, ptr, ptr, ptr, _INT, ptr],
     "bz_mcts_root_policy": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_root_edges": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_best_action": [_PP, ptr, ptr],
@@ -77,6 +93,9 @@ SIGNATURES = {
     "bz_hash_eval": [ptr, ptr, _U64, _INT, ptr, ptr, _I64, ptr],
     "bz_selfplay_init": [_SP, _I64, ptr],
     "bz_selfplay_advance": [_SP, _PP, ptr, ptr],
+    "bz_match_init": [_MP, ptr],
+    "bz_match_layout": [_MP, ptr],
+    "bz_match_advance": [_MP, _PP, ptr],
     "bz_reversi_symmetry": [ptr, ptr, ptr, ptr, ptr, ptr, ptr, _I64, _INT, ptr],
     "bz_record_hash": [ptr, ptr, ptr, ptr, _I64, ptr],
     "bz_philox_u32": [_U64, ptr, ptr, ptr, _I64, ptr],

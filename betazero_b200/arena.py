@@ -5,6 +5,10 @@ reference-compatible board class, in the order of ``ReversiTerminal.play``
 (src/reversi/game_logic/reversi_terminal.py:16-38: moves?, get_move, make_move -- a ValueError
 gives the same player another try --, pass when there is no move, is_game_over, flip player),
 without the prints, and scores with ``get_score`` (reversi_board.py:67-76).
+
+This path plays one game at a time and searches one tree per move.  To measure two nets against each other over
+thousands of games use ``betazero_b200.match.BatchedMatch`` (every game of the match searched in the same launch, the
+same moves as ``MCTSPlayer``s here).
 """
 from __future__ import annotations
 

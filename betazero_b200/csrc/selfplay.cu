@@ -256,6 +256,219 @@ __global__ void __launch_bounds__(256)
     }
 }
 
+// ---- net-versus-net matches ------------------------------------------------------------------------------------------
+// Games 2i and 2i+1 are pair i: same opening, then net A is X in game 2i and O in game 2i+1.  The net to move in game g
+// is its X-net (A for even g) when X is to move, the other net otherwise: 0 = A, 1 = B.
+constexpr int kPairTrees = BZ_MATCH_TREES_PER_PAIR;
+constexpr int kLayoutThreads = 1024;
+
+__device__ __forceinline__ int match_net_to_move(int g, int player) { return (g & 1) ^ (player < 0 ? 1 : 0); }
+
+// the game has ended with (me, opp) seen by `player` to move: result (get_score: more discs wins), counts, counters
+__device__ void match_finish(const bz_match_state &S, int g, uint64_t me, uint64_t opp, int player) {
+    const int cx = __popcll(player > 0 ? me : opp), co = __popcll(player > 0 ? opp : me);
+    const int winner = (cx > co) - (cx < co);  // absolute: +1 X, -1 O, 0 draw
+    BZ_CHECK(g >= 0 && g < S.n_games, 30);  // game row
+    S.result[g] = (int8_t)winner;
+    S.count_x[g] = (uint8_t)cx;
+    S.count_o[g] = (uint8_t)co;
+    const int a_colour = (g & 1) ? -1 : 1;  // net A is X in even games
+    const int r = winner * a_colour;
+    unsigned long long *c = reinterpret_cast<unsigned long long *>(S.counters);
+    atomicAdd(&c[3], 1ull);
+    atomicAdd(&c[r > 0 ? 4 : (r == 0 ? 5 : 6)], 1ull);
+    atomicAdd(&c[7], (unsigned long long)(long long)((cx - co) * a_colour));  // two's complement: signed sum
+}
+
+__device__ __forceinline__ bool game_over(uint64_t me, uint64_t opp, uint64_t cells) {
+    return (legal_mask(me, opp, cells) | legal_mask(opp, me, cells)) == 0;
+}
+
+// a thread per game: start position, the pair's random opening, scoring of games that end inside it
+__global__ void __launch_bounds__(256) match_init_kernel(const bz_match_state S, uint64_t cells) {
+    const int g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= S.n_games) return;
+    uint64_t me = start_me(S.board_size), opp = start_opp(S.board_size);
+    int player = 1, ply = 0;
+    uint8_t *mv = S.moves + (int64_t)g * BZ_MATCH_MAX_PLIES;
+    for (int k = 0; k < BZ_MATCH_MAX_PLIES; ++k) mv[k] = 255u;
+    const uint64_t pair_id = (uint64_t)(S.first_pair_id + g / 2);
+    bool over = game_over(me, opp, cells);
+    while (!over && ply < S.opening_plies && ply < BZ_MATCH_MAX_PLIES) {
+        const uint64_t m = legal_mask(me, opp, cells);
+        unsigned action = 64u;  // pass: the mover has no move (the game is not over, so the opponent has one)
+        if (m) {
+            // the k-th legal move in ascending cell order, k = floor(u32 * moves / 2^32)
+            const uint32_t r = philox_u32(S.seed, pair_id, (uint32_t)ply);
+            int k = (int)(((uint64_t)r * (uint64_t)__popcll(m)) >> 32);
+            uint64_t b = m;
+            for (; k > 0; --k) b &= b - 1;
+            action = (unsigned)(__ffsll((long long)b) - 1);
+        }
+        BZ_CHECK(ply >= 0 && ply < BZ_MATCH_MAX_PLIES, 31);  // move row
+        mv[ply] = (uint8_t)action;
+        apply_legal(me, opp, action);
+        player = -player;
+        ++ply;
+        over = game_over(me, opp, cells);
+    }
+    S.me[g] = me;
+    S.opp[g] = opp;
+    S.player[g] = (int8_t)player;
+    S.ply[g] = ply;
+    S.count_x[g] = 0;
+    S.count_o[g] = 0;
+    S.result[g] = BZ_MATCH_RUNNING;
+    S.tree_of_game[g] = -1;
+    if (over) match_finish(S, g, me, opp, player);
+}
+
+// inclusive block-wide sum of v over kLayoutThreads threads (warp shuffles + one shared row of warp totals)
+__device__ __forceinline__ unsigned block_inclusive_scan(unsigned v, unsigned *warp_tot) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    for (int d = 1; d < 32; d <<= 1) {
+        const unsigned up = __shfl_up_sync(kFull, v, d);
+        if (lane >= d) v += up;
+    }
+    if (lane == 31) warp_tot[w] = v;
+    __syncthreads();
+    if (w == 0) {
+        unsigned t = warp_tot[lane];  // kLayoutThreads / 32 == 32 warps
+        for (int d = 1; d < 32; d <<= 1) {
+            const unsigned up = __shfl_up_sync(kFull, t, d);
+            if (lane >= d) t += up;
+        }
+        warp_tot[lane] = t;
+    }
+    __syncthreads();
+    const unsigned r = v + (w ? warp_tot[w - 1] : 0u);
+    __syncthreads();  // warp_tot is reused by the next scan
+    return r;
+}
+
+// one CTA: stable partition of the live games by the net to move, A's movers first, B's from the next pair boundary
+__global__ void __launch_bounds__(kLayoutThreads) match_layout_kernel(const bz_match_state S) {
+    __shared__ unsigned warp_tot[32];
+    const int tid = threadIdx.x;
+    // pass 1: movers of each net
+    int na = 0, nb = 0;
+    for (int g = tid; g < S.n_games; g += kLayoutThreads) {
+        if (S.result[g] != BZ_MATCH_RUNNING) continue;
+        if (match_net_to_move(g, S.player[g])) ++nb;
+        else ++na;
+    }
+    // both counts in one scan: 16 bits each (n_games < 65536, checked on the host)
+    const unsigned packed_tot = block_inclusive_scan((unsigned)na | ((unsigned)nb << 16), warp_tot);
+    __shared__ unsigned totals;
+    if (tid == kLayoutThreads - 1) totals = packed_tot;
+    __syncthreads();
+    const int tot_a = (int)(totals & 0xFFFFu), tot_b = (int)(totals >> 16);
+    const int a_end = tot_b ? (tot_a + kPairTrees - 1) / kPairTrees * kPairTrees : tot_a;  // B starts on a pair boundary
+    const int n_search = a_end + tot_b;
+    // pass 2: trees of the live games, in game order within each net
+    int base_a = 0, base_b = 0;
+    for (int g0 = 0; g0 < S.n_games; g0 += kLayoutThreads) {
+        const int g = g0 + tid;
+        int net = -1;
+        if (g < S.n_games && S.result[g] == BZ_MATCH_RUNNING) net = match_net_to_move(g, S.player[g]);
+        const unsigned incl = block_inclusive_scan(net == 0 ? 1u : (net == 1 ? 1u << 16 : 0u), warp_tot);
+        if (g < S.n_games) {
+            int t = -1;
+            if (net >= 0) {
+                const unsigned excl = incl - (net == 0 ? 1u : 1u << 16);
+                t = net == 0 ? base_a + (int)(excl & 0xFFFFu) : a_end + base_b + (int)(excl >> 16);
+                BZ_CHECK(t >= 0 && t < n_search && n_search <= S.n_trees, 32);  // tree row
+                S.game_of_tree[t] = g;
+                S.root_me[t] = S.me[g];
+                S.root_opp[t] = S.opp[g];
+            }
+            S.tree_of_game[g] = t;
+        }
+        if (tid == kLayoutThreads - 1) totals = incl;
+        __syncthreads();
+        base_a += (int)(totals & 0xFFFFu);
+        base_b += (int)(totals >> 16);
+        __syncthreads();
+    }
+    // padding between the nets' ranges, and the rows past the searched prefix: empty boards (a finished game, no move
+    // for either side: the search expands nothing there)
+    for (int t = tid; t < S.n_trees; t += kLayoutThreads) {
+        if ((t >= tot_a && t < a_end) || t >= n_search) {
+            S.game_of_tree[t] = -1;
+            S.root_me[t] = 0ull;
+            S.root_opp[t] = 0ull;
+        }
+    }
+    const int n_pairs = (S.n_trees + kPairTrees - 1) / kPairTrees;
+    for (int q = tid; q < n_pairs; q += kLayoutThreads) S.pair_net[q] = (uint8_t)(q * kPairTrees >= a_end ? 1 : 0);
+    if (tid == 0) {
+        S.counters[0] = tot_a + tot_b;
+        S.counters[1] = n_search;
+        S.counters[2] = a_end - tot_a;
+    }
+}
+
+// a warp per game: the most visited root action of the game's tree, record, apply, terminal test, score
+__global__ void __launch_bounds__(kThreads) match_advance_kernel(const bz_match_state S, const bz_tree_pools P, uint64_t cells) {
+    const int g = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (g >= S.n_games) return;
+    const int lane = threadIdx.x & 31;
+    const int t = S.tree_of_game[g];
+    if (t < 0) return;  // ended
+    BZ_CHECK(t < P.n_trees && t < S.n_trees && S.game_of_tree[t] == g, 33);  // tree of the game
+    const uint32_t rmeta = P.root_meta[t];
+    const int n = (int)((rmeta >> BZ_META_N_SHIFT) & 63u);
+    const uint32_t *blk = P.arena + (int64_t)t * P.arena_units * 8 + (int64_t)(rmeta >> BZ_META_OFF_SHIFT) * 8;
+    int Ne = 0, N32 = 0;
+    unsigned act = 127u, act32 = 127u;
+    if (lane < n) {
+        Ne = (int)blk[BZ_NODE_HEADER_WORDS + lane];
+        act = blk[BZ_NODE_HEADER_WORDS + 3 * n + lane] & 127u;
+    }
+    if (n > 32) {
+        N32 = (int)blk[BZ_NODE_HEADER_WORDS + 32];
+        act32 = blk[BZ_NODE_HEADER_WORDS + 3 * n + 32] & 127u;
+    }
+    const int total = __reduce_add_sync(kFull, Ne) + N32;
+    uint64_t me = S.me[g], opp = S.opp[g];
+    const int player = S.player[g], ply = S.ply[g];
+    unsigned action;
+    if (n == 0 || total == 0) {  // a one-iteration search leaves no visits below the root: first legal move, or a pass
+        const uint64_t m = legal_mask(me, opp, cells);
+        action = m ? (unsigned)(__ffsll((long long)m) - 1) : 64u;
+    } else {  // most visited, lowest action id on ties (selfplay_advance_kernel, best_action_kernel)
+        unsigned key = (lane < n && Ne > 0) ? (((unsigned)Ne << 7) | (127u - act)) : 0u;
+        if (n > 32 && N32 > 0) {
+            const unsigned k32 = ((unsigned)N32 << 7) | (127u - act32);
+            key = k32 > key ? k32 : key;
+        }
+        key = __reduce_max_sync(kFull, key);
+        action = 127u - (key & 127u);
+    }
+    if (lane != 0) return;
+    BZ_CHECK(ply >= 0 && ply < BZ_MATCH_MAX_PLIES && action <= 64u, 34);  // move row, action
+    S.moves[(int64_t)g * BZ_MATCH_MAX_PLIES + ply] = (uint8_t)action;
+    apply_legal(me, opp, action);  // the next mover's view
+    S.me[g] = me;
+    S.opp[g] = opp;
+    S.player[g] = (int8_t)(-player);
+    S.ply[g] = ply + 1;
+    S.tree_of_game[g] = -1;  // the next layout assigns a tree again
+    if (game_over(me, opp, cells) || ply + 1 >= BZ_MATCH_MAX_PLIES) match_finish(S, g, me, opp, -player);
+}
+
+int check_match(const bz_match_state *s) {
+    if (!s) return BZ_ERR_ARG;
+    if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
+    if (s->n_games < 0 || (s->n_games & 1) || s->n_games >= (1 << 16) || s->opening_plies < 0 ||
+        s->n_trees < s->n_games + kPairTrees - 1)
+        return BZ_ERR_ARG;
+    if (!s->me || !s->opp || !s->player || !s->ply || !s->result || !s->count_x || !s->count_o || !s->moves ||
+        !s->tree_of_game || !s->game_of_tree || !s->root_me || !s->root_opp || !s->pair_net || !s->counters)
+        return BZ_ERR_ARG;
+    return BZ_OK;
+}
+
 int check_state(const bz_selfplay_state *s) {
     if (!s) return BZ_ERR_ARG;
     if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
@@ -292,6 +505,34 @@ int bz_selfplay_advance(const bz_selfplay_state *st, const bz_tree_pools *pools,
     if (st->n_games == 0) return BZ_OK;
     selfplay_advance_kernel<<<(st->n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
         *st, *pools, action_out, cell_mask(st->board_size));
+    return launch_rc();
+}
+
+int bz_match_init(const bz_match_state *st, bz_stream_t stream) {
+    int rc = check_match(st);
+    if (rc != BZ_OK) return rc;
+    rc = cuda_rc(cudaMemsetAsync(st->counters, 0, 8 * sizeof(int64_t), as_stream(stream)));
+    if (rc != BZ_OK || st->n_games == 0) return rc;
+    match_init_kernel<<<(st->n_games + 255) / 256, 256, 0, as_stream(stream)>>>(*st, cell_mask(st->board_size));
+    return launch_rc();
+}
+
+int bz_match_layout(const bz_match_state *st, bz_stream_t stream) {
+    int rc = check_match(st);
+    if (rc != BZ_OK) return rc;
+    match_layout_kernel<<<1, kLayoutThreads, 0, as_stream(stream)>>>(*st);
+    return launch_rc();
+}
+
+int bz_match_advance(const bz_match_state *st, const bz_tree_pools *pools, bz_stream_t stream) {
+    int rc = check_match(st);
+    if (rc != BZ_OK) return rc;
+    if (!pools || pools->game != BZ_GAME_REVERSI || pools->n_trees != st->n_trees || pools->board_size != st->board_size ||
+        !pools->root_meta || !pools->arena)
+        return BZ_ERR_ARG;
+    if (st->n_games == 0) return BZ_OK;
+    match_advance_kernel<<<(st->n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
+        *st, *pools, cell_mask(st->board_size));
     return launch_rc();
 }
 

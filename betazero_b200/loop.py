@@ -9,11 +9,13 @@ batch order with the same seed, so the replicas stay bit-identical and the broad
 consistency guarantee rather than a necessity; with ``--train-on-rank0`` only rank 0 trains.
 The training loop mirrors the reference's (Adam + cross-entropy, src/tic_tac_toe/SL/train.py:85-113) and, like it,
 saves the model at the end (:204-214) -- here a state_dict checkpoint per iteration (``--checkpoint``), resumable
-(``--resume``).  Prints one JSON line per iteration on rank 0.
+(``--resume``).  Prints one JSON line per iteration on rank 0.  With ``--eval-games N`` rank 0 also plays N games between the
+trained net and the net before training (``match.BatchedMatch``) and adds their score and Elo to the line.
 """
 from __future__ import annotations
 
 import argparse
+import copy
 import json
 import os
 import time
@@ -23,14 +25,14 @@ from types import SimpleNamespace
 import torch
 
 from . import dist as bzd
-from . import mcts, net, selfplay, train
+from . import match, mcts, net, selfplay, train
 
 
 def default_args(**over) -> SimpleNamespace:
     """the command line's defaults as a namespace (for callers that drive iterations from Python: bench.py, tests)"""
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
-                        reuse=False)
+                        reuse=False, eval_games=0)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -44,6 +46,9 @@ class LoopState:
 
     def __init__(self, args, rank: int, world: int):
         self.args, self.rank, self.world = args, rank, world
+        eg = int(getattr(args, "eval_games", 0))
+        if eg < 0 or eg % 2:
+            raise ValueError(f"eval_games must be an even number >= 0 (games are played in pairs); got {eg}")
         self.model = net.make_net(args.net, hidden=args.hidden, seed=args.seed)
         self.master = net.make_net(args.net, hidden=args.hidden, seed=args.seed, dtype=torch.float32)  # fp32 master weights
         self.opt = torch.optim.Adam(self.master.parameters(), lr=args.lr)  # the reference's optimiser family (SL/train.py:87)
@@ -85,6 +90,8 @@ def run_iteration(st: LoopState, it: int) -> dict:
     gather_info = dict(bzd.last_gather)
     ev[2].record()
     n = replay["me"].shape[0]
+    # --eval-games: the net that played this iteration's self-play, to be matched against the trained one
+    snapshot = copy.deepcopy(st.model) if getattr(args, "eval_games", 0) and rank == 0 else None
     losses = []
     if n and (not args.train_on_rank0 or rank == 0):
         g = torch.Generator(device="cuda").manual_seed(args.seed * 1000 + it)
@@ -120,6 +127,13 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["replay_gather"]["algbw_GBps"] = gather_info["gathered_bytes"] / sec / 1e9
         line["replay_gather"]["busbw_GBps"] = gather_info["gathered_bytes"] * (world - 1) / world / sec / 1e9
         line["weight_broadcast_busbw_GBps"] = nbytes / (ms["weight_broadcast"] * 1e-3) / 1e9
+    if snapshot is not None:
+        t_eval = time.perf_counter()
+        r = match.BatchedMatch(st.model, snapshot, args.eval_games, args.sims, n_leaves=args.leaves, board_size=args.size,
+                               seed=args.seed * 1000 + it).play()
+        line["eval"] = {"score": r["score"], "elo": r["elo"], "elo_ci": r["elo_ci"], "wins": r["wins"], "draws": r["draws"],
+                        "losses": r["losses"], "ms": (time.perf_counter() - t_eval) * 1e3}
+        del snapshot
     if caught:
         line["warnings"] = [str(w.message) for w in caught]
     if args.checkpoint and rank == 0:
@@ -163,6 +177,9 @@ def main():
     ap.add_argument("--train-on-rank0", action="store_true")
     ap.add_argument("--reuse", action="store_true", help="keep the searched subtree from move to move (bz_mcts_reroot): --sims "
                                                          "NEW simulations per move on top of the kept ones")
+    ap.add_argument("--eval-games", type=int, default=d.eval_games,
+                    help="rank 0 plays this many games (even) between the trained net and the net before training after "
+                         "every iteration, with --sims / --leaves, and reports them as \"eval\" (0 = off)")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214")
     ap.add_argument("--resume", default=None, help="continue from a checkpoint written by --checkpoint")

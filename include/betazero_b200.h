@@ -240,6 +240,15 @@ int bz_mcts_step(const bz_tree_pools *pools, const void *eval_out, const float *
 int bz_mcts_search_fused(const bz_tree_pools *pools, const void *weight_image_pair, void *eval_out, int n_iterations,
                          bz_stream_t stream);
 
+/* bz_mcts_search_fused with a net per CTA pair: the 56 trees [56 p, 56 p + 56) of the pools are searched with image_a
+ * when pair_net[p] == 0 and with image_b otherwise (net-versus-net matches: each net's movers in whole, pair-aligned tree
+ * ranges).  pair_net: device uint8 [ceil(n_trees / 56)], counted from tree 0 of the pools whatever the chunking (it may
+ * be written by an earlier kernel on the stream, e.g. bz_match_layout).  Same shapes, alignment rules and trees as
+ * bz_mcts_search_fused: a pair's trees are bit-identical to a bz_mcts_search_fused of the same roots with its net.
+ * pair_net == NULL: BZ_ERR_ARG. */
+int bz_mcts_search_fused_two_nets(const bz_tree_pools *pools, const void *image_a, const void *image_b,
+                                  const uint8_t *pair_net, int n_iterations, bz_stream_t stream);
+
 /* Tree reuse across moves (opt-in; the default -- bz_mcts_reset before every search -- is what the goldens pin).
  * After the game of tree t has played action[t] and stands at (new_me[t], new_opp[t]), mover-relative for the side to
  * move there, the tree is re-rooted at the child that action leads to: the child's subtree -- statistics, priors,
@@ -329,6 +338,51 @@ int bz_selfplay_init(const bz_selfplay_state *st, int64_t first_game_id, bz_stre
  * with z and the slot restarts.  action_out (uint8 [n_games]) may be NULL. */
 int bz_selfplay_advance(const bz_selfplay_state *st, const bz_tree_pools *pools, uint8_t *action_out,
                         bz_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Batched net-versus-net matches.  Games 2i and 2i+1 form pair i: both play the same random opening, then net A plays
+ * X in game 2i and net B plays X in game 2i+1.  Every ply: bz_match_layout puts each net's movers into contiguous,
+ * pair-aligned tree ranges, bz_mcts_reset + bz_mcts_search_fused_two_nets search them, bz_match_advance plays the most
+ * visited root action (lowest action on ties) in every live game and scores finished games (get_score,
+ * reversi_board.py:67-76).
+ * ---------------------------------------------------------------------------------------- */
+#define BZ_MATCH_RUNNING 2       /* result of a game that has not ended */
+#define BZ_MATCH_MAX_PLIES 128   /* rows of `moves` per game */
+#define BZ_MATCH_TREES_PER_PAIR 56
+typedef struct bz_match_state {
+    int32_t n_games;       /* even, < 65536 */
+    int32_t board_size;    /* 4, 6, 8 */
+    int32_t opening_plies; /* uniformly random legal moves (Philox keyed by seed, pair id, ply) before the nets play */
+    int32_t n_trees;       /* rows of the tree-ordered arrays: >= n_games + 55 */
+    uint64_t seed;
+    int64_t first_pair_id; /* pair i draws its opening with pair id first_pair_id + i */
+    /* per game [n_games] */
+    uint64_t *me, *opp;    /* current position, mover-relative */
+    int8_t *player;        /* absolute side to move: +1 = X, -1 = O */
+    int32_t *ply;
+    int8_t *result;        /* BZ_MATCH_RUNNING, or the winner: +1 X, -1 O, 0 draw */
+    uint8_t *count_x, *count_o; /* final disc counts (0 while running) */
+    uint8_t *moves;        /* [n_games * BZ_MATCH_MAX_PLIES], action of each ply (64 = pass), 255 after the end */
+    int32_t *tree_of_game; /* tree searched for the game this ply, -1 once it has ended */
+    /* per tree [n_trees] (the layout of the current ply) */
+    int32_t *game_of_tree; /* -1: padding, or past the trees searched this ply */
+    uint64_t *root_me, *root_opp; /* the bz_mcts_reset roots (padding: an empty board, a finished game) */
+    uint8_t *pair_net;     /* [ceil(n_trees / 56)]: 0 net A, 1 net B (bz_mcts_search_fused_two_nets) */
+    /* int64 [8]: 0 live games, 1 trees to search this ply, 2 padding trees this ply (0..2 written by bz_match_layout),
+     * 3 finished games, 4 wins, 5 draws, 6 losses and 7 disc difference, all four from net A's point of view */
+    int64_t *counters;
+} bz_match_state;
+
+/* Every game to the start position, then the opening; games that end inside it are scored.  Zeroes the counters. */
+int bz_match_init(const bz_match_state *st, bz_stream_t stream);
+/* The tree layout of this ply (one CTA): a stable partition of the live games by the net to move -- net A's movers fill
+ * trees [0, nA), padding trees up to the next multiple of 56 follow if net B has movers, then net B's movers.  Writes
+ * tree_of_game, game_of_tree, root_me / root_opp, pair_net and counters 0..2. */
+int bz_match_layout(const bz_match_state *st, bz_stream_t stream);
+/* One ply of every live game from the finished search in `pools` (n_trees == st->n_trees; the trees bz_match_layout
+ * assigned): most visited root action, lowest action id on ties (the first legal move, or a pass, if the root has no
+ * visits); record, apply, terminal test, score. */
+int bz_match_advance(const bz_match_state *st, const bz_tree_pools *pools, bz_stream_t stream);
 
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */
 int bz_philox_u32(uint64_t seed, const int64_t *game_id, const int32_t *ply, uint32_t *out, int64_t n,
