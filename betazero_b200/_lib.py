@@ -59,12 +59,19 @@ class BzMatchState(C.Structure):
     N_SCALARS = 6
 
 
+class BzTournamentState(C.Structure):
+    """Mirror of ``bz_tournament_state`` (include/betazero_b200.h)."""
+
+    _fields_ = [("match", BzMatchState), ("n_entrants", C.c_int32), ("first", ptr), ("second", ptr)]
+
+
 # name -> argtypes; every function returns int.  Must list EVERY symbol of include/betazero_b200.h
 # (tests/test_abi.py cross-checks this table against the header).
 _I64, _INT, _U64, _F = C.c_int64, C.c_int, C.c_uint64, C.c_float
 _PP = C.POINTER(BzTreePools)
 _SP = C.POINTER(BzSelfplayState)
 _MP = C.POINTER(BzMatchState)
+_TP = C.POINTER(BzTournamentState)
 SIGNATURES = {
     "bz_abi_version": [],
     "bz_error_string": [_INT],
@@ -85,6 +92,7 @@ SIGNATURES = {
     "bz_mcts_step": [_PP, ptr, ptr, ptr],
     "bz_mcts_search_fused": [_PP, ptr, ptr, _INT, ptr],
     "bz_mcts_search_fused_two_nets": [_PP, ptr, ptr, ptr, _INT, ptr],
+    "bz_mcts_search_fused_entrants": [_PP, ptr, ptr, _INT, ptr, ptr],
     "bz_mcts_root_policy": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_root_edges": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_best_action": [_PP, ptr, ptr],
@@ -96,6 +104,7 @@ SIGNATURES = {
     "bz_match_init": [_MP, ptr],
     "bz_match_layout": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
+    "bz_tournament_layout": [_TP, ptr],
     "bz_reversi_symmetry": [ptr, ptr, ptr, ptr, ptr, ptr, ptr, _I64, _INT, ptr],
     "bz_record_hash": [ptr, ptr, ptr, ptr, _I64, ptr],
     "bz_philox_u32": [_U64, ptr, ptr, ptr, _I64, ptr],

@@ -457,6 +457,125 @@ __global__ void __launch_bounds__(kThreads) match_advance_kernel(const bz_match_
     if (game_over(me, opp, cells) || ply + 1 >= BZ_MATCH_MAX_PLIES) match_finish(S, g, me, opp, -player);
 }
 
+// ---- tournaments ------------------------------------------------------------------------------------------------------
+// Game pair i is pairing (first[i], second[i]): `first` is X in game 2i and O in game 2i+1.  The entrant to move in game g
+// is its X-entrant when X is to move, the other one otherwise; -1 (BZ_CHECK) for an entrant id >= n_entrants.
+__device__ __forceinline__ int tournament_entrant_to_move(const bz_tournament_state &S, int g) {
+    const int i = g >> 1;
+    const int a = S.first[i], b = S.second[i];
+    const bool x_is_first = (g & 1) == 0, x_to_move = S.match.player[g] > 0;
+    const int e = x_is_first == x_to_move ? a : b;
+    BZ_CHECK(a < S.n_entrants && b < S.n_entrants, 35);  // entrant id
+    return e < S.n_entrants ? e : -1;
+}
+
+// one CTA: stable partition of the live games by the entrant to move -- entrants in id order, games in game order inside
+// an entrant, every non-empty range but the last padded with empty boards to the next multiple of 56 (a CTA pair of
+// the one-launch search loads one entrant).  Ranks: __match_any_sync inside a warp, per-warp counts of each entrant in a
+// 32 x E table scanned over the warps, a running base per entrant across the 1024-game chunks.
+__global__ void __launch_bounds__(kLayoutThreads) tournament_layout_kernel(const bz_tournament_state S) {
+    const bz_match_state &M = S.match;
+    const int E = S.n_entrants;
+    __shared__ unsigned cnt[BZ_MAX_ENTRANTS], start[BZ_MAX_ENTRANTS], pad_end[BZ_MAX_ENTRANTS];
+    __shared__ unsigned wcnt[32][BZ_MAX_ENTRANTS];  // [warp][entrant]: movers, then the warp's first tree in the range
+    __shared__ int n_search_s, last_s;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    if (tid < BZ_MAX_ENTRANTS) cnt[tid] = 0;
+    __syncthreads();
+    // pass 1: movers of each entrant
+    for (int g = tid; g < M.n_games; g += kLayoutThreads) {
+        if (M.result[g] != BZ_MATCH_RUNNING) continue;
+        const int e = tournament_entrant_to_move(S, g);
+        if (e >= 0) atomicAdd(&cnt[e], 1u);
+    }
+    __syncthreads();
+    if (tid == 0) {
+        int last = -1;
+        for (int e = 0; e < E; ++e)
+            if (cnt[e]) last = e;
+        unsigned t = 0;
+        for (int e = 0; e < E; ++e) {
+            start[e] = t;
+            t += cnt[e];
+            if (cnt[e] && e != last) t = (t + kPairTrees - 1) / kPairTrees * kPairTrees;  // the next range: a pair boundary
+            pad_end[e] = t;
+        }
+        n_search_s = (int)t;
+        last_s = last;
+    }
+    __syncthreads();
+    const int n_search = n_search_s, last = last_s;
+    // pass 2: trees of the live games
+    unsigned base_lo = 0, base_hi = 0;  // warp w: trees already given to entrants w and w + 32 by earlier chunks
+    for (int g0 = 0; g0 < M.n_games; g0 += kLayoutThreads) {
+        for (int k = tid; k < 32 * BZ_MAX_ENTRANTS; k += kLayoutThreads) (&wcnt[0][0])[k] = 0;
+        __syncthreads();
+        const int g = g0 + tid;
+        const int e = g < M.n_games && M.result[g] == BZ_MATCH_RUNNING ? tournament_entrant_to_move(S, g) : -1;
+        const unsigned same = __match_any_sync(kFull, e);
+        const unsigned rank = __popc(same & ((1u << lane) - 1u));
+        if (e >= 0 && rank == 0) wcnt[w][e] = __popc(same);
+        __syncthreads();
+        // warp w scans the column of entrants w and w + 32 over the 32 warps (lane = warp)
+        for (int h = 0; h < 2; ++h) {
+            const int ee = w + 32 * h;
+            if (ee >= E) break;
+            const unsigned v = wcnt[lane][ee];
+            unsigned incl = v;
+            for (int d = 1; d < 32; d <<= 1) {
+                const unsigned up = __shfl_up_sync(kFull, incl, d);
+                if (lane >= d) incl += up;
+            }
+            unsigned &base = h ? base_hi : base_lo;
+            wcnt[lane][ee] = start[ee] + base + incl - v;
+            base += __shfl_sync(kFull, incl, 31);
+        }
+        __syncthreads();
+        if (g < M.n_games) {
+            int t = -1;
+            if (e >= 0) {
+                t = (int)(wcnt[w][e] + rank);
+                BZ_CHECK(t >= 0 && t < n_search && n_search <= M.n_trees, 36);  // tree row
+                M.game_of_tree[t] = g;
+                M.root_me[t] = M.me[g];
+                M.root_opp[t] = M.opp[g];
+            }
+            M.tree_of_game[g] = t;
+        }
+        __syncthreads();  // wcnt is cleared for the next chunk
+    }
+    // padding after each range but the last, and the rows past the searched prefix: empty boards (a finished game, no
+    // move for either side: the search expands nothing there)
+    for (int e = 0; e < E; ++e) {
+        const int t = (int)(start[e] + cnt[e]) + tid;
+        if (t < (int)pad_end[e]) {
+            M.game_of_tree[t] = -1;
+            M.root_me[t] = 0ull;
+            M.root_opp[t] = 0ull;
+        }
+    }
+    for (int t = n_search + tid; t < M.n_trees; t += kLayoutThreads) {
+        M.game_of_tree[t] = -1;
+        M.root_me[t] = 0ull;
+        M.root_opp[t] = 0ull;
+    }
+    // the entrant of each CTA pair: the range that holds its first tree; pairs past the prefix: the last entrant
+    const int n_pairs = (M.n_trees + kPairTrees - 1) / kPairTrees;
+    for (int q = tid; q < n_pairs; q += kLayoutThreads) {
+        int owner = last < 0 ? 0 : last;
+        for (int e = 0; e < E; ++e)
+            if (cnt[e] && (unsigned)(q * kPairTrees) >= start[e] && (unsigned)(q * kPairTrees) < pad_end[e]) owner = e;
+        M.pair_net[q] = (uint8_t)owner;
+    }
+    if (tid == 0) {
+        unsigned live = 0;
+        for (int e = 0; e < E; ++e) live += cnt[e];
+        M.counters[0] = live;
+        M.counters[1] = n_search;
+        M.counters[2] = n_search - (int)live;
+    }
+}
+
 int check_match(const bz_match_state *s) {
     if (!s) return BZ_ERR_ARG;
     if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
@@ -465,6 +584,16 @@ int check_match(const bz_match_state *s) {
         return BZ_ERR_ARG;
     if (!s->me || !s->opp || !s->player || !s->ply || !s->result || !s->count_x || !s->count_o || !s->moves ||
         !s->tree_of_game || !s->game_of_tree || !s->root_me || !s->root_opp || !s->pair_net || !s->counters)
+        return BZ_ERR_ARG;
+    return BZ_OK;
+}
+
+int check_tournament(const bz_tournament_state *s) {
+    if (!s) return BZ_ERR_ARG;
+    const int rc = check_match(&s->match);
+    if (rc != BZ_OK) return rc;
+    if (s->n_entrants < 1 || s->n_entrants > BZ_MAX_ENTRANTS || !s->first || !s->second ||
+        s->match.n_trees < s->match.n_games + (kPairTrees - 1) * (s->n_entrants - 1))
         return BZ_ERR_ARG;
     return BZ_OK;
 }
@@ -521,6 +650,13 @@ int bz_match_layout(const bz_match_state *st, bz_stream_t stream) {
     int rc = check_match(st);
     if (rc != BZ_OK) return rc;
     match_layout_kernel<<<1, kLayoutThreads, 0, as_stream(stream)>>>(*st);
+    return launch_rc();
+}
+
+int bz_tournament_layout(const bz_tournament_state *st, bz_stream_t stream) {
+    int rc = check_tournament(st);
+    if (rc != BZ_OK) return rc;
+    tournament_layout_kernel<<<1, kLayoutThreads, 0, as_stream(stream)>>>(*st);
     return launch_rc();
 }
 

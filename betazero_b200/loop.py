@@ -8,8 +8,8 @@ iteration (`dist.gather_replay`, `dist.broadcast_weights`).  Every rank trains o
 batch order with the same seed, so the replicas stay bit-identical and the broadcast is a
 consistency guarantee rather than a necessity; with ``--train-on-rank0`` only rank 0 trains.
 The training loop mirrors the reference's (Adam + cross-entropy, src/tic_tac_toe/SL/train.py:85-113) and, like it,
-saves the model at the end (:204-214) -- here a state_dict checkpoint per iteration (``--checkpoint``), resumable
-(``--resume``).  Prints one JSON line per iteration on rank 0.  With ``--eval-games N`` rank 0 also plays N games between the
+saves the model at the end (:204-214) -- here a state_dict checkpoint per iteration (``--checkpoint``; one file per
+iteration when the path contains ``{iteration}``), resumable (``--resume``).  Prints one JSON line per iteration on rank 0.  With ``--eval-games N`` rank 0 also plays N games between the
 trained net and the net before training (``match.BatchedMatch``) and adds their score and Elo to the line.
 """
 from __future__ import annotations
@@ -71,6 +71,12 @@ class LoopState:
             dst.copy_(src)
         for dst, src in zip(self.model.buffers(), self.master.buffers()):
             dst.copy_(src)
+
+
+def checkpoint_path(pattern: str, it: int) -> str:
+    """``--checkpoint`` with ``{iteration}`` replaced by the iteration number: one file per iteration, kept for a
+    tournament between them (``betazero_b200.tournament``).  Without the placeholder every iteration overwrites one file."""
+    return pattern.replace("{iteration}", str(it))
 
 
 def run_iteration(st: LoopState, it: int) -> dict:
@@ -137,9 +143,10 @@ def run_iteration(st: LoopState, it: int) -> dict:
     if caught:
         line["warnings"] = [str(w.message) for w in caught]
     if args.checkpoint and rank == 0:
-        train.save_checkpoint(args.checkpoint, st.master, st.opt, iteration=it + 1,
+        path = checkpoint_path(args.checkpoint, it)
+        train.save_checkpoint(path, st.master, st.opt, iteration=it + 1,
                               extra={"games_per_gpu": args.games, "sims_per_move": args.sims, "world": world})
-        line["checkpoint"] = args.checkpoint
+        line["checkpoint"] = path
     return line
 
 
@@ -181,7 +188,9 @@ def main():
                     help="rank 0 plays this many games (even) between the trained net and the net before training after "
                          "every iteration, with --sims / --leaves, and reports them as \"eval\" (0 = off)")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
-                                                       "after every iteration (rank 0); SL/train.py:204-214")
+                                                       "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
+                                                       "in the path is replaced by the iteration number, so every "
+                                                       "iteration's checkpoint is kept")
     ap.add_argument("--resume", default=None, help="continue from a checkpoint written by --checkpoint")
     args = ap.parse_args()
     if args.checkpoint:

@@ -249,6 +249,21 @@ int bz_mcts_search_fused(const bz_tree_pools *pools, const void *weight_image_pa
 int bz_mcts_search_fused_two_nets(const bz_tree_pools *pools, const void *image_a, const void *image_b,
                                   const uint8_t *pair_net, int n_iterations, bz_stream_t stream);
 
+/* bz_mcts_search_fused with an entrant table (tournaments: many nets and search budgets in one launch): the 56 trees
+ * [56 p, 56 p + 56) of the pools are searched with images[e] for n_iterations[e] iterations, e = pair_entrant[p].
+ * Generalises bz_mcts_search_fused_two_nets (a two-entry table with equal counts) to per-entrant nets and budgets.
+ * images / n_iterations: host arrays of n_entrants (1 .. BZ_MAX_ENTRANTS) entries, copied into the launch; an image may
+ * appear under several entrants.  pair_entrant: device uint8 [ceil(n_trees / 56)], counted from tree 0 of the pools
+ * whatever the chunking (e.g. written by bz_tournament_layout); an entry >= n_entrants is a bounds-check failure
+ * (BZ_CHECK) and its trees are left as they are, as are the trees of an entrant with 0 iterations.  A pair's trees are
+ * bit-identical to a bz_mcts_search_fused of the same roots with images[e] and n_iterations[e].  The pools' arena must
+ * hold the largest budget.  A launch lasts as long as its largest count: pairs with fewer iterations leave their SMs idle
+ * once they are done.  BZ_ERR_ARG: n_entrants out of range, a NULL image, a negative count, pair_entrant == NULL;
+ * BZ_ERR_UNALIGNED: an image not 16-byte aligned. */
+#define BZ_MAX_ENTRANTS 64
+int bz_mcts_search_fused_entrants(const bz_tree_pools *pools, const void *const *images, const int32_t *n_iterations,
+                                  int n_entrants, const uint8_t *pair_entrant, bz_stream_t stream);
+
 /* Tree reuse across moves (opt-in; the default -- bz_mcts_reset before every search -- is what the goldens pin).
  * After the game of tree t has played action[t] and stands at (new_me[t], new_opp[t]), mover-relative for the side to
  * move there, the tree is re-rooted at the child that action leads to: the child's subtree -- statistics, priors,
@@ -383,6 +398,28 @@ int bz_match_layout(const bz_match_state *st, bz_stream_t stream);
  * assigned): most visited root action, lowest action id on ties (the first legal move, or a pass, if the root has no
  * visits); record, apply, terminal test, score. */
 int bz_match_advance(const bz_match_state *st, const bz_tree_pools *pools, bz_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
+ * the same launches -- in place of a bz_match_* run per pair of nets.  Game pair i is pairing (first[i], second[i]):
+ * both games play the same random opening (pair id first_pair_id + i), then `first` is X in game 2i and O in game 2i+1.
+ * bz_match_init and bz_match_advance run unchanged on &st->match; bz_tournament_layout takes the place of
+ * bz_match_layout, and bz_mcts_search_fused_entrants the place of bz_mcts_search_fused_two_nets.  Counters 3..7 of the
+ * match sum every pairing's results from its `first` entrant's point of view.
+ * ---------------------------------------------------------------------------------------- */
+typedef struct bz_tournament_state {
+    bz_match_state match;  /* games, openings, moves, results; match.pair_net holds ENTRANT ids per 56 trees */
+    int32_t n_entrants;    /* 1 .. BZ_MAX_ENTRANTS */
+    uint8_t *first, *second; /* per game pair [n_games / 2]: `first` is X in game 2i and O in game 2i+1 */
+} bz_tournament_state;
+
+/* The tree layout of this ply (one CTA): a stable partition of the live games by the entrant to move -- entrants in id
+ * order, games in game order inside an entrant, every non-empty range but the last padded with empty boards to the next
+ * multiple of 56.  Writes tree_of_game, game_of_tree, root_me / root_opp, pair_net (entrant ids; pairs past the searched
+ * prefix: the last entrant with movers) and counters 0..2 with bz_match_layout's meanings.  BZ_ERR_ARG: a bad match
+ * state, n_entrants out of range, NULL first / second, match.n_trees < n_games + 55 (n_entrants - 1).  An entrant id
+ * >= n_entrants in first / second is a bounds-check failure (BZ_CHECK); such a game gets no tree. */
+int bz_tournament_layout(const bz_tournament_state *st, bz_stream_t stream);
 
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */
 int bz_philox_u32(uint64_t seed, const int64_t *game_id, const int32_t *ply, uint32_t *out, int64_t n,
