@@ -91,7 +91,6 @@ SIGNATURES = {
     "bz_mcts_expand_backup": [_PP, ptr, ptr, ptr],
     "bz_mcts_step": [_PP, ptr, ptr, ptr],
     "bz_mcts_search_fused": [_PP, ptr, ptr, _INT, ptr],
-    "bz_mcts_search_fused_two_nets": [_PP, ptr, ptr, ptr, _INT, ptr],
     "bz_mcts_search_fused_entrants": [_PP, ptr, ptr, _INT, ptr, ptr],
     "bz_mcts_root_policy": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_root_edges": [_PP, ptr, ptr, ptr, ptr],
@@ -102,7 +101,6 @@ SIGNATURES = {
     "bz_selfplay_init": [_SP, _I64, ptr],
     "bz_selfplay_advance": [_SP, _PP, ptr, ptr],
     "bz_match_init": [_MP, ptr],
-    "bz_match_layout": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
     "bz_tournament_layout": [_TP, ptr],
     "bz_reversi_symmetry": [ptr, ptr, ptr, ptr, ptr, ptr, ptr, _I64, _INT, ptr],
@@ -123,7 +121,7 @@ def lib_path() -> str:
     return _build.LIB
 
 
-ABI_VERSION = 5  # BZ_ABI_VERSION of include/betazero_b200.h this module's structs and signatures mirror
+ABI_VERSION = 6  # BZ_ABI_VERSION of include/betazero_b200.h this module's structs and signatures mirror
 
 
 def load():

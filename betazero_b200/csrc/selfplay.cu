@@ -257,12 +257,9 @@ __global__ void __launch_bounds__(256)
 }
 
 // ---- net-versus-net matches ------------------------------------------------------------------------------------------
-// Games 2i and 2i+1 are pair i: same opening, then net A is X in game 2i and O in game 2i+1.  The net to move in game g
-// is its X-net (A for even g) when X is to move, the other net otherwise: 0 = A, 1 = B.
+// Games 2i and 2i+1 are pair i: same opening, then net A (the pair's first entrant) is X in game 2i and O in game 2i+1.
 constexpr int kPairTrees = BZ_MATCH_TREES_PER_PAIR;
 constexpr int kLayoutThreads = 1024;
-
-__device__ __forceinline__ int match_net_to_move(int g, int player) { return (g & 1) ^ (player < 0 ? 1 : 0); }
 
 // the game has ended with (me, opp) seen by `player` to move: result (get_score: more discs wins), counts, counters
 __device__ void match_finish(const bz_match_state &S, int g, uint64_t me, uint64_t opp, int player) {
@@ -321,91 +318,6 @@ __global__ void __launch_bounds__(256) match_init_kernel(const bz_match_state S,
     S.result[g] = BZ_MATCH_RUNNING;
     S.tree_of_game[g] = -1;
     if (over) match_finish(S, g, me, opp, player);
-}
-
-// inclusive block-wide sum of v over kLayoutThreads threads (warp shuffles + one shared row of warp totals)
-__device__ __forceinline__ unsigned block_inclusive_scan(unsigned v, unsigned *warp_tot) {
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int d = 1; d < 32; d <<= 1) {
-        const unsigned up = __shfl_up_sync(kFull, v, d);
-        if (lane >= d) v += up;
-    }
-    if (lane == 31) warp_tot[w] = v;
-    __syncthreads();
-    if (w == 0) {
-        unsigned t = warp_tot[lane];  // kLayoutThreads / 32 == 32 warps
-        for (int d = 1; d < 32; d <<= 1) {
-            const unsigned up = __shfl_up_sync(kFull, t, d);
-            if (lane >= d) t += up;
-        }
-        warp_tot[lane] = t;
-    }
-    __syncthreads();
-    const unsigned r = v + (w ? warp_tot[w - 1] : 0u);
-    __syncthreads();  // warp_tot is reused by the next scan
-    return r;
-}
-
-// one CTA: stable partition of the live games by the net to move, A's movers first, B's from the next pair boundary
-__global__ void __launch_bounds__(kLayoutThreads) match_layout_kernel(const bz_match_state S) {
-    __shared__ unsigned warp_tot[32];
-    const int tid = threadIdx.x;
-    // pass 1: movers of each net
-    int na = 0, nb = 0;
-    for (int g = tid; g < S.n_games; g += kLayoutThreads) {
-        if (S.result[g] != BZ_MATCH_RUNNING) continue;
-        if (match_net_to_move(g, S.player[g])) ++nb;
-        else ++na;
-    }
-    // both counts in one scan: 16 bits each (n_games < 65536, checked on the host)
-    const unsigned packed_tot = block_inclusive_scan((unsigned)na | ((unsigned)nb << 16), warp_tot);
-    __shared__ unsigned totals;
-    if (tid == kLayoutThreads - 1) totals = packed_tot;
-    __syncthreads();
-    const int tot_a = (int)(totals & 0xFFFFu), tot_b = (int)(totals >> 16);
-    const int a_end = tot_b ? (tot_a + kPairTrees - 1) / kPairTrees * kPairTrees : tot_a;  // B starts on a pair boundary
-    const int n_search = a_end + tot_b;
-    // pass 2: trees of the live games, in game order within each net
-    int base_a = 0, base_b = 0;
-    for (int g0 = 0; g0 < S.n_games; g0 += kLayoutThreads) {
-        const int g = g0 + tid;
-        int net = -1;
-        if (g < S.n_games && S.result[g] == BZ_MATCH_RUNNING) net = match_net_to_move(g, S.player[g]);
-        const unsigned incl = block_inclusive_scan(net == 0 ? 1u : (net == 1 ? 1u << 16 : 0u), warp_tot);
-        if (g < S.n_games) {
-            int t = -1;
-            if (net >= 0) {
-                const unsigned excl = incl - (net == 0 ? 1u : 1u << 16);
-                t = net == 0 ? base_a + (int)(excl & 0xFFFFu) : a_end + base_b + (int)(excl >> 16);
-                BZ_CHECK(t >= 0 && t < n_search && n_search <= S.n_trees, 32);  // tree row
-                S.game_of_tree[t] = g;
-                S.root_me[t] = S.me[g];
-                S.root_opp[t] = S.opp[g];
-            }
-            S.tree_of_game[g] = t;
-        }
-        if (tid == kLayoutThreads - 1) totals = incl;
-        __syncthreads();
-        base_a += (int)(totals & 0xFFFFu);
-        base_b += (int)(totals >> 16);
-        __syncthreads();
-    }
-    // padding between the nets' ranges, and the rows past the searched prefix: empty boards (a finished game, no move
-    // for either side: the search expands nothing there)
-    for (int t = tid; t < S.n_trees; t += kLayoutThreads) {
-        if ((t >= tot_a && t < a_end) || t >= n_search) {
-            S.game_of_tree[t] = -1;
-            S.root_me[t] = 0ull;
-            S.root_opp[t] = 0ull;
-        }
-    }
-    const int n_pairs = (S.n_trees + kPairTrees - 1) / kPairTrees;
-    for (int q = tid; q < n_pairs; q += kLayoutThreads) S.pair_net[q] = (uint8_t)(q * kPairTrees >= a_end ? 1 : 0);
-    if (tid == 0) {
-        S.counters[0] = tot_a + tot_b;
-        S.counters[1] = n_search;
-        S.counters[2] = a_end - tot_a;
-    }
 }
 
 // a warp per game: the most visited root action of the game's tree, record, apply, terminal test, score
@@ -643,13 +555,6 @@ int bz_match_init(const bz_match_state *st, bz_stream_t stream) {
     rc = cuda_rc(cudaMemsetAsync(st->counters, 0, 8 * sizeof(int64_t), as_stream(stream)));
     if (rc != BZ_OK || st->n_games == 0) return rc;
     match_init_kernel<<<(st->n_games + 255) / 256, 256, 0, as_stream(stream)>>>(*st, cell_mask(st->board_size));
-    return launch_rc();
-}
-
-int bz_match_layout(const bz_match_state *st, bz_stream_t stream) {
-    int rc = check_match(st);
-    if (rc != BZ_OK) return rc;
-    match_layout_kernel<<<1, kLayoutThreads, 0, as_stream(stream)>>>(*st);
     return launch_rc();
 }
 

@@ -29,12 +29,49 @@ import torch
 
 from . import _lib
 from ._lib import BzTournamentState, BzTreePools
-from .match import MAX_PLIES, RUNNING, TREES_PER_PAIR, check_net, elo_summary
 from .mcts import PRIOR_LOGITS_BF16, TreePools
 
+TREES_PER_PAIR = 56       # a CTA pair of the one-launch kernel: the unit that loads one net
+MAX_PLIES = 128           # BZ_MATCH_MAX_PLIES
+RUNNING = 2               # BZ_MATCH_RUNNING
 MAX_ENTRANTS = 64         # BZ_MAX_ENTRANTS
 LAUNCH_TREES = 148 * 28   # trees of one launch of the one-launch search; more are searched in chunks
+Z95 = 1.959963984540054   # two-sided 95 % normal quantile
 _C = math.log(10.0) / 400.0
+
+
+def elo(score: float) -> float:
+    """Elo difference of an expected score in [0, 1] (logistic model); +-inf at 1 and 0."""
+    if score >= 1.0:
+        return math.inf
+    if score <= 0.0:
+        return -math.inf
+    return -400.0 * math.log10(1.0 / score - 1.0)
+
+
+def elo_summary(pair_scores) -> dict:
+    """Score, Elo and a 95 % interval from the mean score of each pair (its two games' mean: 0, 1/4, 1/2, 3/4 or 1).
+    The interval is the normal interval of the mean pair score (standard error with n - 1), mapped through ``elo``."""
+    xs = [float(x) for x in pair_scores]
+    n = len(xs)
+    if n == 0:
+        return {"score": math.nan, "elo": math.nan, "elo_ci": [math.nan, math.nan], "score_se": math.nan, "pairs": 0}
+    mean = sum(xs) / n
+    se = math.sqrt(sum((x - mean) ** 2 for x in xs) / (n - 1) / n) if n > 1 else 0.0
+    lo, hi = mean - Z95 * se, mean + Z95 * se
+    return {"score": mean, "elo": elo(mean), "elo_ci": [elo(lo), elo(hi)], "score_se": se, "pairs": n}
+
+
+def check_net(net) -> None:
+    """The one-launch kernel covers the bf16 128-256-256-256-(65+1) MLP only; there is no other path."""
+    from .net import PolicyValueMLP
+
+    ok = (isinstance(net, PolicyValueMLP) and net.fc1.in_features == 128 and net.fc1.out_features == 256
+          and net.fc2.out_features == 256 and net.fc3.out_features == 256 and net.n_actions == 65 and net.raw_width == 72
+          and net.fc1.weight.dtype == torch.bfloat16 and net.fc1.weight.is_cuda)
+    if not ok:
+        raise ValueError("matches and tournaments play the bf16 128-256-256-256-(65+1) Reversi MLP on a GPU only "
+                         "(the net the one-launch search runs)")
 
 
 def _components(n: int, edges) -> int:
@@ -124,10 +161,10 @@ def fit_ratings(n_entrants: int, pairings, pair_scores, max_iter: int = 100) -> 
 class Tournament:
     """Every pairing of ``entrants`` -- a list of ``(net, n_sims)``; one net may appear with several budgets and then
     shares its weight image -- for ``games_per_pairing`` (even) games, all searched at once.  ``play()`` returns the
-    result."""
+    result.  Game pair i draws its opening with pair id ``first_pair_id + i``."""
 
     def __init__(self, entrants, games_per_pairing: int, n_leaves: int = 4, board_size: int = 8, c_puct: float = 1.25,
-                 opening_plies: int = 4, seed: int = 0, pairings=None, device="cuda"):
+                 opening_plies: int = 4, seed: int = 0, pairings=None, first_pair_id: int = 0, device="cuda"):
         entrants = list(entrants)
         E = len(entrants)
         if not 2 <= E <= MAX_ENTRANTS:
@@ -191,7 +228,7 @@ class Tournament:
         s = BzTournamentState()
         m = s.match
         m.n_games, m.board_size, m.opening_plies, m.n_trees = G, self.board_size, int(opening_plies), T
-        m.seed, m.first_pair_id = int(seed), 0
+        m.seed, m.first_pair_id = int(seed), int(first_pair_id)
         for name, _ in m._fields_[m.N_SCALARS:]:
             setattr(m, name, getattr(self, name).data_ptr())
         s.n_entrants, s.first, s.second = E, self.first.data_ptr(), self.second.data_ptr()
@@ -207,6 +244,9 @@ class Tournament:
 
     # -- the steps of a ply -------------------------------------------------------------------------------------------
     def init(self) -> None:
+        """the openings; the entrants' weight images (``prepare_inference``) must exist"""
+        for k, (n, _) in enumerate(self.entrants):
+            self._images[k] = n._image_pair.data_ptr()
         _lib.check(self._L.bz_match_init(self._mref, _lib.stream_ptr()), "bz_match_init")
 
     def layout(self) -> tuple[int, int]:
@@ -234,8 +274,6 @@ class Tournament:
             n.prepare_inference()  # the weight images of the current parameters (in place)
             if getattr(n, "_image_pair", None) is None:
                 raise ValueError("the net has no weight image for the one-launch kernel")
-        for k, (n, _) in enumerate(self.entrants):
-            self._images[k] = n._image_pair.data_ptr()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         self.init()

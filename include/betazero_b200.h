@@ -32,7 +32,7 @@ extern "C" {
 #define BZ_OK 0
 #define BZ_ERR_ARG (-1)
 #define BZ_ERR_UNALIGNED (-2)
-#define BZ_ABI_VERSION 5
+#define BZ_ABI_VERSION 6
 
 #define BZ_REVERSI_ACTIONS 65
 #define BZ_TTT_ACTIONS 9
@@ -240,18 +240,8 @@ int bz_mcts_step(const bz_tree_pools *pools, const void *eval_out, const float *
 int bz_mcts_search_fused(const bz_tree_pools *pools, const void *weight_image_pair, void *eval_out, int n_iterations,
                          bz_stream_t stream);
 
-/* bz_mcts_search_fused with a net per CTA pair: the 56 trees [56 p, 56 p + 56) of the pools are searched with image_a
- * when pair_net[p] == 0 and with image_b otherwise (net-versus-net matches: each net's movers in whole, pair-aligned tree
- * ranges).  pair_net: device uint8 [ceil(n_trees / 56)], counted from tree 0 of the pools whatever the chunking (it may
- * be written by an earlier kernel on the stream, e.g. bz_match_layout).  Same shapes, alignment rules and trees as
- * bz_mcts_search_fused: a pair's trees are bit-identical to a bz_mcts_search_fused of the same roots with its net.
- * pair_net == NULL: BZ_ERR_ARG. */
-int bz_mcts_search_fused_two_nets(const bz_tree_pools *pools, const void *image_a, const void *image_b,
-                                  const uint8_t *pair_net, int n_iterations, bz_stream_t stream);
-
 /* bz_mcts_search_fused with an entrant table (tournaments: many nets and search budgets in one launch): the 56 trees
  * [56 p, 56 p + 56) of the pools are searched with images[e] for n_iterations[e] iterations, e = pair_entrant[p].
- * Generalises bz_mcts_search_fused_two_nets (a two-entry table with equal counts) to per-entrant nets and budgets.
  * images / n_iterations: host arrays of n_entrants (1 .. BZ_MAX_ENTRANTS) entries, copied into the launch; an image may
  * appear under several entrants.  pair_entrant: device uint8 [ceil(n_trees / 56)], counted from tree 0 of the pools
  * whatever the chunking (e.g. written by bz_tournament_layout); an entry >= n_entrants is a bounds-check failure
@@ -355,11 +345,13 @@ int bz_selfplay_advance(const bz_selfplay_state *st, const bz_tree_pools *pools,
                         bz_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
- * Batched net-versus-net matches.  Games 2i and 2i+1 form pair i: both play the same random opening, then net A plays
- * X in game 2i and net B plays X in game 2i+1.  Every ply: bz_match_layout puts each net's movers into contiguous,
- * pair-aligned tree ranges, bz_mcts_reset + bz_mcts_search_fused_two_nets search them, bz_match_advance plays the most
+ * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
+ * the same launches; a net-versus-net match is the tournament of two entrants and the one pairing (0, 1).  Game pair i
+ * is pairing (first[i], second[i]): both games play the same random opening (pair id first_pair_id + i), then `first`
+ * is X in game 2i and O in game 2i+1.  Every ply: bz_tournament_layout puts each entrant's movers into contiguous,
+ * pair-aligned tree ranges, bz_mcts_reset + bz_mcts_search_fused_entrants search them, bz_match_advance plays the most
  * visited root action (lowest action on ties) in every live game and scores finished games (get_score,
- * reversi_board.py:67-76).
+ * reversi_board.py:67-76).  bz_match_init and bz_match_advance take the tournament state's `match`.
  * ---------------------------------------------------------------------------------------- */
 #define BZ_MATCH_RUNNING 2       /* result of a game that has not ended */
 #define BZ_MATCH_MAX_PLIES 128   /* rows of `moves` per game */
@@ -382,33 +374,22 @@ typedef struct bz_match_state {
     /* per tree [n_trees] (the layout of the current ply) */
     int32_t *game_of_tree; /* -1: padding, or past the trees searched this ply */
     uint64_t *root_me, *root_opp; /* the bz_mcts_reset roots (padding: an empty board, a finished game) */
-    uint8_t *pair_net;     /* [ceil(n_trees / 56)]: 0 net A, 1 net B (bz_mcts_search_fused_two_nets) */
-    /* int64 [8]: 0 live games, 1 trees to search this ply, 2 padding trees this ply (0..2 written by bz_match_layout),
-     * 3 finished games, 4 wins, 5 draws, 6 losses and 7 disc difference, all four from net A's point of view */
+    uint8_t *pair_net;     /* [ceil(n_trees / 56)]: entrant ids, the pair_entrant of bz_mcts_search_fused_entrants */
+    /* int64 [8]: 0 live games, 1 trees to search this ply, 2 padding trees this ply (0..2 written by
+     * bz_tournament_layout), 3 finished games, 4 wins, 5 draws, 6 losses and 7 disc difference, all four summed over
+     * every pairing from its `first` entrant's point of view */
     int64_t *counters;
 } bz_match_state;
 
 /* Every game to the start position, then the opening; games that end inside it are scored.  Zeroes the counters. */
 int bz_match_init(const bz_match_state *st, bz_stream_t stream);
-/* The tree layout of this ply (one CTA): a stable partition of the live games by the net to move -- net A's movers fill
- * trees [0, nA), padding trees up to the next multiple of 56 follow if net B has movers, then net B's movers.  Writes
- * tree_of_game, game_of_tree, root_me / root_opp, pair_net and counters 0..2. */
-int bz_match_layout(const bz_match_state *st, bz_stream_t stream);
-/* One ply of every live game from the finished search in `pools` (n_trees == st->n_trees; the trees bz_match_layout
+/* One ply of every live game from the finished search in `pools` (n_trees == st->n_trees; the trees bz_tournament_layout
  * assigned): most visited root action, lowest action id on ties (the first legal move, or a pass, if the root has no
  * visits); record, apply, terminal test, score. */
 int bz_match_advance(const bz_match_state *st, const bz_tree_pools *pools, bz_stream_t stream);
 
-/* ------------------------------------------------------------------------------------------
- * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
- * the same launches -- in place of a bz_match_* run per pair of nets.  Game pair i is pairing (first[i], second[i]):
- * both games play the same random opening (pair id first_pair_id + i), then `first` is X in game 2i and O in game 2i+1.
- * bz_match_init and bz_match_advance run unchanged on &st->match; bz_tournament_layout takes the place of
- * bz_match_layout, and bz_mcts_search_fused_entrants the place of bz_mcts_search_fused_two_nets.  Counters 3..7 of the
- * match sum every pairing's results from its `first` entrant's point of view.
- * ---------------------------------------------------------------------------------------- */
 typedef struct bz_tournament_state {
-    bz_match_state match;  /* games, openings, moves, results; match.pair_net holds ENTRANT ids per 56 trees */
+    bz_match_state match;  /* games, openings, moves, results, the layout of the current ply */
     int32_t n_entrants;    /* 1 .. BZ_MAX_ENTRANTS */
     uint8_t *first, *second; /* per game pair [n_games / 2]: `first` is X in game 2i and O in game 2i+1 */
 } bz_tournament_state;
@@ -416,9 +397,9 @@ typedef struct bz_tournament_state {
 /* The tree layout of this ply (one CTA): a stable partition of the live games by the entrant to move -- entrants in id
  * order, games in game order inside an entrant, every non-empty range but the last padded with empty boards to the next
  * multiple of 56.  Writes tree_of_game, game_of_tree, root_me / root_opp, pair_net (entrant ids; pairs past the searched
- * prefix: the last entrant with movers) and counters 0..2 with bz_match_layout's meanings.  BZ_ERR_ARG: a bad match
- * state, n_entrants out of range, NULL first / second, match.n_trees < n_games + 55 (n_entrants - 1).  An entrant id
- * >= n_entrants in first / second is a bounds-check failure (BZ_CHECK); such a game gets no tree. */
+ * prefix: the last entrant with movers) and counters 0..2.  BZ_ERR_ARG: a bad match state, n_entrants out of range, NULL
+ * first / second, match.n_trees < n_games + 55 (n_entrants - 1).  An entrant id >= n_entrants in first / second is a
+ * bounds-check failure (BZ_CHECK); such a game gets no tree. */
 int bz_tournament_layout(const bz_tournament_state *st, bz_stream_t stream);
 
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */

@@ -79,7 +79,6 @@ def main():
                "ply_ms": e[0].elapsed_time(e[3]), "ply_wall_ms": wall * 1e3,
                "search_ms": e[1].elapsed_time(e[2]), "layout_ms": e[0].elapsed_time(e[1]), "advance_ms": e[2].elapsed_time(e[3])}
         m.plies += 1
-        m.sims += (n_search - pad) * S
         if m.plies <= 20:  # the same process, alternating: a self-play ply of G trees
             e[0].record()
             sp.play_move()

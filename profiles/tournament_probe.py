@@ -4,11 +4,11 @@ padding trees every ply fits one launch (3752 + 385 <= 4144 trees).
 
     python profiles/tournament_probe.py [--out FILE]
 
-Compared in the same process: a BatchedMatch of 3752 games at 800 simulations (the same tree count, one net pair), and
-the same tournament with every budget at 800, which isolates what mixed budgets cost: a launch lasts as long as its
-largest budget, so the pairs of 200-simulation entrants idle for the rest of it.  Every configuration runs once as a
-warm-up, then --repeats times; wall times are host clocks around work that ends in a device synchronise.  The GPU name
-and power limit are read in the same run and stored with the numbers.
+Compared in the same process: a BatchedMatch of 3752 games at 800 simulations (the same tree count: a tournament of two
+entrants, one net pair), and the same tournament with every budget at 800, which isolates what mixed budgets cost: a
+launch lasts as long as its largest budget, so the pairs of 200-simulation entrants idle for the rest of it.  Every
+configuration runs once as a warm-up, then --repeats times; wall times are host clocks around work that ends in a device
+synchronise.  The GPU name and power limit are read in the same run and stored with the numbers.
 """
 from __future__ import annotations
 

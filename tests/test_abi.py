@@ -26,7 +26,7 @@ def test_header_symbols_are_exported_and_bound():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in the header but not exported"
     assert sorted(_lib.SIGNATURES) == names, "ctypes table and header disagree"
-    assert lib.bz_abi_version() == _lib.ABI_VERSION == 5
+    assert lib.bz_abi_version() == _lib.ABI_VERSION == 6
     assert lib.bz_error_string(0) == b"ok" and b"argument" in lib.bz_error_string(-1)
 
 

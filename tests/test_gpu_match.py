@@ -1,6 +1,6 @@
-"""Batched net-versus-net matches: bz_mcts_search_fused_two_nets builds, for every CTA pair, exactly the trees the
-single-net one-launch search builds with that pair's net; BatchedMatch plays the games MCTSPlayer plays one at a time,
-independently of the batch around them, with a consistent per-ply tree layout."""
+"""Batched net-versus-net matches: bz_mcts_search_fused_entrants with two nets of equal budgets builds, for every CTA
+pair, exactly the trees the single-net one-launch search builds with that pair's net; BatchedMatch plays the games
+MCTSPlayer plays one at a time, independently of the batch around them, with a consistent per-ply tree layout."""
 import ctypes
 
 import numpy as np
@@ -22,7 +22,8 @@ def _roots(B, seed, size=8):
 
 
 def _search(model, me, opp, n_sims, K, size=8, two=None):
-    """one-launch search of the roots with `model`; two = (model_b, pair_net): bz_mcts_search_fused_two_nets"""
+    """one-launch search of the roots with `model`; two = (model_b, pair_net): bz_mcts_search_fused_entrants with the
+    entrants (model, n_sims) and (model_b, n_sims)"""
     from betazero_b200 import _lib, mcts
 
     B = me.numel()
@@ -35,9 +36,10 @@ def _search(model, me, opp, n_sims, K, size=8, two=None):
     else:
         model_b, pair_net = two
         model_b.prepare_inference()
-        L = _lib.load()
-        _lib.check(L.bz_mcts_search_fused_two_nets(s.pools._ref, _lib.dptr(model._image_pair), _lib.dptr(model_b._image_pair),
-                                                   _lib.dptr(pair_net), n_sims // K, _lib.stream_ptr()), "two_nets")
+        images = (ctypes.c_void_p * 2)(model._image_pair.data_ptr(), model_b._image_pair.data_ptr())
+        iters = (ctypes.c_int32 * 2)(n_sims // K, n_sims // K)
+        _lib.check(_lib.load().bz_mcts_search_fused_entrants(s.pools._ref, images, iters, 2, _lib.dptr(pair_net),
+                                                             _lib.stream_ptr()), "entrants")
     torch.cuda.synchronize()
     s.check_errors()
     return s
@@ -57,7 +59,7 @@ def _tree_state(s):
 
 @pytest.mark.parametrize("K", [1, 2, 4])
 @pytest.mark.parametrize("B", [56, 57, 300, 4144, 4145, 9000])  # above 4144 trees: chunks, one launch each
-def test_two_net_search_equals_the_single_net_searches(B, K):
+def test_two_entrant_search_equals_the_single_net_searches(B, K):
     from betazero_b200 import net
 
     a, b = net.make_net("mlp", seed=10 + B + K), net.make_net("mlp", seed=20 + B + K)
@@ -79,7 +81,7 @@ def test_two_net_search_equals_the_single_net_searches(B, K):
 
 
 @pytest.mark.parametrize("size", [6, 4])
-def test_two_net_search_small_boards(size):
+def test_two_entrant_search_small_boards(size):
     from betazero_b200 import net
 
     a, b = net.make_net("mlp", seed=31), net.make_net("mlp", seed=32)
@@ -90,20 +92,6 @@ def test_two_net_search_small_boards(size):
     got = _tree_state(_search(a, me, opp, 32, 4, size, two=(b, pair_net.cuda())))
     for x, ya, yb in zip(got, ref_a, ref_b):
         assert torch.equal(x, torch.where(sel_b.view(-1, *([1] * (x.dim() - 1))), yb, ya))
-
-
-def test_two_net_search_refuses_a_missing_pair_net():
-    from betazero_b200 import _lib, mcts, net
-
-    model = net.make_net("mlp", seed=1)
-    model.prepare_inference()
-    p = mcts.TreePools(64, 8, n_leaves=4, prior_mode=mcts.PRIOR_LOGITS_BF16, eval_stride=72)
-    L = _lib.load()
-    img = _lib.dptr(model._image_pair)
-    assert L.bz_mcts_search_fused_two_nets(p._ref, img, img, None, 2, _lib.stream_ptr()) == -1  # BZ_ERR_ARG
-    pn = torch.zeros(2, dtype=torch.uint8, device="cuda")
-    odd = ctypes.c_void_p(model._image_pair.data_ptr() + 8)
-    assert L.bz_mcts_search_fused_two_nets(p._ref, img, odd, _lib.dptr(pn), 2, _lib.stream_ptr()) == -2  # BZ_ERR_UNALIGNED
 
 
 def _match(a, b, n_games, n_sims, K=4, size=8, opening=4, seed=0):

@@ -212,8 +212,6 @@ def test_layout_invariants_every_ply():
     t = _tournament(entrants, 40, K=4, size=6, opening=3, seed=4, pairings=[(0, 1), (2, 0), (1, 3), (4, 3), (2, 4)])
     for n in (a, b):
         n.prepare_inference()
-    for k, (n, _) in enumerate(entrants):
-        t._images[k] = n._image_pair.data_ptr()
     G = t.n_games
     t.init()
     g_idx = torch.arange(G)
