@@ -139,13 +139,13 @@ class PolicyValueMLP(nn.Module):
                 raise RuntimeError(f"unknown / unavailable MLP kernel {fused!r}")
             if out is None:
                 out = torch.empty((B, self.raw_width), dtype=torch.bfloat16, device=planes.device)
-            x = planes.reshape(B, -1)
+            x = planes.flatten(1)  # [B, 128]; reshape(B, -1) cannot size an empty batch
             L = _lib.load()
             fn, name = ((L.bz_mlp_forward_pair2, "bz_mlp_forward_pair2") if fused == "pair2"
                         else (L.bz_mlp_forward_pair, "bz_mlp_forward_pair"))
             _lib.check(fn(_lib.dptr(x), _lib.dptr(self._image_pair), _lib.dptr(out), B, _lib.stream_ptr()), name)
             return out
-        x = planes.reshape(B, -1).to(self.fc1.weight.dtype)
+        x = planes.flatten(1).to(self.fc1.weight.dtype)
         x = torch._addmm_activation(self.fc1.bias, x, self._w[0])
         x = torch._addmm_activation(self.fc2.bias, x, self._w[1])
         x = torch._addmm_activation(self.fc3.bias, x, self._w[2])
