@@ -16,7 +16,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbetazero_b200.so")
-SOURCES = ("env.cu", "mcts.cu", "selfplay.cu", "mlp_pair.cu", "mlp_pair2.cu")
+SOURCES = ("env.cu", "mcts.cu", "selfplay.cu", "mlp_pair.cu", "mlp_pair2.cu", "minimax.cu")
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--fmad=false",  # PUCT arithmetic must round op by op (bit-exact visit counts); intrinsics enforce it too

@@ -90,6 +90,24 @@ static __device__ int g_bz_check[4];  // [0] first failing check's code, [1] blo
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// ---- Philox4x32-10 (counter-based RNG; results depend only on (seed, game id, ply)) -------------
+// self-play move sampling and match openings (selfplay.cu), the minimax players' random move (minimax.cu)
+__host__ __device__ inline uint32_t philox_u32(uint64_t seed, uint64_t game_id, uint32_t ply) {
+    uint32_t c0 = (uint32_t)game_id, c1 = (uint32_t)(game_id >> 32), c2 = ply, c3 = 0;
+    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+    for (int r = 0; r < 10; ++r) {
+        const uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
+        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
+        c1 = (uint32_t)p1;
+        c3 = (uint32_t)p0;
+        c0 = n0;
+        c2 = n2;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    return c0;
+}
+
 // streaming (read-once / write-once) 128-bit global accesses that do not allocate in L1
 __device__ __forceinline__ ulonglong2 ld_stream_u64x2(const uint64_t *p) {
     ulonglong2 r;

@@ -5,6 +5,7 @@
 // them to the replay buffer and restarts the slot.  One warp per game slot == per tree.
 #include "bitboard.cuh"
 #include "common.cuh"
+#include "minimax.cuh"
 
 namespace bz {
 namespace {
@@ -13,23 +14,6 @@ constexpr unsigned kFull = 0xFFFFFFFFu;
 constexpr int kWarpsPerCta = 4;
 constexpr int kThreads = kWarpsPerCta * 32;
 constexpr int A = BZ_REVERSI_ACTIONS;
-
-// ---- Philox4x32-10 (counter-based RNG; results depend only on (seed, game id, ply)) -------------
-__host__ __device__ inline uint32_t philox_u32(uint64_t seed, uint64_t game_id, uint32_t ply) {
-    uint32_t c0 = (uint32_t)game_id, c1 = (uint32_t)(game_id >> 32), c2 = ply, c3 = 0;
-    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-    for (int r = 0; r < 10; ++r) {
-        const uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
-        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
-        c1 = (uint32_t)p1;
-        c3 = (uint32_t)p0;
-        c0 = n0;
-        c2 = n2;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-    return c0;
-}
 
 __global__ void __launch_bounds__(256) selfplay_init_kernel(const bz_selfplay_state S, int64_t first_game_id) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -321,41 +305,50 @@ __global__ void __launch_bounds__(256) match_init_kernel(const bz_match_state S,
 }
 
 // a warp per game: the most visited root action of the game's tree, record, apply, terminal test, score
-__global__ void __launch_bounds__(kThreads) match_advance_kernel(const bz_match_state S, const bz_tree_pools P, uint64_t cells) {
+// Tournaments with minimax entrants: the game of a tree whose CTA pair's entrant is in `minimax_entrants` (a bit per
+// entrant) plays minimax_action[t] instead.
+__global__ void __launch_bounds__(kThreads) match_advance_kernel(const bz_match_state S, const bz_tree_pools P, uint64_t cells,
+                                                                 uint64_t minimax_entrants, const uint8_t *minimax_action) {
     const int g = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
     if (g >= S.n_games) return;
     const int lane = threadIdx.x & 31;
     const int t = S.tree_of_game[g];
     if (t < 0) return;  // ended
-    BZ_CHECK(t < P.n_trees && t < S.n_trees && S.game_of_tree[t] == g, 33);  // tree of the game
-    const uint32_t rmeta = P.root_meta[t];
-    const int n = (int)((rmeta >> BZ_META_N_SHIFT) & 63u);
-    const uint32_t *blk = P.arena + (int64_t)t * P.arena_units * 8 + (int64_t)(rmeta >> BZ_META_OFF_SHIFT) * 8;
-    int Ne = 0, N32 = 0;
-    unsigned act = 127u, act32 = 127u;
-    if (lane < n) {
-        Ne = (int)blk[BZ_NODE_HEADER_WORDS + lane];
-        act = blk[BZ_NODE_HEADER_WORDS + 3 * n + lane] & 127u;
-    }
-    if (n > 32) {
-        N32 = (int)blk[BZ_NODE_HEADER_WORDS + 32];
-        act32 = blk[BZ_NODE_HEADER_WORDS + 3 * n + 32] & 127u;
-    }
-    const int total = __reduce_add_sync(kFull, Ne) + N32;
+    BZ_CHECK(t < S.n_trees && S.game_of_tree[t] == g, 33);  // tree of the game
     uint64_t me = S.me[g], opp = S.opp[g];
     const int player = S.player[g], ply = S.ply[g];
     unsigned action;
-    if (n == 0 || total == 0) {  // a one-iteration search leaves no visits below the root: first legal move, or a pass
-        const uint64_t m = legal_mask(me, opp, cells);
-        action = m ? (unsigned)(__ffsll((long long)m) - 1) : 64u;
-    } else {  // most visited, lowest action id on ties (selfplay_advance_kernel, best_action_kernel)
-        unsigned key = (lane < n && Ne > 0) ? (((unsigned)Ne << 7) | (127u - act)) : 0u;
-        if (n > 32 && N32 > 0) {
-            const unsigned k32 = ((unsigned)N32 << 7) | (127u - act32);
-            key = k32 > key ? k32 : key;
+    if (minimax_entrants && ((minimax_entrants >> (S.pair_net[t / kPairTrees] & 63)) & 1)) {
+        action = minimax_action[t];
+        BZ_CHECK(action <= 64u, 37);  // a minimax move of a live game
+    } else {  // a net entrant: the most visited root action
+        BZ_CHECK(t < P.n_trees, 33);  // tree of the game
+        const uint32_t rmeta = P.root_meta[t];
+        const int n = (int)((rmeta >> BZ_META_N_SHIFT) & 63u);
+        const uint32_t *blk = P.arena + (int64_t)t * P.arena_units * 8 + (int64_t)(rmeta >> BZ_META_OFF_SHIFT) * 8;
+        int Ne = 0, N32 = 0;
+        unsigned act = 127u, act32 = 127u;
+        if (lane < n) {
+            Ne = (int)blk[BZ_NODE_HEADER_WORDS + lane];
+            act = blk[BZ_NODE_HEADER_WORDS + 3 * n + lane] & 127u;
         }
-        key = __reduce_max_sync(kFull, key);
-        action = 127u - (key & 127u);
+        if (n > 32) {
+            N32 = (int)blk[BZ_NODE_HEADER_WORDS + 32];
+            act32 = blk[BZ_NODE_HEADER_WORDS + 3 * n + 32] & 127u;
+        }
+        const int total = __reduce_add_sync(kFull, Ne) + N32;
+        if (n == 0 || total == 0) {  // a one-iteration search leaves no visits below the root: first legal move, or a pass
+            const uint64_t m = legal_mask(me, opp, cells);
+            action = m ? (unsigned)(__ffsll((long long)m) - 1) : 64u;
+        } else {  // most visited, lowest action id on ties (selfplay_advance_kernel, best_action_kernel)
+            unsigned key = (lane < n && Ne > 0) ? (((unsigned)Ne << 7) | (127u - act)) : 0u;
+            if (n > 32 && N32 > 0) {
+                const unsigned k32 = ((unsigned)N32 << 7) | (127u - act32);
+                key = k32 > key ? k32 : key;
+            }
+            key = __reduce_max_sync(kFull, key);
+            action = 127u - (key & 127u);
+        }
     }
     if (lane != 0) return;
     BZ_CHECK(ply >= 0 && ply < BZ_MATCH_MAX_PLIES && action <= 64u, 34);  // move row, action
@@ -573,7 +566,56 @@ int bz_match_advance(const bz_match_state *st, const bz_tree_pools *pools, bz_st
         return BZ_ERR_ARG;
     if (st->n_games == 0) return BZ_OK;
     match_advance_kernel<<<(st->n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
-        *st, *pools, cell_mask(st->board_size));
+        *st, *pools, cell_mask(st->board_size), 0ull, nullptr);
+    return launch_rc();
+}
+
+int bz_tournament_minimax(const bz_tournament_state *st, const int32_t *entrant_depth, void *workspace, uint8_t *action,
+                          int64_t *nodes_total, bz_stream_t stream) {
+    int rc = check_tournament(st);
+    if (rc != BZ_OK) return rc;
+    if (!entrant_depth || !workspace || !action) return BZ_ERR_ARG;
+    if (!aligned16(workspace)) return BZ_ERR_UNALIGNED;
+    MinimaxRoots R = {};
+    R.me = st->match.root_me;
+    R.opp = st->match.root_opp;
+    R.n = st->match.n_trees;
+    R.game_of_tree = st->match.game_of_tree;
+    R.pair_entrant = st->match.pair_net;
+    R.key_base = 2 * st->match.first_pair_id;
+    for (int e = 0; e < BZ_MAX_ENTRANTS; ++e) R.entrant_depth[e] = kMinimaxNotSearched;
+    for (int e = 0; e < st->n_entrants; ++e) {
+        const int d = entrant_depth[e];
+        if (d < -1 || d > BZ_MINIMAX_MAX_DEPTH) return BZ_ERR_ARG;
+        if (d >= 0) R.entrant_depth[e] = (uint8_t)d;
+    }
+    return minimax_launch(R, st->match.seed, st->match.board_size, workspace, action, nullptr, nullptr, nodes_total,
+                          as_stream(stream));
+}
+
+int bz_tournament_advance(const bz_tournament_state *st, const bz_tree_pools *pools, const int32_t *entrant_depth,
+                          const uint8_t *action, bz_stream_t stream) {
+    int rc = check_tournament(st);
+    if (rc != BZ_OK) return rc;
+    if (!entrant_depth || !action) return BZ_ERR_ARG;
+    uint64_t bits = 0;
+    bool nets = false;
+    for (int e = 0; e < st->n_entrants; ++e) {
+        const int d = entrant_depth[e];
+        if (d < -1 || d > BZ_MINIMAX_MAX_DEPTH) return BZ_ERR_ARG;
+        if (d >= 0) bits |= 1ull << e;
+        else nets = true;
+    }
+    bz_tree_pools P = {};
+    if (nets || pools) {
+        if (!pools || pools->game != BZ_GAME_REVERSI || pools->n_trees != st->match.n_trees ||
+            pools->board_size != st->match.board_size || !pools->root_meta || !pools->arena)
+            return BZ_ERR_ARG;
+        P = *pools;
+    }
+    if (st->match.n_games == 0) return BZ_OK;
+    match_advance_kernel<<<(st->match.n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
+        st->match, P, cell_mask(st->match.board_size), bits, action);
     return launch_rc();
 }
 

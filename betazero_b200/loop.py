@@ -10,7 +10,9 @@ consistency guarantee rather than a necessity; with ``--train-on-rank0`` only ra
 The training loop mirrors the reference's (Adam + cross-entropy, src/tic_tac_toe/SL/train.py:85-113) and, like it,
 saves the model at the end (:204-214) -- here a state_dict checkpoint per iteration (``--checkpoint``; one file per
 iteration when the path contains ``{iteration}``), resumable (``--resume``).  Prints one JSON line per iteration on rank 0.  With ``--eval-games N`` rank 0 also plays N games between the
-trained net and the net before training (``match.BatchedMatch``) and adds their score and Elo to the line.
+trained net and the net before training (``match.BatchedMatch``) and adds their score and Elo to the line; with
+``--eval-minimax DEPTH`` as well, it plays N more games between the trained net and the reference's minimax player of that
+depth (``tournament.Minimax``) and adds them as ``eval_minimax``: a yardstick that stays the same across iterations.
 """
 from __future__ import annotations
 
@@ -25,14 +27,14 @@ from types import SimpleNamespace
 import torch
 
 from . import dist as bzd
-from . import match, mcts, net, selfplay, train
+from . import match, mcts, minimax, net, selfplay, train
 
 
 def default_args(**over) -> SimpleNamespace:
     """the command line's defaults as a namespace (for callers that drive iterations from Python: bench.py, tests)"""
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
-                        reuse=False, eval_games=0)
+                        reuse=False, eval_games=0, eval_minimax=None)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -49,6 +51,11 @@ class LoopState:
         eg = int(getattr(args, "eval_games", 0))
         if eg < 0 or eg % 2:
             raise ValueError(f"eval_games must be an even number >= 0 (games are played in pairs); got {eg}")
+        em = getattr(args, "eval_minimax", None)
+        if em is not None:
+            minimax.check_depth(em)
+            if eg == 0:
+                raise ValueError("eval_minimax plays --eval-games games: set eval_games > 0")
         self.model = net.make_net(args.net, hidden=args.hidden, seed=args.seed)
         self.master = net.make_net(args.net, hidden=args.hidden, seed=args.seed, dtype=torch.float32)  # fp32 master weights
         self.opt = torch.optim.Adam(self.master.parameters(), lr=args.lr)  # the reference's optimiser family (SL/train.py:87)
@@ -140,6 +147,13 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["eval"] = {"score": r["score"], "elo": r["elo"], "elo_ci": r["elo_ci"], "wins": r["wins"], "draws": r["draws"],
                         "losses": r["losses"], "ms": (time.perf_counter() - t_eval) * 1e3}
         del snapshot
+    if getattr(args, "eval_minimax", None) is not None and rank == 0:
+        t_eval = time.perf_counter()
+        r = match.BatchedMatch(st.model, match.Minimax(args.eval_minimax), args.eval_games, args.sims, n_leaves=args.leaves,
+                               board_size=args.size, seed=args.seed * 1000 + it).play()
+        line["eval_minimax"] = {"depth": int(args.eval_minimax), "score": r["score"], "elo": r["elo"], "elo_ci": r["elo_ci"],
+                                "wins": r["wins"], "draws": r["draws"], "losses": r["losses"],
+                                "minimax_nodes": r["minimax_nodes"], "ms": (time.perf_counter() - t_eval) * 1e3}
     if caught:
         line["warnings"] = [str(w.message) for w in caught]
     if args.checkpoint and rank == 0:
@@ -187,6 +201,9 @@ def main():
     ap.add_argument("--eval-games", type=int, default=d.eval_games,
                     help="rank 0 plays this many games (even) between the trained net and the net before training after "
                          "every iteration, with --sims / --leaves, and reports them as \"eval\" (0 = off)")
+    ap.add_argument("--eval-minimax", type=int, default=d.eval_minimax, metavar="DEPTH",
+                    help="rank 0 also plays --eval-games games between the trained net and the reference's minimax player "
+                         "of this depth (0 .. 8) after every iteration, and reports them as \"eval_minimax\"")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

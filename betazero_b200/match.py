@@ -16,18 +16,19 @@ import argparse
 import json
 import math
 
-from .tournament import MAX_PLIES, RUNNING, TREES_PER_PAIR, Tournament, check_net, elo, elo_summary  # noqa: F401
+from .tournament import MAX_PLIES, RUNNING, TREES_PER_PAIR, Minimax, Tournament, check_net, elo, elo_summary  # noqa: F401
 
 
 class BatchedMatch(Tournament):
-    """``n_games`` (even) games between ``net_a`` and ``net_b``, all searched at once.  ``play()`` returns the result."""
+    """``n_games`` (even) games between ``net_a`` and ``net_b``, all searched at once.  ``play()`` returns the result.
+    ``net_b`` may be ``Minimax(depth)``: net A against the reference's minimax player (a fixed yardstick)."""
 
     def __init__(self, net_a, net_b, n_games: int, n_sims: int, n_leaves: int = 4, board_size: int = 8,
                  c_puct: float = 1.25, opening_plies: int = 4, seed: int = 0, first_pair_id: int = 0, device="cuda"):
         n_games = int(n_games)
         if n_games <= 0 or n_games % 2 or n_games >= 1 << 16:
             raise ValueError(f"n_games must be even, in 2 .. 65534 (games 2i and 2i+1 are a pair); got {n_games}")
-        super().__init__([(net_a, n_sims), (net_b, n_sims)], n_games, n_leaves=n_leaves, board_size=board_size,
+        super().__init__([(net_a, n_sims), net_b if isinstance(net_b, Minimax) else (net_b, n_sims)], n_games, n_leaves=n_leaves, board_size=board_size,
                          c_puct=c_puct, opening_plies=opening_plies, seed=seed, first_pair_id=first_pair_id,
                          device=device)
 
@@ -38,7 +39,8 @@ class BatchedMatch(Tournament):
                "losses": p["losses"], "disc_diff": int(self.counters[7])}
         out.update({k: p[k] for k in ("score", "elo", "elo_ci", "score_se", "pairs")})
         out.update({k: r[k] for k in ("plies", "simulations", "wall_s", "sims_per_s")})
-        out.update({"n_sims": self.n_sims[0], "n_leaves": self.n_leaves, "board_size": self.board_size})
+        out.update({"n_sims": self.n_sims[0], "n_leaves": self.n_leaves, "board_size": self.board_size,
+                    "minimax_nodes": r["minimax_nodes"]})
         out.update({k: r[k] for k in ("result", "moves", "count_x", "count_o")})
         return out
 

@@ -20,7 +20,7 @@ from abc import ABC, abstractmethod
 import numpy as np
 import torch
 
-from . import env, mcts
+from . import env, mcts, minimax
 from .boards import _grid_to_bits
 
 
@@ -179,3 +179,39 @@ class AIPlayer(ReversiPlayer):
 
     def get_move(self, board):
         return self._impl.get_move(board)
+
+
+class OptimalPlayer(ReversiPlayer):
+    """The reference's depth-limited minimax ``OptimalPlayer(symbol, max_depth)`` (reversi_players.py:35-77) on the GPU
+    kernel (``bz_minimax_moves``): disc-difference evaluation, first best move in row-major order, no pass handling
+    inside the search.  Where the search returns no move (``max_depth = 0``, or every move worth -inf) the reference
+    plays ``random.choice`` (:42-43); here that move is drawn with Philox keyed by ``seed`` and ``game_key`` and counted
+    by the discs on the board, so a game replays exactly (oracle/minimax_ref.py).  ``(None, None)`` when there is no
+    move (:32)."""
+
+    def __init__(self, symbol, max_depth: int, size: int = 8, seed: int = 0, game_key: int = 0):
+        self.symbol, self.max_depth = symbol, minimax.check_depth(max_depth)
+        self.size, self.seed, self.game_key = int(size), int(seed), int(game_key)
+        self.last_value = None
+        self.last_nodes = None
+
+    def get_move(self, board):
+        if int(board.size) != self.size:
+            raise ValueError(f"this player was built for {self.size}x{self.size} boards")
+        me, opp = _grid_to_bits(np.asarray(board.board), self.symbol, 8)
+        a, v, n = minimax.best_moves(env.to_device_u64(np.array([me], np.uint64)),
+                                     env.to_device_u64(np.array([opp], np.uint64)), self.max_depth, self.size, self.seed,
+                                     self.game_key)
+        a = int(a[0].item())
+        self.last_value, self.last_nodes = int(v[0].item()), int(n[0].item())
+        if a >= 64:  # pass (64) or finished game (255)
+            return None, None
+        return a >> 3, a & 7
+
+
+class RandomPlayer(OptimalPlayer):
+    """The reference's ``RandomPlayer(symbol)`` (reversi_players.py:26-32): a uniformly random legal move, here the
+    Philox move of ``OptimalPlayer`` at depth 0."""
+
+    def __init__(self, symbol, size: int = 8, seed: int = 0, game_key: int = 0):
+        super().__init__(symbol, 0, size=size, seed=seed, game_key=game_key)

@@ -14,7 +14,16 @@ budgets are equal.  Each ply:
 A launch lasts as long as its largest budget: the CTA pairs of entrants with smaller budgets finish early and leave
 their SMs idle for the rest of it.
 
+An entrant may also be ``Minimax(depth)``: the reference's own opponents, its depth-limited ``OptimalPlayer`` and (depth
+0) its ``RandomPlayer`` (reversi_players.py:26-77; ``players.OptimalPlayer``).  They put the nets on a fixed scale: a
+checkpoint's rating against ``Minimax(4)`` means the same in every run.  A minimax entrant keeps its range of trees in
+the layout but is searched with 0 iterations (its trees are not touched); ``bz_tournament_minimax`` finds its moves
+(``bz_minimax_moves`` with the match seed and game key ``2 first_pair_id + g``) and ``bz_tournament_advance`` plays them
+next to the nets' most visited actions.  Plies on which no net moves skip the tree search; a tournament of minimax
+entrants only allocates no trees at all.
+
     python -m betazero_b200.tournament A.pt B.pt C.pt --sims 800 --entrant-sims 800,800,200 --games-per-pairing 134
+    python -m betazero_b200.tournament A.pt B.pt --minimax 0,2,4
 """
 from __future__ import annotations
 
@@ -27,7 +36,7 @@ import time
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, minimax
 from ._lib import BzTournamentState, BzTreePools
 from .mcts import PRIOR_LOGITS_BF16, TreePools
 
@@ -158,10 +167,21 @@ def fit_ratings(n_entrants: int, pairings, pair_scores, max_iter: int = 100) -> 
     return r, se
 
 
+class Minimax:
+    """A tournament entrant that plays the reference's depth-limited minimax ``OptimalPlayer`` (``depth`` 0 .. 8; 0 is
+    its ``RandomPlayer``): in a ``Tournament``'s entrant list in place of ``(net, n_sims)``, or as ``BatchedMatch``'s B."""
+
+    def __init__(self, depth: int):
+        self.depth = minimax.check_depth(depth)
+
+    def __repr__(self):
+        return f"Minimax({self.depth})"
+
+
 class Tournament:
-    """Every pairing of ``entrants`` -- a list of ``(net, n_sims)``; one net may appear with several budgets and then
-    shares its weight image -- for ``games_per_pairing`` (even) games, all searched at once.  ``play()`` returns the
-    result.  Game pair i draws its opening with pair id ``first_pair_id + i``."""
+    """Every pairing of ``entrants`` -- a list of ``(net, n_sims)`` and ``Minimax(depth)``; one net may appear with
+    several budgets and then shares its weight image -- for ``games_per_pairing`` (even) games, all searched at once.
+    ``play()`` returns the result.  Game pair i draws its opening with pair id ``first_pair_id + i``."""
 
     def __init__(self, entrants, games_per_pairing: int, n_leaves: int = 4, board_size: int = 8, c_puct: float = 1.25,
                  opening_plies: int = 4, seed: int = 0, pairings=None, first_pair_id: int = 0, device="cuda"):
@@ -172,9 +192,10 @@ class Tournament:
         n_leaves, gpp = int(n_leaves), int(games_per_pairing)
         if n_leaves not in (1, 2, 4):
             raise ValueError(f"n_leaves must be 1, 2 or 4 (the one-launch search); got {n_leaves}")
-        sims = [int(s) for _, s in entrants]
-        for s in sims:
-            if s < n_leaves or s % n_leaves:
+        depths = [x.depth if isinstance(x, Minimax) else -1 for x in entrants]  # -1: a net entrant
+        sims = [0 if d >= 0 else int(x[1]) for x, d in zip(entrants, depths)]
+        for s, d in zip(sims, depths):
+            if d < 0 and (s < n_leaves or s % n_leaves):
                 raise ValueError(f"every budget must be a positive multiple of n_leaves; got {s} and {n_leaves}")
         if gpp <= 0 or gpp % 2:
             raise ValueError(f"games_per_pairing must be even and positive (games are played in pairs); got {gpp}")
@@ -198,17 +219,19 @@ class Tournament:
         if n_games >= 1 << 16:
             raise ValueError(f"{n_games} games in all; a tournament holds fewer than 65536")
         nets = []  # distinct nets, in order of first appearance
-        for n, _ in entrants:
-            if not any(n is m for m in nets):
+        for x, d in zip(entrants, depths):
+            n = x[0] if d < 0 else None
+            if n is not None and not any(n is m for m in nets):
                 check_net(n)
                 nets.append(n)
         self.entrants, self.nets, self.pairings = entrants, nets, pairings
         self.n_entrants, self.n_sims, self.n_leaves, self.board_size = E, sims, n_leaves, int(board_size)
+        self.depths = depths
         self.games_per_pairing, self.n_games = gpp, n_games
         self.device = torch.device(device)
         self.n_trees = n_games + (TREES_PER_PAIR - 1) * (E - 1)  # every range but the last padded to a pair boundary
-        self.pools = TreePools(self.n_trees, max(sims), board_size=board_size, c_puct=c_puct, n_leaves=n_leaves,
-                               prior_mode=PRIOR_LOGITS_BF16, eval_stride=72, device=device)
+        self.pools = (TreePools(self.n_trees, max(sims), board_size=board_size, c_puct=c_puct, n_leaves=n_leaves,
+                                prior_mode=PRIOR_LOGITS_BF16, eval_stride=72, device=device) if nets else None)
         dev, G, T = self.device, n_games, self.n_trees
 
         def e(n, dt):
@@ -237,6 +260,13 @@ class Tournament:
         self._ref, self._mref = C.byref(s), C.byref(s.match)
         self._images = (C.c_void_p * E)()
         self._iters = (C.c_int32 * E)(*[x // n_leaves for x in sims])
+        self._depths = (C.c_int32 * E)(*depths)
+        self.has_minimax = any(d >= 0 for d in depths)
+        if self.has_minimax:
+            self.minimax_action = e(T, torch.uint8)
+            self.minimax_nodes = torch.zeros(1, dtype=torch.int64, device=dev)
+            self._minimax_ws = minimax.workspace(T, dev)
+        self._net_moves = self._minimax_moves = bool(nets)  # who moves this ply (layout)
         self._L = _lib.load()
         self.plies = 0
         self.padding, self.chunks = [], []  # padding trees and launches of every ply
@@ -245,18 +275,33 @@ class Tournament:
     # -- the steps of a ply -------------------------------------------------------------------------------------------
     def init(self) -> None:
         """the openings; the entrants' weight images (``prepare_inference``) must exist"""
-        for k, (n, _) in enumerate(self.entrants):
-            self._images[k] = n._image_pair.data_ptr()
+        for k, (x, d) in enumerate(zip(self.entrants, self.depths)):
+            # a minimax entrant runs 0 iterations and loads no weights, but the entry wants an image for it
+            self._images[k] = (x[0] if d < 0 else self.nets[0])._image_pair.data_ptr() if self.nets else None
+        if self.has_minimax:
+            self.minimax_nodes.zero_()
         _lib.check(self._L.bz_match_init(self._mref, _lib.stream_ptr()), "bz_match_init")
 
     def layout(self) -> tuple[int, int]:
         """the tree layout of this ply; returns (trees to search, padding trees) -- one device-to-host read"""
         _lib.check(self._L.bz_tournament_layout(self._ref, _lib.stream_ptr()), "bz_tournament_layout")
-        c = self.counters[:3].tolist()
+        if not self.has_minimax:
+            c = self.counters[:3].tolist()
+            return int(c[1]), int(c[2])
+        if not self.nets:
+            c = self.counters[:3].tolist()
+            self._net_moves, self._minimax_moves = False, c[1] > 0
+            return int(c[1]), int(c[2])
+        c = torch.cat((self.counters[:3], self.pair_net.to(torch.int64))).tolist()
+        movers = {self.depths[e] >= 0 for e in c[3:3 + -(-int(c[1]) // TREES_PER_PAIR)]}
+        self._net_moves, self._minimax_moves = False in movers, True in movers
         return int(c[1]), int(c[2])
 
     def search(self, n_search: int) -> None:
-        """reset the first ``n_search`` trees at the layout's roots and search them, each CTA pair as its entrant"""
+        """reset the first ``n_search`` trees at the layout's roots and search them, each CTA pair as its entrant (nothing
+        on a ply where no net moves)"""
+        if not self._net_moves:
+            return
         q = BzTreePools.from_buffer_copy(self.pools.c_struct)  # a prefix of the pools: every array starts at tree 0
         q.n_trees = n_search
         ref, st = C.byref(q), _lib.stream_ptr()
@@ -265,8 +310,20 @@ class Tournament:
                                                          _lib.dptr(self.pair_net), st), "bz_mcts_search_fused_entrants")
         self._errors |= self.pools.error[:n_search].amax()  # stream-ordered: read once, after the tournament
 
+    def minimax_search(self) -> None:
+        """the minimax entrants' moves of this ply"""
+        if self.has_minimax and self._minimax_moves:
+            _lib.check(self._L.bz_tournament_minimax(self._ref, self._depths, _lib.dptr(self._minimax_ws),
+                                                     _lib.dptr(self.minimax_action), _lib.dptr(self.minimax_nodes),
+                                                     _lib.stream_ptr()), "bz_tournament_minimax")
+
     def advance(self) -> None:
-        _lib.check(self._L.bz_match_advance(self._mref, self.pools._ref, _lib.stream_ptr()), "bz_match_advance")
+        if not self.has_minimax:
+            _lib.check(self._L.bz_match_advance(self._mref, self.pools._ref, _lib.stream_ptr()), "bz_match_advance")
+            return
+        _lib.check(self._L.bz_tournament_advance(self._ref, self.pools._ref if self.pools else None, self._depths,
+                                                 _lib.dptr(self.minimax_action), _lib.stream_ptr()),
+                   "bz_tournament_advance")
 
     # -- the whole tournament -----------------------------------------------------------------------------------------
     def play(self) -> dict:
@@ -282,13 +339,14 @@ class Tournament:
             if n_search == 0:
                 break
             self.search(n_search)
+            self.minimax_search()
             self.advance()
             self.plies += 1
             self.padding.append(pad)
             self.chunks.append(-(-n_search // LAUNCH_TREES))
         torch.cuda.synchronize()
         wall = time.perf_counter() - t0
-        if int(self._errors.item()):
+        if self.pools is not None and int(self._errors.item()):
             raise _lib.BzError("tree pool overflow during the tournament")
         return self.results(wall)
 
@@ -300,7 +358,8 @@ class Tournament:
         first, second = self.first.cpu().numpy()[np.arange(G) // 2], self.second.cpu().numpy()[np.arange(G) // 2]
         x_ent = np.where(np.arange(G) % 2 == 0, first, second)
         o_ent = np.where(np.arange(G) % 2 == 0, second, first)
-        # simulations: every recorded move after the opening was searched by the entrant to move, with its budget
+        # simulations: every recorded move after the opening was searched by the entrant to move, with its budget (0 for a
+        # minimax entrant)
         budget = np.array(self.n_sims)
         k = np.arange(MAX_PLIES)[None, :]
         searched = (moves != 255) & (k >= self.opening_plies)
@@ -331,6 +390,9 @@ class Tournament:
                 "games": G, "games_per_pairing": self.games_per_pairing, "finished": int((~running).sum()),
                 "pairings": per, "crosstable": cross.tolist(), "ratings": ratings.tolist(), "rating_se": se.tolist(),
                 "plies": self.plies, "simulations": sims, "wall_s": wall_s,
+                "kinds": ["minimax" if d >= 0 else "net" for d in self.depths],
+                "depths": [d if d >= 0 else None for d in self.depths],
+                "minimax_nodes": int(self.minimax_nodes.item()) if self.has_minimax else 0,
                 "sims_per_s": sims / wall_s if wall_s > 0 else math.nan,
                 "padding_per_ply": float(pads.mean()) if pads.size else 0.0,
                 "max_padding": int(pads.max()) if pads.size else 0,
@@ -344,7 +406,9 @@ PER_GAME = ("pairing", "result", "moves", "count_x", "count_o")
 
 def main():
     ap = argparse.ArgumentParser(description="a round-robin tournament between checkpoints on one GPU")
-    ap.add_argument("checkpoints", nargs="+", help="checkpoints (train.save_checkpoint); one entrant each, a path may repeat")
+    ap.add_argument("checkpoints", nargs="*", help="checkpoints (train.save_checkpoint); one entrant each, a path may repeat")
+    ap.add_argument("--minimax", default=None, help="comma-separated depths (0 .. 8): one minimax entrant each, after the "
+                                                    "checkpoints (the reference's OptimalPlayer; depth 0 is its RandomPlayer)")
     ap.add_argument("--sims", type=int, default=800, help="simulations per move of every entrant")
     ap.add_argument("--entrant-sims", default=None, help="comma-separated simulations per move, one per entrant (overrides --sims)")
     ap.add_argument("--games-per-pairing", type=int, default=134, help="even; 28 pairings x 134 games fit one launch per ply")
@@ -363,9 +427,12 @@ def main():
     for p in args.checkpoints:
         if p not in loaded:
             loaded[p] = train.load_net(p)
-    r = Tournament([(loaded[p], s) for p, s in zip(args.checkpoints, sims)], args.games_per_pairing, n_leaves=args.leaves,
+    entrants = [(loaded[p], s) for p, s in zip(args.checkpoints, sims)]
+    entrants += [Minimax(int(d)) for d in args.minimax.split(",")] if args.minimax else []
+    r = Tournament(entrants, args.games_per_pairing, n_leaves=args.leaves,
                    board_size=args.size, c_puct=args.c_puct, opening_plies=args.opening_plies, seed=args.seed).play()
     r["checkpoints"] = args.checkpoints
+    r["minimax"] = [e.depth for e in entrants if isinstance(e, Minimax)]
     print(json.dumps({k: v for k, v in r.items() if k not in PER_GAME}), flush=True)
 
 

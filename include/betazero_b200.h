@@ -402,6 +402,48 @@ typedef struct bz_tournament_state {
  * bounds-check failure (BZ_CHECK); such a game gets no tree. */
 int bz_tournament_layout(const bz_tournament_state *st, bz_stream_t stream);
 
+/* Minimax entrants (the reference's depth-limited OptimalPlayer, reversi_players.py:35-77, and RandomPlayer as its depth 0;
+ * see bz_minimax_moves).  entrant_depth: a host array of n_entrants entries, -1 for a net entrant, 0 .. BZ_MINIMAX_MAX_DEPTH
+ * for a minimax entrant.  A minimax entrant keeps its range of trees in bz_tournament_layout and is given 0 iterations in
+ * bz_mcts_search_fused_entrants (its trees are then not touched).
+ * bz_tournament_minimax: for every tree t < match.n_trees of a minimax entrant's range that holds a game g
+ * (game_of_tree[t] >= 0), action[t] = the bz_minimax_moves move of the root (root_me[t], root_opp[t]) at the entrant's
+ * depth with the match's seed and key 2 first_pair_id + g; action[t] = 255 for every other tree.  workspace:
+ * bz_minimax_workspace_bytes(match.n_trees) bytes, 16-byte aligned.  nodes_total (may be NULL): device int64 [1], the
+ * nodes searched are added to it.
+ * bz_tournament_advance: bz_match_advance for tournaments with minimax entrants -- the game of a minimax entrant's tree
+ * plays action[t], every other game exactly what bz_match_advance plays.  pools may be NULL when every entrant is minimax.
+ * BZ_ERR_ARG (both): a bad tournament state, an entry of entrant_depth out of range, a NULL action or workspace; and for
+ * bz_tournament_advance a NULL or mismatched pools with a net entrant. */
+int bz_tournament_minimax(const bz_tournament_state *st, const int32_t *entrant_depth, void *workspace, uint8_t *action,
+                          int64_t *nodes_total, bz_stream_t stream);
+int bz_tournament_advance(const bz_tournament_state *st, const bz_tree_pools *pools, const int32_t *entrant_depth,
+                          const uint8_t *action, bz_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Depth-limited minimax: the reference's OptimalPlayer.get_move (src/reversi/players/reversi_players.py:35-77; the
+ * definition is oracle/minimax_ref.py).  For every root i (mover-relative (me[i], opp[i]), the mover is the player):
+ *  - minimax(node, depth): if depth >= max_depth or the game is over (reversi_board.py:61-65), the disc difference from
+ *    the player's point of view (evaluate_board via get_score, :71-77; no win bonus).  Otherwise the player's nodes
+ *    (even depths) take the maximum over their moves in row-major order, the opponent's nodes the minimum (:50-69).
+ *  - No pass handling: a node whose side has no move in a game that is not over is worth -inf at the player's nodes and
+ *    +inf at the opponent's (the loops of :51-59 and :61-69 never run).  value = +-127 stands for +-inf.
+ *  - The move is the first root move whose value is strictly above every earlier one (:56-58).  When there is none --
+ *    depth[i] == 0, or every child is worth -inf -- the move is drawn as the reference's random.choice (:42-43) is, here
+ *    reproducibly: u = Philox4x32-10(seed, key 2^32 + key[i], counter popcount(me | opp)), the k-th legal move in
+ *    ascending cell order with k = floor(u * moves / 2^32).  RandomPlayer (:26-32) is depth 0.
+ *  - action: the move (row*8 + col), 64 when the player has no move (a pass), 255 when the game is over.  value: the
+ *    root's minimax value (int8).  nodes: minimax calls searched for the root, the root included (may be NULL).
+ * depth: uint8 [n], 0 .. BZ_MINIMAX_MAX_DEPTH; a root with a larger depth is a bounds-check failure (BZ_CHECK) and is
+ * not searched (action 255, value 0, nodes 0).  workspace: bz_minimax_workspace_bytes(n) bytes, 16-byte aligned.  The
+ * search is alpha-beta, split at the root (one full-window search per root move); every result equals plain minimax.
+ * BZ_ERR_ARG: size not 4 / 6 / 8, n < 0 or n >= 2^25, a NULL pointer other than nodes; BZ_ERR_UNALIGNED: workspace. */
+#define BZ_MINIMAX_MAX_DEPTH 8
+int bz_minimax_moves(const uint64_t *me, const uint64_t *opp, const uint8_t *depth, const uint64_t *key, uint64_t seed,
+                     int64_t n, int size, void *workspace, uint8_t *action, int8_t *value, int64_t *nodes,
+                     bz_stream_t stream);
+int64_t bz_minimax_workspace_bytes(int64_t n);
+
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */
 int bz_philox_u32(uint64_t seed, const int64_t *game_id, const int32_t *ply, uint32_t *out, int64_t n,
                   bz_stream_t stream);

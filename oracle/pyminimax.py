@@ -1,0 +1,75 @@
+"""TEST INFRASTRUCTURE ONLY -- ctypes front end of oracle/libminimax.so (minimax.c), the C restatement of the minimax
+definition (minimax_ref.py) without pruning: the checker of bz_minimax_moves.  Built with gcc on first use, like
+pyoracle's library (content hash beside the library, inter-process lock)."""
+from __future__ import annotations
+
+import ctypes as C
+import fcntl
+import hashlib
+import os
+import subprocess
+
+import numpy as np
+
+_HERE = os.path.dirname(os.path.abspath(__file__))
+_SRC = os.path.join(_HERE, "minimax.c")
+_SO = os.path.join(_HERE, "libminimax.so")
+_CFLAGS = ["-O2", "-fPIC", "-shared", "-fopenmp", "-Wall", "-Wextra", "-std=c11"]
+_lib = None
+
+
+def _src_hash() -> str:
+    h = hashlib.sha256(" ".join(_CFLAGS).encode())
+    with open(_SRC, "rb") as f:
+        h.update(f.read())
+    return h.hexdigest()
+
+
+def build(force: bool = False) -> str:
+    stamp = _SO + ".srchash"
+
+    def stale():
+        try:
+            return not os.path.exists(_SO) or open(stamp).read().strip() != _src_hash()
+        except OSError:
+            return True
+
+    if not force and not stale():
+        return _SO
+    with open(_SO + ".lock", "w") as lock:
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        try:
+            if force or stale():
+                tmp = f"{_SO}.tmp.{os.getpid()}"
+                subprocess.check_call(["gcc", *_CFLAGS, "-o", tmp, _SRC])
+                os.replace(tmp, _SO)
+                with open(stamp + ".tmp", "w") as f:
+                    f.write(_src_hash())
+                os.replace(stamp + ".tmp", stamp)
+        finally:
+            fcntl.flock(lock, fcntl.LOCK_UN)
+    return _SO
+
+
+def lib():
+    global _lib
+    if _lib is None:
+        build()
+        L = C.CDLL(_SO)
+        p = C.c_void_p
+        L.orc_minimax_moves.argtypes = [p, p, p, p, C.c_uint64, C.c_int64, C.c_int, p, p, p]
+        L.orc_minimax_moves.restype = None
+        _lib = L
+    return _lib
+
+
+def minimax_moves(me, opp, depth, keys, seed: int = 0, size: int = 8):
+    """plain minimax of every root (bz_minimax_moves' semantics): (action uint8, value int8, nodes int64) [n]"""
+    me, opp = np.ascontiguousarray(me, np.uint64), np.ascontiguousarray(opp, np.uint64)
+    n = me.size
+    depth = np.ascontiguousarray(np.broadcast_to(depth, (n,)), np.uint8)
+    keys = np.ascontiguousarray(np.broadcast_to(keys, (n,)), np.uint64)
+    act, val, nodes = np.empty(n, np.uint8), np.empty(n, np.int8), np.empty(n, np.int64)
+    lib().orc_minimax_moves(me.ctypes.data, opp.ctypes.data, depth.ctypes.data, keys.ctypes.data, int(seed), n, int(size),
+                            act.ctypes.data, val.ctypes.data, nodes.ctypes.data)
+    return act, val, nodes

@@ -4,5 +4,5 @@ set -e
 name=$1; shift
 mkdir -p build/exp
 nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 --fmad=false -Xcompiler -fPIC -shared "$@" \
-  -o build/exp/lib_$name.so betazero_b200/csrc/{env,mcts,selfplay,mlp_pair,mlp_pair2}.cu
+  -o build/exp/lib_$name.so betazero_b200/csrc/{env,mcts,selfplay,mlp_pair,mlp_pair2,minimax}.cu
 echo build/exp/lib_$name.so
