@@ -107,6 +107,8 @@ SIGNATURES = {
     "bz_tournament_advance": [_TP, _PP, ptr, ptr, ptr],
     "bz_minimax_moves": [ptr, ptr, ptr, ptr, _U64, _I64, _INT, ptr, ptr, ptr, ptr, ptr],
     "bz_minimax_workspace_bytes": [_I64],
+    "bz_endgame_solve": [ptr, ptr, _I64, _INT, ptr, ptr, ptr, ptr, ptr, ptr],
+    "bz_endgame_workspace_bytes": [_I64],
     "bz_reversi_symmetry": [ptr, ptr, ptr, ptr, ptr, ptr, ptr, _I64, _INT, ptr],
     "bz_record_hash": [ptr, ptr, ptr, ptr, _I64, ptr],
     "bz_philox_u32": [_U64, ptr, ptr, ptr, _I64, ptr],

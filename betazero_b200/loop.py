@@ -13,6 +13,9 @@ iteration when the path contains ``{iteration}``), resumable (``--resume``).  Pr
 trained net and the net before training (``match.BatchedMatch``) and adds their score and Elo to the line; with
 ``--eval-minimax DEPTH`` as well, it plays N more games between the trained net and the reference's minimax player of that
 depth (``tournament.Minimax``) and adds them as ``eval_minimax``: a yardstick that stays the same across iterations.
+With ``--eval-endgame EMPTIES`` rank 0 scores the trained net's moves on a fixed suite of 4096 positions with that many
+empty squares against the exact solver (``betazero_b200.endgame``), at 0 simulations and at ``--sims`` / ``--leaves``, and
+adds ``eval_endgame``; the suite is drawn and solved once per run.
 """
 from __future__ import annotations
 
@@ -27,19 +30,22 @@ from types import SimpleNamespace
 import torch
 
 from . import dist as bzd
-from . import match, mcts, minimax, net, selfplay, train
+from . import endgame, match, mcts, minimax, net, selfplay, train
 
 
 def default_args(**over) -> SimpleNamespace:
     """the command line's defaults as a namespace (for callers that drive iterations from Python: bench.py, tests)"""
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
-                        reuse=False, eval_games=0, eval_minimax=None)
+                        reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
         setattr(a, k, v)
     return a
+
+
+ENDGAME_POSITIONS = 4096  # --eval-endgame: one launch of the one-launch search
 
 
 class LoopState:
@@ -56,6 +62,13 @@ class LoopState:
             minimax.check_depth(em)
             if eg == 0:
                 raise ValueError("eval_minimax plays --eval-games games: set eval_games > 0")
+        self.endgame_suite = None  # --eval-endgame: drawn and solved once per run (rank 0)
+        ee = getattr(args, "eval_endgame", None)
+        if ee is not None:
+            if not 1 <= int(ee) <= minimax.SOLVE_MAX_EMPTIES:
+                raise ValueError(f"eval_endgame must be in 1 .. {minimax.SOLVE_MAX_EMPTIES} empty squares; got {ee}")
+            if rank == 0:
+                self.endgame_suite = endgame.solve_suite(endgame.positions(ENDGAME_POSITIONS, int(ee), args.size, args.seed))
         self.model = net.make_net(args.net, hidden=args.hidden, seed=args.seed)
         self.master = net.make_net(args.net, hidden=args.hidden, seed=args.seed, dtype=torch.float32)  # fp32 master weights
         self.opt = torch.optim.Adam(self.master.parameters(), lr=args.lr)  # the reference's optimiser family (SL/train.py:87)
@@ -154,6 +167,11 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["eval_minimax"] = {"depth": int(args.eval_minimax), "score": r["score"], "elo": r["elo"], "elo_ci": r["elo_ci"],
                                 "wins": r["wins"], "draws": r["draws"], "losses": r["losses"],
                                 "minimax_nodes": r["minimax_nodes"], "ms": (time.perf_counter() - t_eval) * 1e3}
+    if st.endgame_suite is not None:
+        t_eval = time.perf_counter()
+        r = endgame.evaluate(st.model, st.endgame_suite, (0, args.sims), args.leaves)
+        line["eval_endgame"] = {"empties": r["empties"], "positions": r["positions"], "budgets": r["budgets"],
+                                "random": r["baselines"]["random"], "ms": (time.perf_counter() - t_eval) * 1e3}
     if caught:
         line["warnings"] = [str(w.message) for w in caught]
     if args.checkpoint and rank == 0:
@@ -204,6 +222,9 @@ def main():
     ap.add_argument("--eval-minimax", type=int, default=d.eval_minimax, metavar="DEPTH",
                     help="rank 0 also plays --eval-games games between the trained net and the reference's minimax player "
                          "of this depth (0 .. 8) after every iteration, and reports them as \"eval_minimax\"")
+    ap.add_argument("--eval-endgame", type=int, default=d.eval_endgame, metavar="EMPTIES",
+                    help="rank 0: score the trained net's moves on 4096 positions with EMPTIES empty squares (at most 20) "
+                         "against the exact solver, at 0 simulations and at --sims, and report them as \"eval_endgame\"")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

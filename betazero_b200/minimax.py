@@ -3,12 +3,17 @@
 is oracle/minimax_ref.py, the semantics are in include/betazero_b200.h).
 
     action, value, nodes = best_moves(me, opp, depth=4, size=8, seed=0, keys=game_keys)
+
+``solve`` is the exact endgame solver (``bz_endgame_solve``): the perfect player's move and every move's final disc
+difference for positions with at most 20 empty squares.
+
+    action, value, move_value, nodes = solve(me, opp, size=8)
 """
 from __future__ import annotations
 
 import torch
 
-from . import _lib
+from . import _lib, env
 
 MAX_DEPTH = 8  # BZ_MINIMAX_MAX_DEPTH
 
@@ -58,3 +63,37 @@ def best_moves(me: torch.Tensor, opp: torch.Tensor, depth, size: int = 8, seed: 
                                   int(seed) & (2**64 - 1), n, int(size), _lib.dptr(ws), _lib.dptr(action),
                                   _lib.dptr(value), _lib.dptr(nodes), _lib.stream_ptr()), "bz_minimax_moves")
     return action, value, nodes
+
+
+SOLVE_MAX_EMPTIES = 20  # BZ_SOLVE_MAX_EMPTIES
+
+
+def solve(me: torch.Tensor, opp: torch.Tensor, size: int = 8):
+    """The exact endgame value of every mover-relative root (me, opp: int64 CUDA tensors holding uint64 bitboards) with
+    at most 20 empty squares (``bz_endgame_solve``; the definition is oracle/endgame_ref.py).
+
+    Returns CUDA tensors (action uint8 [n]: the first best move, row*8 + col, 64 = a forced pass, 255 = game over;
+    value int8 [n]: the final disc difference for the mover under perfect play, empty squares to nobody; move_value int8
+    [n, 65]: the value of every legal move for the mover, the pass at 64, -128 for an action that is not legal; nodes
+    int64 [n]: positions the search entered).  ``ValueError`` for a root with more than 20 empties (one device read)."""
+    if size not in (4, 6, 8):
+        raise ValueError("size must be 4, 6 or 8 (Reversi)")
+    n = me.numel()
+    if opp.numel() != n:
+        raise ValueError("me and opp must have one entry per root")
+    dev = me.device
+    me, opp = me.contiguous(), opp.contiguous()
+    if n:
+        _, _, cm, co = env.terminal(me, opp, size)  # the disc counts
+        if int((cm.int() + co.int()).min()) < size * size - SOLVE_MAX_EMPTIES:
+            raise ValueError(f"the endgame solver takes positions with at most {SOLVE_MAX_EMPTIES} empty squares")
+    action = torch.empty(n, dtype=torch.uint8, device=dev)
+    value = torch.empty(n, dtype=torch.int8, device=dev)
+    move_value = torch.empty((n, 65), dtype=torch.int8, device=dev)
+    nodes = torch.empty(n, dtype=torch.int64, device=dev)
+    L = _lib.load()
+    ws = torch.empty(max(int(L.bz_endgame_workspace_bytes(n)), 16), dtype=torch.uint8, device=dev)
+    _lib.check(L.bz_endgame_solve(_lib.dptr(me), _lib.dptr(opp), n, int(size), _lib.dptr(ws), _lib.dptr(action),
+                                  _lib.dptr(value), _lib.dptr(move_value), _lib.dptr(nodes), _lib.stream_ptr()),
+               "bz_endgame_solve")
+    return action, value, move_value, nodes

@@ -215,3 +215,26 @@ class RandomPlayer(OptimalPlayer):
 
     def __init__(self, symbol, size: int = 8, seed: int = 0, game_key: int = 0):
         super().__init__(symbol, 0, size=size, seed=seed, game_key=game_key)
+
+
+class PerfectPlayer(ReversiPlayer):
+    """The perfect player of the endgame: the exact solver's move (``minimax.solve``, ``bz_endgame_solve``), the first
+    move in row-major order that reaches the best final disc difference.  It takes boards with at most 20 empty squares
+    (``ValueError`` otherwise) and returns ``(None, None)`` when there is no move (reversi_players.py:32)."""
+
+    def __init__(self, symbol, size: int = 8):
+        self.symbol, self.size = symbol, int(size)
+        self.last_value = None
+        self.last_nodes = None
+
+    def get_move(self, board):
+        if int(board.size) != self.size:
+            raise ValueError(f"this player was built for {self.size}x{self.size} boards")
+        me, opp = _grid_to_bits(np.asarray(board.board), self.symbol, 8)
+        a, v, _, n = minimax.solve(env.to_device_u64(np.array([me], np.uint64)),
+                                   env.to_device_u64(np.array([opp], np.uint64)), self.size)
+        a = int(a[0].item())
+        self.last_value, self.last_nodes = int(v[0].item()), int(n[0].item())
+        if a >= 64:  # pass (64) or finished game (255)
+            return None, None
+        return a >> 3, a & 7

@@ -444,6 +444,27 @@ int bz_minimax_moves(const uint64_t *me, const uint64_t *opp, const uint8_t *dep
                      bz_stream_t stream);
 int64_t bz_minimax_workspace_bytes(int64_t n);
 
+/* ------------------------------------------------------------------------------------------
+ * Exact endgame solver: the perfect player (the definition is oracle/endgame_ref.py; DESIGN.md section 2).  For
+ * every mover-relative root i (me[i], opp[i]) with e = size^2 - popcount(me | opp) <= BZ_SOLVE_MAX_EMPTIES empties:
+ *  - value(node): if the mover has a legal move, the maximum over its moves of -value(child); else, if the opponent has
+ *    one (a pass, reversi_terminal.py:31-35), -value(node with the sides swapped); else (game over)
+ *    popcount(me) - popcount(opp), the reference's counts (get_score, reversi_board.py:67-85): empty squares go to nobody.
+ *  - value[i]: the root's value (int8).  move_value: int8 [n, 65], -value(child) of every legal move; index 64 holds the
+ *    value of a forced pass; every action that is not legal holds -128.
+ *  - action[i]: the first maximum of move_value in cell order (the reference's strict ">"), 64 when the mover must pass,
+ *    255 when the game is over.
+ *  - nodes (may be NULL): positions entered for the root, the root and the positions after passes included.
+ * A root with more empties than BZ_SOLVE_MAX_EMPTIES is a bounds-check failure (BZ_CHECK) and is not searched: action
+ * 255, value 0, every move value -128, nodes 0.  workspace: bz_endgame_workspace_bytes(n) bytes, 16-byte aligned.  The
+ * search is alpha-beta with the full window, split at two plies (one search per root move and reply); every result
+ * but nodes equals plain negamax.  BZ_ERR_ARG: size not 4 / 6 / 8, n < 0 or n >= 2^25, a NULL pointer other than
+ * nodes; BZ_ERR_UNALIGNED: workspace. */
+#define BZ_SOLVE_MAX_EMPTIES 20
+int bz_endgame_solve(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
+                     int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream);
+int64_t bz_endgame_workspace_bytes(int64_t n);
+
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */
 int bz_philox_u32(uint64_t seed, const int64_t *game_id, const int32_t *ply, uint32_t *out, int64_t n,
                   bz_stream_t stream);
