@@ -45,6 +45,18 @@ class BzSelfplayState(C.Structure):
     ]
 
 
+class BzSelfplayEndgameState(C.Structure):
+    """Mirror of ``bz_selfplay_endgame_state`` (include/betazero_b200.h)."""
+
+    _fields_ = [
+        ("empties", C.c_int32), ("cap", C.c_int32), ("max_plies", C.c_int32), ("reserved", C.c_int32),
+        ("me", ptr), ("opp", ptr), ("player", ptr), ("ply", ptr), ("game_id", ptr), ("row", ptr),
+        ("hist_me", ptr), ("hist_opp", ptr), ("hist_player", ptr), ("hist_action", ptr), ("hist_pi", ptr),
+        ("count", ptr), ("counters", ptr),
+    ]
+    N_SCALARS = 4
+
+
 class BzMatchState(C.Structure):
     """Mirror of ``bz_match_state`` (include/betazero_b200.h)."""
 
@@ -70,6 +82,7 @@ class BzTournamentState(C.Structure):
 _I64, _INT, _U64, _F = C.c_int64, C.c_int, C.c_uint64, C.c_float
 _PP = C.POINTER(BzTreePools)
 _SP = C.POINTER(BzSelfplayState)
+_EP = C.POINTER(BzSelfplayEndgameState)
 _MP = C.POINTER(BzMatchState)
 _TP = C.POINTER(BzTournamentState)
 SIGNATURES = {
@@ -100,6 +113,9 @@ SIGNATURES = {
     "bz_hash_eval": [ptr, ptr, _U64, _INT, ptr, ptr, _I64, ptr],
     "bz_selfplay_init": [_SP, _I64, ptr],
     "bz_selfplay_advance": [_SP, _PP, ptr, ptr],
+    "bz_selfplay_advance_endgame": [_SP, _EP, _PP, ptr, ptr],
+    "bz_selfplay_endgame_play": [_SP, _EP, ptr, ptr],
+    "bz_selfplay_endgame_workspace_bytes": [_I64],
     "bz_match_init": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
     "bz_tournament_layout": [_TP, ptr],

@@ -15,7 +15,8 @@
 //
 // The endgame solver (bz_endgame_solve; definition: oracle/endgame_ref.py) searches to the end of the game with
 // negamax and passes, split at two plies; it has its own prep, search and finish kernels and shares the workspace
-// layout, the scan, item_root and the hand-out (take_item) with the minimax search.
+// layout, the scan, item_root and the hand-out (take_item) with the minimax search.  Self-play's endgame queue
+// (selfplay.cu) runs the same kernels with its root count read from device memory (endgame_launch_live).
 #include "bitboard.cuh"
 #include "common.cuh"
 #include "minimax.cuh"
@@ -320,10 +321,19 @@ __device__ __forceinline__ int solve_empties(uint64_t me, uint64_t opp, uint64_t
     return __popcll(cells) - __popcll((me | opp) & cells);
 }
 
+// kLive: the roots are [0, *live) of n (the self-play endgame queue: launch shapes depend on n only); the others get
+// no items
+template <bool kLive>
 __global__ void __launch_bounds__(256) endgame_prep_kernel(const uint64_t *me_, const uint64_t *opp_, int64_t n,
-                                                           uint64_t cells, Workspace W, uint8_t *action, int8_t *value) {
+                                                           uint64_t cells, Workspace W, uint8_t *action, int8_t *value,
+                                                           const int32_t *live) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if (kLive && i >= *live) {
+        W.nodes[i] = 0;
+        W.offset[i] = 0;
+        return;
+    }
     int *mv = reinterpret_cast<int *>(W.vals) + i * kMoveSlots;
     for (int j = 0; j < kMoveSlots; ++j) mv[j] = kUnset;
     const uint64_t me = me_[i], opp = opp_[i];
@@ -463,11 +473,12 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
     }
 }
 
+template <bool kLive>
 __global__ void __launch_bounds__(256) endgame_finish_kernel(const uint64_t *me_, const uint64_t *opp_, int64_t n,
                                                              uint64_t cells, Workspace W, uint8_t *action, int8_t *value,
-                                                             int8_t *move_value, int64_t *nodes) {
+                                                             int8_t *move_value, int64_t *nodes, const int32_t *live) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= n) return;
+    if (i >= n || (kLive && i >= *live)) return;
     const int *mv = reinterpret_cast<const int *>(W.vals) + i * kMoveSlots;
     int8_t *out = move_value + i * kMoveSlots;
     if (W.offset[i + 1] != W.offset[i]) {  // searched
@@ -528,16 +539,30 @@ int endgame_launch(const uint64_t *me, const uint64_t *opp, int64_t n, int size,
         const int64_t c = n - b < kSolveChunk ? n - b : kSolveChunk;
         const Workspace W = carve(workspace, c);
         const unsigned blocks = (unsigned)((c + 255) / 256);
-        endgame_prep_kernel<<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b);
+        endgame_prep_kernel<false><<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b, nullptr);
         minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, c);
         endgame_search_kernel<<<persistent_grid(c * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me + b, opp + b, c,
                                                                                                          cells, W);
-        endgame_finish_kernel<<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b,
-                                                          move_value + b * kMoveSlots, nodes ? nodes + b : nullptr);
+        endgame_finish_kernel<false><<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b,
+                                                                 move_value + b * kMoveSlots, nodes ? nodes + b : nullptr,
+                                                                 nullptr);
         const int rc = launch_rc();
         if (rc != BZ_OK) return rc;
     }
     return BZ_OK;
+}
+
+int endgame_launch_live(const uint64_t *me, const uint64_t *opp, int64_t n, const int32_t *live, int size, void *workspace,
+                        uint8_t *action, int8_t *value, int8_t *move_value, cudaStream_t stream) {
+    if (n <= 0 || n > kSolveChunk) return BZ_ERR_ARG;
+    const uint64_t cells = cell_mask(size);
+    const Workspace W = carve(workspace, n);
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    endgame_prep_kernel<true><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, live);
+    minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, n);  // the roots past *live have no items: no item maps to them
+    endgame_search_kernel<<<persistent_grid(n * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me, opp, n, cells, W);
+    endgame_finish_kernel<true><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, move_value, nullptr, live);
+    return launch_rc();
 }
 
 }  // namespace bz

@@ -26,11 +26,110 @@ __global__ void __launch_bounds__(256) selfplay_init_kernel(const bz_selfplay_st
     S.game_id[s] = first_game_id + s;
 }
 
-__global__ void __launch_bounds__(kThreads)
-    selfplay_advance_kernel(const bz_selfplay_state S, const bz_tree_pools P, uint8_t *action_out, uint64_t cells) {
-    const int s = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
-    if (s >= S.n_games) return;
-    const int lane = threadIdx.x & 31;
+// the game of slot s has left it (finished, or handed over to the endgame queue): the start position, the next game id
+__device__ __forceinline__ void restart_slot(const bz_selfplay_state &S, int s, int64_t gid) {
+    S.me[s] = start_me(S.board_size);
+    S.opp[s] = start_opp(S.board_size);
+    S.player[s] = 1;
+    S.ply[s] = 0;
+    S.game_id[s] = gid + S.id_stride;
+}
+
+// a warp: the game `gid` has ended at (me, opp), seen by the side to move after `player`'s last move; score it and copy
+// its nrec history rows, block `block` of max_plies rows in hist_*, to the replay buffer (whole or not at all); lane 0 counts
+__device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uint64_t *hist_me, const uint64_t *hist_opp,
+                                           const int8_t *hist_player, const float *hist_pi, int block, int max_plies,
+                                           int nrec, int64_t gid, uint64_t me, uint64_t opp, int player, int lane) {
+    const int cm = __popcll(me), co = __popcll(opp);
+    const int winner = ((cm > co) - (cm < co)) * (-player);  // absolute: +1 X, -1 O, 0 draw
+    // counters[0] = rows COMMITTED to the replay buffer: a game reserves its rows with a compare-and-swap and takes
+    // nothing when it does not fit, so [0, counters[0]) never contains a row that no game wrote
+    unsigned long long rb = ~0ull;  // ~0: no room, the game is dropped (counted in counters[5])
+    if (lane == 0) {
+        unsigned long long cur = S.counters[0];
+        while (cur + (unsigned long long)nrec <= (unsigned long long)S.replay_cap) {
+            const unsigned long long seen = atomicCAS(&S.counters[0], cur, cur + (unsigned long long)nrec);
+            if (seen == cur) {
+                rb = cur;
+                break;
+            }
+            cur = seen;
+        }
+        atomicAdd(&S.counters[1], 1ull);
+        atomicAdd(&S.counters[3 + winner], 1ull);
+        atomicAdd(&S.counters[6], 1ull);
+    }
+    rb = __shfl_sync(kFull, rb, 0);
+    __syncwarp();  // the record written above is visible to the copying lanes
+    const int64_t h0 = (int64_t)block * max_plies;
+    if (rb != ~0ull) {
+        BZ_CHECK(rb + (unsigned long long)nrec <= (unsigned long long)S.replay_cap && nrec <= S.max_plies, 22);  // replay rows
+        for (int r = lane; r < nrec; r += 32) {
+            S.rp_me[rb + r] = hist_me[h0 + r];
+            S.rp_opp[rb + r] = hist_opp[h0 + r];
+            S.rp_z[rb + r] = (int8_t)(winner * hist_player[h0 + r]);
+            S.rp_game[rb + r] = gid;
+            S.rp_ply[rb + r] = (int16_t)r;
+        }
+        const int64_t nf = (int64_t)nrec * A;  // pi rows are contiguous in both buffers
+        const float *src = hist_pi + h0 * A;
+        float *dst = S.rp_pi + (int64_t)rb * A;
+        for (int64_t i = lane; i < nf; i += 32) dst[i] = src[i];
+    } else if (lane == 0) {
+        atomicAdd(&S.counters[5], (unsigned long long)nrec);
+    }
+}
+
+// a warp: move the game of slot s -- (me, opp) with `player` to move, nrec history rows -- to the next free entry of the
+// endgame queue, its rows to the entry's history block (row == entry: the queue fills from an empty state between solver
+// phases); false, and counted, when the queue is full
+__device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_selfplay_endgame_state &EG, int s, int lane,
+                                         uint64_t me, uint64_t opp, int player, int nrec, int64_t gid) {
+    int q = -1;
+    if (lane == 0) {
+        int cur = *EG.count;
+        while (cur < EG.cap) {
+            const int seen = atomicCAS(EG.count, cur, cur + 1);
+            if (seen == cur) {
+                q = cur;
+                break;
+            }
+            cur = seen;
+        }
+        if (q < 0) atomicAdd(&EG.counters[2], 1ull);
+    }
+    q = __shfl_sync(kFull, q, 0);
+    if (q < 0) return false;
+    BZ_CHECK(q < EG.cap && nrec <= EG.max_plies && nrec <= S.max_plies, 23);  // queue entry, history rows
+    __syncwarp();  // the record written above is visible to the copying lanes
+    const int64_t src = (int64_t)s * S.max_plies, dst = (int64_t)q * EG.max_plies;
+    for (int r = lane; r < nrec; r += 32) {
+        EG.hist_me[dst + r] = S.hist_me[src + r];
+        EG.hist_opp[dst + r] = S.hist_opp[src + r];
+        EG.hist_player[dst + r] = S.hist_player[src + r];
+        EG.hist_action[dst + r] = S.hist_action[src + r];
+    }
+    const int64_t nf = (int64_t)nrec * A;
+    for (int64_t i = lane; i < nf; i += 32) EG.hist_pi[dst * A + i] = S.hist_pi[src * A + i];
+    if (lane == 0) {
+        EG.me[q] = me;
+        EG.opp[q] = opp;
+        EG.player[q] = (int8_t)player;
+        EG.ply[q] = nrec;
+        EG.game_id[q] = gid;
+        EG.row[q] = q;
+        atomicAdd(&S.counters[1], 1ull);
+        atomicAdd(&EG.counters[0], 1ull);
+    }
+    return true;
+}
+
+// a warp per game slot: the move from the root visit counts, the record, the move applied, the terminal test; a finished
+// game is flushed and its slot restarts.  kEndgame: a game whose move leaves EG->empties empties or fewer for the first
+// time goes to the endgame queue instead (and its slot restarts) when the queue has room.
+template <bool kEndgame>
+__device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const bz_tree_pools &P, uint8_t *action_out,
+                                             uint64_t cells, const bz_selfplay_endgame_state *EG, int s, int lane) {
 
     // root statistics: lane i holds edge i (ascending action id); a 33rd edge is read uniformly
     const uint32_t rmeta = P.root_meta[s];
@@ -100,10 +199,20 @@ __global__ void __launch_bounds__(kThreads)
     }
 
     // --- apply, terminal test -----------------------------------------------------------------
+    [[maybe_unused]] const uint64_t occupied = me | opp;
     apply_legal(me, opp, action);  // now the NEXT mover's view; next player = -player
     const bool over = (legal_mask(me, opp, cells) | legal_mask(opp, me, cells)) == 0;
     const int nrec = ply + 1;
     if (!over && nrec < S.max_plies) {
+        if constexpr (kEndgame) {
+            // the first position at E empties or fewer (the move placed a disc): a game the full queue refuses is not
+            // offered again and is searched to its end
+            if (__popcll(cells) - __popcll(me | opp) <= EG->empties && EG->empties < __popcll(cells) - __popcll(occupied) &&
+                handover(S, *EG, s, lane, me, opp, -player, nrec, gid)) {
+                if (lane == 0) restart_slot(S, s, gid);
+                return;
+            }
+        }
         if (lane == 0) {
             S.me[s] = me;
             S.opp[s] = opp;
@@ -115,51 +224,128 @@ __global__ void __launch_bounds__(kThreads)
     }
 
     // --- finished: score, flush the history to the replay buffer, restart the slot ----------------
-    const int cm = __popcll(me), co = __popcll(opp);
-    const int winner = ((cm > co) - (cm < co)) * (-player);  // absolute: +1 X, -1 O, 0 draw
-    // counters[0] = rows COMMITTED to the replay buffer: a game reserves its rows with a compare-and-swap and takes
-    // nothing when it does not fit, so [0, counters[0]) never contains a row that no game wrote
-    unsigned long long rb = ~0ull;  // ~0: no room, the game is dropped (counted in counters[5])
+    flush_game(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, nrec, gid, me, opp, player, lane);
+    if (lane == 0) restart_slot(S, s, gid);
+}
+
+__global__ void __launch_bounds__(kThreads)
+    selfplay_advance_kernel(const bz_selfplay_state S, const bz_tree_pools P, uint8_t *action_out, uint64_t cells) {
+    const int s = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (s >= S.n_games) return;
+    advance_slot<false>(S, P, action_out, cells, nullptr, s, threadIdx.x & 31);
+}
+
+__global__ void __launch_bounds__(kThreads)
+    selfplay_advance_endgame_kernel(const bz_selfplay_state S, const bz_tree_pools P, uint8_t *action_out, uint64_t cells,
+                                    const __grid_constant__ bz_selfplay_endgame_state EG) {
+    const int s = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (s >= S.n_games) return;
+    advance_slot<true>(S, P, action_out, cells, &EG, s, threadIdx.x & 31);
+}
+
+// ---- the endgame queue: one solver ply of every pending game -----------------------------------------------------------
+// a warp per entry i < count: record the position with pi = 1/k on each of the k moves whose value is the root value
+// (a forced pass: one-hot on 64), play the solver's first best move, flush a finished game (ply = -1 marks the entry)
+__global__ void __launch_bounds__(kThreads)
+    endgame_ply_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_endgame_state EG,
+                       const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value, uint64_t cells) {
+    const int i = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (i >= *EG.count) return;
+    const int lane = threadIdx.x & 31;
+    const int ply = EG.ply[i], player = EG.player[i], b = EG.row[i];
+    const int64_t gid = EG.game_id[i];
+    uint64_t me = EG.me[i], opp = EG.opp[i];
+    const unsigned action = solve_action[i];
+    const int v = solve_value[i];
+    const int8_t *mv = move_value + (int64_t)i * A;
+    const bool o0 = mv[lane] == v, o1 = mv[lane + 32] == v, o64 = mv[64] == v;  // illegal actions hold -128 < any value
+    const int k = __popc(__ballot_sync(kFull, o0)) + __popc(__ballot_sync(kFull, o1)) + (o64 ? 1 : 0);
+    const int64_t h = (int64_t)b * EG.max_plies + ply;
+    BZ_CHECK(i < EG.cap && b >= 0 && b < EG.cap && ply >= 0 && ply < EG.max_plies && action <= 64u && k >= 1, 24);
+    const float p = __fdiv_rn(1.0f, (float)(k > 0 ? k : 1));
+    float *pi = EG.hist_pi + h * A;
+    pi[lane] = o0 ? p : 0.f;
+    pi[lane + 32] = o1 ? p : 0.f;
     if (lane == 0) {
-        unsigned long long cur = S.counters[0];
-        while (cur + (unsigned long long)nrec <= (unsigned long long)S.replay_cap) {
-            const unsigned long long seen = atomicCAS(&S.counters[0], cur, cur + (unsigned long long)nrec);
-            if (seen == cur) {
-                rb = cur;
-                break;
+        pi[64] = o64 ? p : 0.f;
+        EG.hist_me[h] = me;
+        EG.hist_opp[h] = opp;
+        EG.hist_player[h] = (int8_t)player;
+        EG.hist_action[h] = (uint8_t)action;
+        atomicAdd(&EG.counters[1], 1ull);
+    }
+    apply_legal(me, opp, action);  // the next mover's view
+    const bool over = (legal_mask(me, opp, cells) | legal_mask(opp, me, cells)) == 0;
+    const int nrec = ply + 1;
+    if (!over && nrec < EG.max_plies) {
+        if (lane == 0) {
+            EG.me[i] = me;
+            EG.opp[i] = opp;
+            EG.player[i] = (int8_t)(-player);
+            EG.ply[i] = nrec;
+            atomicAdd(&S.counters[1], 1ull);
+        }
+        return;
+    }
+    flush_game(S, EG.hist_me, EG.hist_opp, EG.hist_player, EG.hist_pi, b, EG.max_plies, nrec, gid, me, opp, player,
+               lane);
+    if (lane == 0) {
+        EG.ply[i] = -1;
+        atomicAdd(&EG.counters[3], 1ull);
+    }
+}
+
+// one CTA: the live entries (ply >= 0) of [0, count) to the front, in order; count = their number.  In place: a chunk's
+// entries are read before any of them is written, and every entry moves down, never into a later chunk.
+__global__ void __launch_bounds__(1024) endgame_compact_kernel(const __grid_constant__ bz_selfplay_endgame_state EG) {
+    __shared__ int warp_base[32];
+    __shared__ int chunk_live;
+    const int n = *EG.count;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    int carry = 0;
+    for (int base = 0; base < n; base += 1024) {
+        const int i = base + tid;
+        const bool live = i < n && EG.ply[i] >= 0;
+        uint64_t me = 0, opp = 0;
+        int64_t gid = 0;
+        int ply = 0, row = 0, player = 0;
+        if (live) {
+            me = EG.me[i];
+            opp = EG.opp[i];
+            gid = EG.game_id[i];
+            ply = EG.ply[i];
+            row = EG.row[i];
+            player = EG.player[i];
+        }
+        const unsigned bal = __ballot_sync(kFull, live);
+        if (lane == 0) warp_base[w] = __popc(bal);
+        __syncthreads();
+        if (w == 0) {
+            const int c = warp_base[lane];
+            int incl = c;
+            for (int d = 1; d < 32; d <<= 1) {
+                const int up = __shfl_up_sync(kFull, incl, d);
+                if (lane >= d) incl += up;
             }
-            cur = seen;
+            warp_base[lane] = incl - c;
+            if (lane == 31) chunk_live = incl;
         }
-        atomicAdd(&S.counters[1], 1ull);
-        atomicAdd(&S.counters[3 + winner], 1ull);
-        atomicAdd(&S.counters[6], 1ull);
-    }
-    rb = __shfl_sync(kFull, rb, 0);
-    __syncwarp();  // the record written above is visible to the copying lanes
-    const int64_t h0 = (int64_t)s * S.max_plies;
-    if (rb != ~0ull) {
-        BZ_CHECK(rb + (unsigned long long)nrec <= (unsigned long long)S.replay_cap && nrec <= S.max_plies, 22);  // replay rows
-        for (int r = lane; r < nrec; r += 32) {
-            S.rp_me[rb + r] = S.hist_me[h0 + r];
-            S.rp_opp[rb + r] = S.hist_opp[h0 + r];
-            S.rp_z[rb + r] = (int8_t)(winner * S.hist_player[h0 + r]);
-            S.rp_game[rb + r] = gid;
-            S.rp_ply[rb + r] = (int16_t)r;
+        __syncthreads();
+        if (live) {
+            const int d = carry + warp_base[w] + __popc(bal & ((1u << lane) - 1u));
+            BZ_CHECK(d <= i && d < EG.cap, 25);  // entries move down
+            EG.me[d] = me;
+            EG.opp[d] = opp;
+            EG.game_id[d] = gid;
+            EG.ply[d] = ply;
+            EG.row[d] = row;
+            EG.player[d] = (int8_t)player;
         }
-        const int64_t nf = (int64_t)nrec * A;  // pi rows are contiguous in both buffers
-        const float *src = S.hist_pi + h0 * A;
-        float *dst = S.rp_pi + (int64_t)rb * A;
-        for (int64_t i = lane; i < nf; i += 32) dst[i] = src[i];
-    } else if (lane == 0) {
-        atomicAdd(&S.counters[5], (unsigned long long)nrec);
+        carry += chunk_live;
+        __syncthreads();
     }
-    if (lane == 0) {
-        S.me[s] = start_me(S.board_size);
-        S.opp[s] = start_opp(S.board_size);
-        S.player[s] = 1;
-        S.ply[s] = 0;
-        S.game_id[s] = gid + S.id_stride;
-    }
+    __syncthreads();  // every thread has read count
+    if (tid == 0) *EG.count = carry;
 }
 
 __global__ void __launch_bounds__(256)
@@ -503,6 +689,17 @@ int check_tournament(const bz_tournament_state *s) {
     return BZ_OK;
 }
 
+int check_endgame(const bz_selfplay_state *s, const bz_selfplay_endgame_state *e) {
+    if (!e) return BZ_ERR_ARG;
+    const int cells = s->board_size * s->board_size;
+    if (e->empties < 1 || e->empties > BZ_SOLVE_MAX_EMPTIES || e->empties > cells - 5) return BZ_ERR_ARG;
+    if (e->cap < 1 || e->cap > (1 << 22) || e->max_plies != s->max_plies) return BZ_ERR_ARG;
+    if (!e->me || !e->opp || !e->player || !e->ply || !e->game_id || !e->row || !e->hist_me || !e->hist_opp ||
+        !e->hist_player || !e->hist_action || !e->hist_pi || !e->count || !e->counters)
+        return BZ_ERR_ARG;
+    return BZ_OK;
+}
+
 int check_state(const bz_selfplay_state *s) {
     if (!s) return BZ_ERR_ARG;
     if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
@@ -540,6 +737,57 @@ int bz_selfplay_advance(const bz_selfplay_state *st, const bz_tree_pools *pools,
     selfplay_advance_kernel<<<(st->n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
         *st, *pools, action_out, cell_mask(st->board_size));
     return launch_rc();
+}
+
+int bz_selfplay_advance_endgame(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                const bz_tree_pools *pools, uint8_t *action_out, bz_stream_t stream) {
+    int rc = check_state(st);
+    if (rc != BZ_OK) return rc;
+    rc = check_endgame(st, eg);
+    if (rc != BZ_OK) return rc;
+    if (!pools || pools->game != BZ_GAME_REVERSI || pools->n_trees != st->n_games || pools->board_size != st->board_size ||
+        !pools->root_meta || !pools->arena)
+        return BZ_ERR_ARG;
+    if (st->n_games == 0) return BZ_OK;
+    selfplay_advance_endgame_kernel<<<(st->n_games + kWarpsPerCta - 1) / kWarpsPerCta, kThreads, 0, as_stream(stream)>>>(
+        *st, *pools, action_out, cell_mask(st->board_size), *eg);
+    return launch_rc();
+}
+
+// the solve's workspace, then its action [cap], value [cap] and move values [cap, 65], each 16-byte aligned
+static int64_t endgame_play_align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
+
+int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap) {
+    if (cap < 1) return 0;
+    return endgame_play_align16(endgame_workspace_bytes(cap)) + 2 * endgame_play_align16(cap) +
+           endgame_play_align16(cap * A);
+}
+
+int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
+                             bz_stream_t stream) {
+    int rc = check_state(st);
+    if (rc != BZ_OK) return rc;
+    rc = check_endgame(st, eg);
+    if (rc != BZ_OK) return rc;
+    if (!workspace) return BZ_ERR_ARG;
+    if (!aligned16(workspace)) return BZ_ERR_UNALIGNED;
+    const int64_t cap = eg->cap;
+    char *p = static_cast<char *>(workspace) + endgame_play_align16(endgame_workspace_bytes(cap));
+    uint8_t *action = reinterpret_cast<uint8_t *>(p);
+    int8_t *value = reinterpret_cast<int8_t *>(p + endgame_play_align16(cap));
+    int8_t *move_value = value + endgame_play_align16(cap);
+    const cudaStream_t s = as_stream(stream);
+    const uint64_t cells = cell_mask(st->board_size);
+    for (int k = 0; k < 2 * eg->empties; ++k) {
+        rc = endgame_launch_live(eg->me, eg->opp, cap, eg->count, st->board_size, workspace, action, value, move_value, s);
+        if (rc != BZ_OK) return rc;
+        endgame_ply_kernel<<<(unsigned)((cap + kWarpsPerCta - 1) / kWarpsPerCta), kThreads, 0, s>>>(*st, *eg, action, value,
+                                                                                                    move_value, cells);
+        endgame_compact_kernel<<<1, 1024, 0, s>>>(*eg);
+        rc = launch_rc();
+        if (rc != BZ_OK) return rc;
+    }
+    return BZ_OK;
 }
 
 int bz_match_init(const bz_match_state *st, bz_stream_t stream) {

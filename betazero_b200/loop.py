@@ -15,7 +15,10 @@ trained net and the net before training (``match.BatchedMatch``) and adds their 
 depth (``tournament.Minimax``) and adds them as ``eval_minimax``: a yardstick that stays the same across iterations.
 With ``--eval-endgame EMPTIES`` rank 0 scores the trained net's moves on a fixed suite of 4096 positions with that many
 empty squares against the exact solver (``betazero_b200.endgame``), at 0 simulations and at ``--sims`` / ``--leaves``, and
-adds ``eval_endgame``; the suite is drawn and solved once per run.
+adds ``eval_endgame``; the suite is drawn and solved once per run.  With ``--endgame-empties E`` self-play hands every game to
+the exact solver once a searched move leaves at most E empty squares, and runs a solver phase every ``--endgame-every``
+plies (``selfplay.BatchedSelfPlay``); the line then has an ``endgame`` entry with the solver's counts and the time of its
+phases.
 """
 from __future__ import annotations
 
@@ -37,7 +40,7 @@ def default_args(**over) -> SimpleNamespace:
     """the command line's defaults as a namespace (for callers that drive iterations from Python: bench.py, tests)"""
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
-                        reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None)
+                        reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None, endgame_empties=0, endgame_every=8)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -81,7 +84,9 @@ class LoopState:
         self.sp = selfplay.BatchedSelfPlay(args.games, args.sims, self.evaluator, board_size=args.size,
                                            temp_plies=args.temp_plies, seed=args.seed, rank=rank, world=world,
                                            n_leaves=args.leaves, reuse=bool(getattr(args, "reuse", False)),
-                                           graph_unroll=min(16, max(1, args.sims // args.leaves - 1)))
+                                           graph_unroll=min(16, max(1, args.sims // args.leaves - 1)),
+                                           endgame_empties=int(getattr(args, "endgame_empties", 0)),
+                                           endgame_every=int(getattr(args, "endgame_every", 8)))
         self.sp.prepare()
 
     @torch.no_grad()
@@ -104,6 +109,7 @@ def run_iteration(st: LoopState, it: int) -> dict:
     args, rank, world, sp = st.args, st.rank, st.world, st.sp
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
     torch.cuda.synchronize()
+    eg_ms0, eg_stats0 = (sp.endgame_ms(), sp.stats()) if sp.eg is not None else (0.0, None)
     t0 = time.perf_counter()
     ev[0].record()
     for _ in range(args.plies):
@@ -153,6 +159,13 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["replay_gather"]["algbw_GBps"] = gather_info["gathered_bytes"] / sec / 1e9
         line["replay_gather"]["busbw_GBps"] = gather_info["gathered_bytes"] * (world - 1) / world / sec / 1e9
         line["weight_broadcast_busbw_GBps"] = nbytes / (ms["weight_broadcast"] * 1e-3) / 1e9
+    if sp.eg is not None:
+        line["endgame"] = {"empties": sp.endgame_empties, "every": sp.endgame_every,
+                           "games": stats["endgame_games"] - eg_stats0["endgame_games"],
+                           "plies": stats["endgame_plies"] - eg_stats0["endgame_plies"],
+                           "pending": stats["endgame_pending"],
+                           "overflow": stats["endgame_overflow"] - eg_stats0["endgame_overflow"],
+                           "ms": sp.endgame_ms() - eg_ms0}
     if snapshot is not None:
         t_eval = time.perf_counter()
         r = match.BatchedMatch(st.model, snapshot, args.eval_games, args.sims, n_leaves=args.leaves, board_size=args.size,
@@ -225,6 +238,11 @@ def main():
     ap.add_argument("--eval-endgame", type=int, default=d.eval_endgame, metavar="EMPTIES",
                     help="rank 0: score the trained net's moves on 4096 positions with EMPTIES empty squares (at most 20) "
                          "against the exact solver, at 0 simulations and at --sims, and report them as \"eval_endgame\"")
+    ap.add_argument("--endgame-empties", type=int, default=d.endgame_empties, metavar="E",
+                    help="hand every self-play game to the exact endgame solver once a searched move leaves at most E "
+                         "empty squares (1 .. 20; 0 = off): perfect play and exact z labels for the end of every game")
+    ap.add_argument("--endgame-every", type=int, default=d.endgame_every, metavar="K",
+                    help="with --endgame-empties: run a solver phase on the queued games every K plies")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

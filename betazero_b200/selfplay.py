@@ -7,6 +7,12 @@ Per ply, for ALL game slots at once:
     replay buffer, restart the slot) -> next search from the new positions.
 Games shard embarrassingly: rank r of W owns game ids {r*B + s + k*W*B}; move sampling is keyed by
 (seed, game id, ply), so a game's content does not depend on which GPU / slot played it.
+
+Endgame handover (opt-in, ``endgame_empties=E``): a game whose searched move leaves at most E empty squares moves to a
+device-side queue and its slot restarts; every ``endgame_every`` plies the exact solver plays every queued game to its end
+(bz_selfplay_advance_endgame, bz_selfplay_endgame_play).  Its records up to the handover are those the game has without
+the feature, the solver's records carry pi uniform over the optimal moves, and every z is the exact outcome of the
+handover position.
 """
 from __future__ import annotations
 
@@ -15,10 +21,19 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import BzSelfplayState
+from ._lib import BzSelfplayEndgameState, BzSelfplayState
 from .mcts import BatchedMCTS, TreePools
 
 N_ACTIONS = 65
+SOLVE_MAX_EMPTIES = 20  # BZ_SOLVE_MAX_EMPTIES
+
+
+def check_endgame_empties(empties, board_size: int) -> int:
+    """0 (off) or 1 .. min(20, size^2 - 5): the start position is always searched"""
+    e, hi = int(empties), min(SOLVE_MAX_EMPTIES, int(board_size) ** 2 - 5)
+    if e != 0 and not 1 <= e <= hi:
+        raise ValueError(f"endgame_empties must be 0 (off) or in 1 .. {hi} on a {board_size}x{board_size} board; got {empties}")
+    return e
 
 
 class BatchedSelfPlay:
@@ -26,8 +41,16 @@ class BatchedSelfPlay:
                  temp_plies: int = 0, seed: int = 0, replay_cap: int | None = None, rank: int = 0, world: int = 1,
                  arena_units: int | None = None, use_graph: bool = True, graph_unroll: int = 16,
                  dirichlet_alpha: float = 0.0, dirichlet_eps: float = 0.25, n_leaves: int = 1, device="cuda",
-                 one_launch: bool | None = None, reuse: bool = False):
+                 one_launch: bool | None = None, reuse: bool = False, endgame_empties: int = 0, endgame_every: int = 8,
+                 endgame_cap: int | None = None):
         self.n_games, self.n_sims, self.board_size = int(n_games), int(n_sims), int(board_size)
+        self.endgame_empties = check_endgame_empties(endgame_empties, board_size)
+        self.endgame_every = int(endgame_every)
+        if self.endgame_every < 1:
+            raise ValueError(f"endgame_every must be >= 1; got {endgame_every}")
+        self.endgame_cap = int(endgame_cap if endgame_cap is not None else max(self.n_games, 1))
+        if not 1 <= self.endgame_cap <= 1 << 22:
+            raise ValueError(f"endgame_cap must be in 1 .. 2^22; got {endgame_cap}")
         self.rank, self.world = int(rank), int(world)
         self.device = torch.device(device)
         # reuse: a move's search continues on the subtree of the move played (opt-in; bz_mcts_reroot) -- n_sims MORE
@@ -70,6 +93,35 @@ class BatchedSelfPlay:
         self._dropped_seen = 0  # counters[5] at the last drain (overflow is reported, never silent)
         _lib.check(self._L.bz_selfplay_init(self._ref, self.rank * self.n_games, _lib.stream_ptr()), "bz_selfplay_init")
         self.launches += 1
+        self.eg = None
+        self._advances = 0
+        self._eg_events = []  # (start, end) CUDA events of the solver phases not yet summed
+        self._eg_ms = 0.0
+        if self.endgame_empties:
+            self._init_endgame()
+
+    def _init_endgame(self) -> None:
+        Q, dev = self.endgame_cap, self.device
+        H = Q * self.max_plies
+
+        def e(n, dt):
+            return torch.empty(n, dtype=dt, device=dev)
+
+        self.eg_me, self.eg_opp = e(Q, torch.int64), e(Q, torch.int64)
+        self.eg_player, self.eg_ply, self.eg_game_id, self.eg_row = (e(Q, torch.int8), e(Q, torch.int32),
+                                                                     e(Q, torch.int64), e(Q, torch.int32))
+        self.eg_hist_me, self.eg_hist_opp = e(H, torch.int64), e(H, torch.int64)
+        self.eg_hist_player, self.eg_hist_action = e(H, torch.int8), e(H, torch.uint8)
+        self.eg_hist_pi = e(H * N_ACTIONS, torch.float32)
+        self.eg_count = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.eg_counters = torch.zeros(4, dtype=torch.int64, device=dev)
+        self.eg_workspace = e(max(int(self._L.bz_selfplay_endgame_workspace_bytes(Q)), 16), torch.uint8)
+        g = BzSelfplayEndgameState()
+        g.empties, g.cap, g.max_plies = self.endgame_empties, Q, self.max_plies
+        for name, _ in BzSelfplayEndgameState._fields_[BzSelfplayEndgameState.N_SCALARS:]:
+            setattr(g, name, getattr(self, "eg_" + name).data_ptr())
+        self.eg = g
+        self._eg_ref = C.byref(g)
 
     # -- one lockstep ply for every game ----------------------------------------------------------
     def search(self) -> None:
@@ -84,9 +136,39 @@ class BatchedSelfPlay:
         self._moves += 1
 
     def advance(self) -> None:
-        _lib.check(self._L.bz_selfplay_advance(self._ref, self.pools._ref, _lib.dptr(self.last_action),
-                                               _lib.stream_ptr()), "bz_selfplay_advance")
+        if self.eg is None:
+            _lib.check(self._L.bz_selfplay_advance(self._ref, self.pools._ref, _lib.dptr(self.last_action),
+                                                   _lib.stream_ptr()), "bz_selfplay_advance")
+            self.launches += 1
+            return
+        _lib.check(self._L.bz_selfplay_advance_endgame(self._ref, self._eg_ref, self.pools._ref, _lib.dptr(self.last_action),
+                                                       _lib.stream_ptr()), "bz_selfplay_advance_endgame")
         self.launches += 1
+        self._advances += 1
+        if self._advances % self.endgame_every == 0:
+            self.endgame_play()
+
+    def endgame_play(self) -> None:
+        """One solver phase: every game in the endgame queue is played to its end by the exact solver and flushed to the
+        replay buffer (a fixed number of launches, no host synchronisation).  ``advance`` calls it every
+        ``endgame_every`` plies."""
+        if self.eg is None:
+            raise RuntimeError("endgame_play needs endgame_empties > 0")
+        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        t0.record()
+        _lib.check(self._L.bz_selfplay_endgame_play(self._ref, self._eg_ref, _lib.dptr(self.eg_workspace),
+                                                    _lib.stream_ptr()), "bz_selfplay_endgame_play")
+        t1.record()
+        self._eg_events.append((t0, t1))
+        self.launches += 6 * 2 * self.endgame_empties  # per solver ply: the solve's four kernels, the move, the compaction
+
+    def endgame_ms(self) -> float:
+        """milliseconds spent in solver phases so far (CUDA events; waits for the phases recorded since the last call)"""
+        for t0, t1 in self._eg_events:
+            t1.synchronize()
+            self._eg_ms += t0.elapsed_time(t1)
+        self._eg_events = []
+        return self._eg_ms
 
     def play_move(self) -> None:
         self.search()
@@ -99,11 +181,18 @@ class BatchedSelfPlay:
     # -- results ---------------------------------------------------------------------------------
     def stats(self) -> dict:
         c = self.counters.cpu().tolist()
-        return {"replay_records": c[0], "plies": c[1], "o_wins": c[2], "draws": c[3], "x_wins": c[4],
-                "dropped": c[5], "games": c[6]}
+        out = {"replay_records": c[0], "plies": c[1], "o_wins": c[2], "draws": c[3], "x_wins": c[4],
+               "dropped": c[5], "games": c[6]}
+        # endgame handover: games the solver finished, plies it played, games waiting in the queue, handovers refused
+        # because the queue was full (those games are searched to their end in their slots)
+        eg = self.eg_counters.cpu().tolist() if self.eg is not None else [0, 0, 0, 0]
+        out.update({"endgame_games": eg[3], "endgame_plies": eg[1],
+                    "endgame_pending": int(self.eg_count.item()) if self.eg is not None else 0, "endgame_overflow": eg[2]})
+        return out
 
     def drain_replay(self) -> dict:
-        """Returns the finished games' records (device tensors, copies) and empties the buffer."""
+        """Returns the finished games' records (device tensors, copies) and empties the buffer.  Games in the endgame
+        queue are games in progress, like those in the slots: a later solver phase finishes them."""
         c = self.counters.cpu().tolist()
         n = min(int(c[0]), self.replay_cap)  # counters[0] counts committed rows only (a game that does not fit takes none)
         if c[5] > self._dropped_seen:

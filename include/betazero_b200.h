@@ -344,6 +344,54 @@ int bz_selfplay_init(const bz_selfplay_state *st, int64_t first_game_id, bz_stre
 int bz_selfplay_advance(const bz_selfplay_state *st, const bz_tree_pools *pools, uint8_t *action_out,
                         bz_stream_t stream);
 
+/* Endgame handover (opt-in): the exact solver (bz_endgame_solve) plays the end of every self-play game.
+ * A game leaves its slot for a device-side PENDING QUEUE when a searched move leaves a position that is not over and has
+ * at most `empties` empty squares for the first time; the slot restarts at once with the next game id, as if the game had
+ * finished.
+ * bz_selfplay_endgame_play then plays every pending game to its end with the perfect player, one batched solve per ply:
+ * the move is the solver's first best move (a forced pass is a pass), and the record's pi is 1/k (__fdiv_rn) on each of
+ * the k actions whose move value equals the root value (one-hot on 64 for a forced pass).  A game that ends is flushed
+ * to the replay buffer exactly as bz_selfplay_advance flushes one (reservation, whole-game drops in counters[5], the
+ * winner counters, z = winner * player for every record, the searched prefix included).  Play after the handover is
+ * perfect, so every z is the exact outcome of the handover position.  The queue entry keeps the game's history rows;
+ * `row` maps an entry to its history block (entries are compacted after every solver ply, their rows stay in place). */
+typedef struct bz_selfplay_endgame_state {
+    int32_t empties;   /* E: 1 .. min(BZ_SOLVE_MAX_EMPTIES, board_size^2 - 5) */
+    int32_t cap;       /* queue entries, 1 .. 2^22 */
+    int32_t max_plies; /* history rows per entry: the self-play state's max_plies */
+    int32_t reserved;
+    /* per entry [cap] */
+    uint64_t *me, *opp; /* current position, mover-relative */
+    int8_t *player;     /* absolute side to move */
+    int32_t *ply;       /* rows recorded so far */
+    int64_t *game_id;
+    int32_t *row;       /* history block of the entry */
+    /* history blocks [cap * max_plies] (pi: [.., 65]) */
+    uint64_t *hist_me, *hist_opp;
+    int8_t *hist_player;
+    uint8_t *hist_action;
+    float *hist_pi;
+    /* device int32 [1]: pending games, entries [0, count) */
+    int32_t *count;
+    /* device uint64 [4]: 0 games handed over, 1 plies played by the solver, 2 handovers refused because the queue was
+     * full (the game stays in its slot and is searched to its end), 3 games the solver finished */
+    unsigned long long *counters;
+} bz_selfplay_endgame_state;
+
+/* bz_selfplay_advance plus the handover.  A game the full queue refuses stays in its slot and is searched to its end.  The self-play counters count
+ * the handover ply as a ply played.  count and counters start at zero (the caller zeroes them once).  BZ_ERR_ARG: what
+ * bz_selfplay_advance refuses, a NULL pointer in eg, empties or cap out of range, eg->max_plies != st->max_plies. */
+int bz_selfplay_advance_endgame(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                const bz_tree_pools *pools, uint8_t *action_out, bz_stream_t stream);
+/* One solver phase: 2 * empties solver plies (a game with E empties ends within 2E plies: a pass is always followed
+ * by a move), each a solve of the pending positions, the move, the record, the flush of finished games and the
+ * compaction of the live entries.  The launch shapes depend on cap only; a step with no pending game exits on the
+ * device.  The queue is empty afterwards, and the self-play counters count every solver ply as a ply played.
+ * workspace: bz_selfplay_endgame_workspace_bytes(cap) bytes, 16-byte aligned. */
+int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
+                             bz_stream_t stream);
+int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap);
+
 /* ------------------------------------------------------------------------------------------
  * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
  * the same launches; a net-versus-net match is the tournament of two entrants and the one pairing (0, 1).  Game pair i
