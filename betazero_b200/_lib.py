@@ -115,6 +115,7 @@ SIGNATURES = {
     "bz_selfplay_advance": [_SP, _PP, ptr, ptr],
     "bz_selfplay_advance_endgame": [_SP, _EP, _PP, ptr, ptr],
     "bz_selfplay_endgame_play": [_SP, _EP, ptr, ptr],
+    "bz_selfplay_endgame_play_wld": [_SP, _EP, ptr, ptr],
     "bz_selfplay_endgame_workspace_bytes": [_I64],
     "bz_match_init": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
@@ -125,6 +126,7 @@ SIGNATURES = {
     "bz_minimax_workspace_bytes": [_I64],
     "bz_endgame_solve": [ptr, ptr, _I64, _INT, ptr, ptr, ptr, ptr, ptr, ptr],
     "bz_endgame_workspace_bytes": [_I64],
+    "bz_endgame_solve_wld": [ptr, ptr, _I64, _INT, ptr, ptr, ptr, ptr, ptr, ptr],
     "bz_reversi_symmetry": [ptr, ptr, ptr, ptr, ptr, ptr, ptr, _I64, _INT, ptr],
     "bz_record_hash": [ptr, ptr, ptr, ptr, _I64, ptr],
     "bz_philox_u32": [_U64, ptr, ptr, ptr, _I64, ptr],

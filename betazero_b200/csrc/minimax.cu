@@ -15,8 +15,10 @@
 //
 // The endgame solver (bz_endgame_solve; definition: oracle/endgame_ref.py) searches to the end of the game with
 // negamax and passes, split at two plies; it has its own prep, search and finish kernels and shares the workspace
-// layout, the scan, item_root and the hand-out (take_item) with the minimax search.  Self-play's endgame queue
-// (selfplay.cu) runs the same kernels with its root count read from device memory (endgame_launch_live).
+// layout, the scan, item_root and the hand-out (take_item) with the minimax search.  Its win/draw/loss form
+// (bz_endgame_solve_wld) is the same kernels instantiated with kWld: a null window and fastest-first move ordering.
+// Self-play's endgame queue (selfplay.cu) runs the same kernels with its root count read from device memory
+// (endgame_launch_live).
 #include "bitboard.cuh"
 #include "common.cuh"
 #include "minimax.cuh"
@@ -303,10 +305,24 @@ __global__ void __launch_bounds__(256) minimax_finish_kernel(const MinimaxRoots 
 // row-major order and the full window, so the item's value is exact.  move_value[a] is the minimum over a's items
 // (atomicMin into the workspace), and the finish kernel takes the first maximum.  A root that must pass has the pass as
 // its one move.  Workspace, scan, item_root and the persistent hand-out are those of the minimax search.
+//
+// The win/draw/loss solve (kWld; bz_endgame_solve_wld) runs the same items with the null window (-1, 1): fail-soft, an
+// item's value v >= 1 is a win, v <= -1 a loss and 0 an exact draw, so clamped to [-1, 1] it is the sign of the exact
+// value, and so is the minimum over a move's replies.  At every node with at least kOrderEmpties empties it tries the
+// moves fastest first: fewest legal replies for the opponent first, ties in cell order.  Below that it keeps the
+// row-major descent, where ordering costs more than the cutoffs it finds.  Items share no bounds, so an item's node
+// count depends on its root alone.
 constexpr int kSolveLevels = BZ_SOLVE_MAX_EMPTIES + 1;  // a level per disc placed; a pass stays on its level
 constexpr int kMoveSlots = 65;  // move values per root: 64 cells and the pass
 constexpr int kUnset = 127;     // a move value no item has bounded yet
 constexpr int64_t kSolveChunk = (int64_t)1 << 22;  // roots per set of launches: at most 380 items each fit 32-bit offsets
+#ifndef BZ_SOLVE_ORDER_EMPTIES
+#define BZ_SOLVE_ORDER_EMPTIES 6  // the fastest of T = 6, 8, 10, 12 and none at 12 and 14 empties (profiles/README.md)
+#endif
+constexpr int kOrderEmpties = BZ_SOLVE_ORDER_EMPTIES;
+// an item's first node has at most BZ_SOLVE_MAX_EMPTIES - 1 empties, so levels below this hold every ordered node
+constexpr int kOrderLevels = BZ_SOLVE_MAX_EMPTIES - kOrderEmpties > 0 ? BZ_SOLVE_MAX_EMPTIES - kOrderEmpties : 1;
+constexpr int kOrderMoves = BZ_SOLVE_MAX_EMPTIES;  // a move per empty square at most
 
 // the k-th move of a root whose legal moves are m (the pass when m == 0): its action and child, mover-relative
 __device__ __forceinline__ unsigned root_move(uint64_t me, uint64_t opp, uint64_t m, int k, uint64_t &cme, uint64_t &copp) {
@@ -321,9 +337,23 @@ __device__ __forceinline__ int solve_empties(uint64_t me, uint64_t opp, uint64_t
     return __popcll(cells) - __popcll((me | opp) & cells);
 }
 
+// fastest first: the moves m of (me, opp) as keys (the opponent's legal-move count after the move) << 6 | cell, in
+// ascending order (ties in cell order); the ordering's positions are not counted as nodes
+__device__ __forceinline__ void order_moves(uint64_t me, uint64_t opp, uint64_t m, uint64_t cells, uint16_t *keys) {
+    for (int n = 0; m; m &= m - 1, ++n) {
+        const unsigned a = (unsigned)(__ffsll((long long)m) - 1);
+        uint64_t cme = me, copp = opp;
+        apply_legal(cme, copp, a);
+        const unsigned key = (unsigned)__popcll(legal_mask(cme, copp, cells)) << 6 | a;
+        int j = n;
+        for (; j > 0 && keys[j - 1] > key; --j) keys[j] = keys[j - 1];
+        keys[j] = (uint16_t)key;
+    }
+}
+
 // kLive: the roots are [0, *live) of n (the self-play endgame queue: launch shapes depend on n only); the others get
-// no items
-template <bool kLive>
+// no items.  kWld: a finished root's value is the sign of its disc difference.
+template <bool kLive, bool kWld>
 __global__ void __launch_bounds__(256) endgame_prep_kernel(const uint64_t *me_, const uint64_t *opp_, int64_t n,
                                                            uint64_t cells, Workspace W, uint8_t *action, int8_t *value,
                                                            const int32_t *live) {
@@ -344,7 +374,8 @@ __global__ void __launch_bounds__(256) endgame_prep_kernel(const uint64_t *me_, 
     const uint64_t m = legal_mask(me, opp, cells);
     if (!fits || (m == 0 && legal_mask(opp, me, cells) == 0)) {  // not searched, or the game is over
         action[i] = 255u;
-        value[i] = (int8_t)(fits ? __popcll(me) - __popcll(opp) : 0);
+        const int d = __popcll(me) - __popcll(opp);
+        value[i] = (int8_t)(fits ? (kWld ? (d > 0) - (d < 0) : d) : 0);
         nd = fits;
     } else {
         const int moves = m ? __popcll(m) : 1;
@@ -361,6 +392,7 @@ __global__ void __launch_bounds__(256) endgame_prep_kernel(const uint64_t *me_, 
     W.offset[i] = cnt;
 }
 
+template <bool kWld>
 __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const uint64_t *me_, const uint64_t *opp_,
                                                                         int64_t n, uint64_t cells, Workspace W) {
     const unsigned total = W.counter[1];
@@ -369,6 +401,10 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
     // must pass is held as the position after the pass, with bit k of `passed` set and its window negated
     uint64_t s_me[kSolveLevels], s_opp[kSolveLevels], s_rem[kSolveLevels];
     int s_best[kSolveLevels], s_alpha[kSolveLevels], s_beta[kSolveLevels];
+    // kWld: a level with bit k of `ordered` set descends in the order of s_order[k] (order_moves' keys), from s_cur[k]
+    uint16_t s_order[kOrderLevels][kOrderMoves];
+    uint8_t s_cur[kOrderLevels];
+    unsigned ordered = 0;
     unsigned passed = 0;
     int k = -1;  // level of the node being searched; -1: no item
     int v = 0;
@@ -405,6 +441,14 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
         s_best[k] = -kWindow;
         s_alpha[k] = alpha;
         s_beta[k] = beta;
+        if constexpr (kWld) {
+            ordered &= ~(1u << k);
+            if (k < kOrderLevels && solve_empties(me, opp, cells) >= kOrderEmpties) {
+                order_moves(me, opp, m, cells, s_order[k]);
+                s_cur[k] = 0;
+                ordered |= 1u << k;
+            }
+        }
         leaf = false;
     };
 
@@ -426,18 +470,22 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
                 r -= c;
             }
             BZ_CHECK(r < (cm ? (unsigned)__popcll(cm) : 1u), 71);  // reply
+            constexpr int w = kWld ? 1 : kWindow;  // the null window, or the full one
             if (cm) {
                 apply_legal(cme, copp, kth_bit(cm, (int)r));
-                enter(cme, copp, -kWindow, kWindow);
+                enter(cme, copp, -w, w);
             } else if (legal_mask(copp, cme, cells)) {
-                enter(copp, cme, -kWindow, kWindow);  // the child passes: the item is the position after the pass
+                enter(copp, cme, -w, w);  // the child passes: the item is the position after the pass
             } else {
                 v = __popcll(copp) - __popcll(cme);  // the child's game is over: the root mover's count
                 leaf = true;
             }
-        } else if (!leaf) {  // descend into the next move of level k, row-major
+        } else if (!leaf) {  // descend into the next move of level k: row-major, or in the level's order
             const uint64_t rem = s_rem[k];
-            const uint64_t x = rem & (0ull - rem);
+            uint64_t x = rem & (0ull - rem);
+            if constexpr (kWld) {
+                if ((ordered >> k) & 1u) x = 1ull << (s_order[k][s_cur[k]++] & 63u);
+            }
             s_rem[k] = rem ^ x;
             uint64_t me = s_me[k], opp = s_opp[k];
             apply_legal(me, opp, (unsigned)(__ffsll((long long)x) - 1));
@@ -452,6 +500,7 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
             if (k == 0) {
                 // the item's first node belongs to the root's mover: a move's value is its items' minimum
                 BZ_CHECK(root * kMoveSlots + move < n * kMoveSlots, 73);  // move value slot
+                if constexpr (kWld) v = v > 1 ? 1 : (v < -1 ? -1 : v);  // a bound beyond the null window: its sign
                 atomicMin(&mv[root * kMoveSlots + move], v);
                 if (nodes) atomicAdd(&W.nodes[root], nodes);
                 k = -1;
@@ -532,20 +581,29 @@ int64_t endgame_workspace_bytes(int64_t n) {
     return 16 + align16(4 * (c + 1)) + align16(8 * c) + align16(4 * kMoveSlots * c);
 }
 
+// the solver's four launches over n <= kSolveChunk roots (live: the roots [0, *live), see endgame_prep_kernel)
+template <bool kLive, bool kWld>
+void endgame_kernels(const uint64_t *me, const uint64_t *opp, int64_t n, const int32_t *live, uint64_t cells,
+                     const Workspace &W, uint8_t *action, int8_t *value, int8_t *move_value, int64_t *nodes,
+                     cudaStream_t stream) {
+    const unsigned blocks = (unsigned)((n + 255) / 256);
+    endgame_prep_kernel<kLive, kWld><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, live);
+    minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, n);  // the roots past *live have no items: no item maps to them
+    endgame_search_kernel<kWld><<<persistent_grid(n * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me, opp, n,
+                                                                                                         cells, W);
+    endgame_finish_kernel<kLive><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, move_value, nodes,
+                                                             live);
+}
+
 int endgame_launch(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
-                   int8_t *value, int8_t *move_value, int64_t *nodes, cudaStream_t stream) {
+                   int8_t *value, int8_t *move_value, int64_t *nodes, bool wld, cudaStream_t stream) {
     const uint64_t cells = cell_mask(size);
     for (int64_t b = 0; b < n; b += kSolveChunk) {  // stream order makes the chunks' reuse of the workspace safe
         const int64_t c = n - b < kSolveChunk ? n - b : kSolveChunk;
         const Workspace W = carve(workspace, c);
-        const unsigned blocks = (unsigned)((c + 255) / 256);
-        endgame_prep_kernel<false><<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b, nullptr);
-        minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, c);
-        endgame_search_kernel<<<persistent_grid(c * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me + b, opp + b, c,
-                                                                                                         cells, W);
-        endgame_finish_kernel<false><<<blocks, 256, 0, stream>>>(me + b, opp + b, c, cells, W, action + b, value + b,
-                                                                 move_value + b * kMoveSlots, nodes ? nodes + b : nullptr,
-                                                                 nullptr);
+        (wld ? endgame_kernels<false, true> : endgame_kernels<false, false>)(
+            me + b, opp + b, c, nullptr, cells, W, action + b, value + b, move_value + b * kMoveSlots,
+            nodes ? nodes + b : nullptr, stream);
         const int rc = launch_rc();
         if (rc != BZ_OK) return rc;
     }
@@ -553,15 +611,11 @@ int endgame_launch(const uint64_t *me, const uint64_t *opp, int64_t n, int size,
 }
 
 int endgame_launch_live(const uint64_t *me, const uint64_t *opp, int64_t n, const int32_t *live, int size, void *workspace,
-                        uint8_t *action, int8_t *value, int8_t *move_value, cudaStream_t stream) {
+                        uint8_t *action, int8_t *value, int8_t *move_value, bool wld, cudaStream_t stream) {
     if (n <= 0 || n > kSolveChunk) return BZ_ERR_ARG;
-    const uint64_t cells = cell_mask(size);
     const Workspace W = carve(workspace, n);
-    const unsigned blocks = (unsigned)((n + 255) / 256);
-    endgame_prep_kernel<true><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, live);
-    minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, n);  // the roots past *live have no items: no item maps to them
-    endgame_search_kernel<<<persistent_grid(n * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me, opp, n, cells, W);
-    endgame_finish_kernel<true><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, move_value, nullptr, live);
+    (wld ? endgame_kernels<true, true> : endgame_kernels<true, false>)(me, opp, n, live, cell_mask(size), W, action,
+                                                                       value, move_value, nullptr, stream);
     return launch_rc();
 }
 
@@ -591,13 +645,23 @@ int bz_minimax_moves(const uint64_t *me, const uint64_t *opp, const uint8_t *dep
 
 int64_t bz_endgame_workspace_bytes(int64_t n) { return endgame_workspace_bytes(n); }
 
-int bz_endgame_solve(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
-                     int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream) {
+static int endgame_solve(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
+                         int8_t *value, int8_t *move_value, int64_t *nodes, bool wld, bz_stream_t stream) {
     if (!(size == 4 || size == 6 || size == 8) || n < 0 || n >= (int64_t)1 << 25) return BZ_ERR_ARG;
     if (n == 0) return BZ_OK;
     if (!me || !opp || !workspace || !action || !value || !move_value) return BZ_ERR_ARG;
     if (!aligned16(workspace)) return BZ_ERR_UNALIGNED;
-    return endgame_launch(me, opp, n, size, workspace, action, value, move_value, nodes, as_stream(stream));
+    return endgame_launch(me, opp, n, size, workspace, action, value, move_value, nodes, wld, as_stream(stream));
+}
+
+int bz_endgame_solve(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
+                     int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream) {
+    return endgame_solve(me, opp, n, size, workspace, action, value, move_value, nodes, false, stream);
+}
+
+int bz_endgame_solve_wld(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
+                         int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream) {
+    return endgame_solve(me, opp, n, size, workspace, action, value, move_value, nodes, true, stream);
 }
 
 }  // extern "C"

@@ -30,10 +30,11 @@ int64_t minimax_workspace_bytes(int64_t n);
 // value and nodes (per root) and nodes_total (one int64, added to) may be null
 int64_t endgame_workspace_bytes(int64_t n);
 
-// bz_endgame_solve of the roots [0, *live) of n <= 2^22 (device count; the launch shapes depend on n only): action, value
-// and move_value are written for those roots alone.  workspace: endgame_workspace_bytes(n) bytes.
+// bz_endgame_solve (wld: bz_endgame_solve_wld) of the roots [0, *live) of n <= 2^22 (device count; the launch shapes
+// depend on n only): action, value and move_value are written for those roots alone.  workspace:
+// endgame_workspace_bytes(n) bytes.
 int endgame_launch_live(const uint64_t *me, const uint64_t *opp, int64_t n, const int32_t *live, int size, void *workspace,
-                        uint8_t *action, int8_t *value, int8_t *move_value, cudaStream_t stream);
+                        uint8_t *action, int8_t *value, int8_t *move_value, bool wld, cudaStream_t stream);
 
 int minimax_launch(const MinimaxRoots &roots, uint64_t seed, int size, void *workspace, uint8_t *action, int8_t *value,
                    int64_t *nodes, int64_t *nodes_total, cudaStream_t stream);

@@ -763,8 +763,8 @@ int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap) {
            endgame_play_align16(cap * A);
 }
 
-int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
-                             bz_stream_t stream) {
+static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace, bool wld,
+                        bz_stream_t stream) {
     int rc = check_state(st);
     if (rc != BZ_OK) return rc;
     rc = check_endgame(st, eg);
@@ -779,7 +779,8 @@ int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endg
     const cudaStream_t s = as_stream(stream);
     const uint64_t cells = cell_mask(st->board_size);
     for (int k = 0; k < 2 * eg->empties; ++k) {
-        rc = endgame_launch_live(eg->me, eg->opp, cap, eg->count, st->board_size, workspace, action, value, move_value, s);
+        rc = endgame_launch_live(eg->me, eg->opp, cap, eg->count, st->board_size, workspace, action, value, move_value, wld,
+                                 s);
         if (rc != BZ_OK) return rc;
         endgame_ply_kernel<<<(unsigned)((cap + kWarpsPerCta - 1) / kWarpsPerCta), kThreads, 0, s>>>(*st, *eg, action, value,
                                                                                                     move_value, cells);
@@ -788,6 +789,16 @@ int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endg
         if (rc != BZ_OK) return rc;
     }
     return BZ_OK;
+}
+
+int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
+                             bz_stream_t stream) {
+    return endgame_play(st, eg, workspace, false, stream);
+}
+
+int bz_selfplay_endgame_play_wld(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
+                                 bz_stream_t stream) {
+    return endgame_play(st, eg, workspace, true, stream);
 }
 
 int bz_match_init(const bz_match_state *st, bz_stream_t stream) {

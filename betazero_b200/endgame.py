@@ -14,6 +14,10 @@ search (the most visited move, lowest id on ties: the rule of matches), per budg
 next to the random player's expected scores (exact, from the move values) and ``Minimax(d)``'s moves
 (``minimax.best_moves``).  No opponent and no game noise: with a fixed seed a number means the same in every run.
 
+A win/draw/loss suite (``Suite.wld``, ``--wld``) is solved by ``minimax.solve(wld=True)``: its move values are only
+signs, so every move score is ``wld_accuracy`` alone (``move_accuracy`` and ``mean_disc_loss`` are absent); the value
+metrics use only signs and are those of the exact suite.
+
     python -m betazero_b200.endgame A.pt B.pt --empties 12 --positions 4096 --sims 0,800 --minimax 2,4
 """
 from __future__ import annotations
@@ -33,12 +37,14 @@ GAMES_PER_BATCH = 4096  # random games played side by side while a suite is draw
 @dataclass
 class Suite:
     """mover-relative positions (int64 CUDA tensors of uint64 bitboards) and, once ``solve_suite`` ran, the solver's
-    results: value int8 [n], move_value int8 [n, 65], nodes int64 [n] (numpy), and the solve's time"""
+    results: value int8 [n], move_value int8 [n, 65], nodes int64 [n] (numpy), and the solve's time.  ``wld``: solve
+    for win / draw / loss only (the values are signs)"""
     me: torch.Tensor
     opp: torch.Tensor
     size: int
     empties: int
     seed: int
+    wld: bool = False
     value: np.ndarray | None = None
     move_value: np.ndarray | None = None
     nodes: np.ndarray | None = None
@@ -100,12 +106,12 @@ def positions(n: int, empties: int, size: int = 8, seed: int = 0, device="cuda")
 
 
 def solve_suite(suite: Suite) -> Suite:
-    """fills the suite's exact values (once; a solved suite is returned as it is)"""
+    """fills the suite's exact (or, ``suite.wld``, win/draw/loss) values (once; a solved suite is returned as it is)"""
     if suite.move_value is not None:
         return suite
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    _, v, mv, nodes = minimax.solve(suite.me, suite.opp, suite.size)
+    _, v, mv, nodes = minimax.solve(suite.me, suite.opp, suite.size, wld=suite.wld)
     e1.record()
     torch.cuda.synchronize()
     suite.solve_ms = e0.elapsed_time(e1)
@@ -113,26 +119,31 @@ def solve_suite(suite: Suite) -> Suite:
     return suite
 
 
-def move_metrics(move_value: np.ndarray, value: np.ndarray, played: np.ndarray) -> dict:
-    """accuracy of the played moves (cell ids) against the exact move values"""
+def move_metrics(move_value: np.ndarray, value: np.ndarray, played: np.ndarray, wld: bool = False) -> dict:
+    """accuracy of the played moves (cell ids) against the exact move values (``wld``: against their signs, so only
+    ``wld_accuracy``)"""
     mv = move_value.astype(np.int64)
     best = value.astype(np.int64)
     pv = mv[np.arange(len(played)), np.asarray(played, np.int64)]
     if (pv == -128).any():
         raise ValueError("a played move is not legal")
-    return {"move_accuracy": float(np.mean(pv == best)), "wld_accuracy": float(np.mean(np.sign(pv) == np.sign(best))),
-            "mean_disc_loss": float(np.mean(best - pv))}
+    out = {"wld_accuracy": float(np.mean(np.sign(pv) == np.sign(best)))}
+    if not wld:
+        out = {"move_accuracy": float(np.mean(pv == best)), **out, "mean_disc_loss": float(np.mean(best - pv))}
+    return out
 
 
-def random_metrics(move_value: np.ndarray, value: np.ndarray) -> dict:
-    """the random player's expected scores: every legal move equally likely"""
+def random_metrics(move_value: np.ndarray, value: np.ndarray, wld: bool = False) -> dict:
+    """the random player's expected scores: every legal move equally likely (``wld``: ``wld_accuracy`` only)"""
     mv = move_value.astype(np.int64)
     best = value.astype(np.int64)[:, None]
     legal = mv != -128
     n_legal = legal.sum(1)
-    return {"move_accuracy": float(np.mean(((mv == best) & legal).sum(1) / n_legal)),
-            "wld_accuracy": float(np.mean(((np.sign(mv) == np.sign(best)) & legal).sum(1) / n_legal)),
-            "mean_disc_loss": float(np.mean(np.where(legal, best - mv, 0).sum(1) / n_legal))}
+    out = {"wld_accuracy": float(np.mean(((np.sign(mv) == np.sign(best)) & legal).sum(1) / n_legal))}
+    if not wld:
+        out = {"move_accuracy": float(np.mean(((mv == best) & legal).sum(1) / n_legal)), **out,
+               "mean_disc_loss": float(np.mean(np.where(legal, best - mv, 0).sum(1) / n_legal))}
+    return out
 
 
 def value_metrics(head: np.ndarray, value: np.ndarray) -> dict:
@@ -170,10 +181,11 @@ def evaluate(net, suite: Suite, sims=(0, 800), n_leaves: int = 4, minimax_depths
         s = int(s)
         if s == 0:
             played, head = raw_policy(net, suite.me, suite.opp, suite.size)
-            r = move_metrics(suite.move_value, suite.value, played)
+            r = move_metrics(suite.move_value, suite.value, played, suite.wld)
             r.update(value_metrics(head, suite.value))
         else:
-            r = move_metrics(suite.move_value, suite.value, searched_moves(net, suite.me, suite.opp, s, n_leaves, suite.size))
+            r = move_metrics(suite.move_value, suite.value, searched_moves(net, suite.me, suite.opp, s, n_leaves, suite.size),
+                             suite.wld)
         out["budgets"][str(s)] = r
     out["baselines"] = baselines(suite, minimax_depths)
     return out
@@ -181,17 +193,18 @@ def evaluate(net, suite: Suite, sims=(0, 800), n_leaves: int = 4, minimax_depths
 
 def baselines(suite: Suite, minimax_depths=()) -> dict:
     solve_suite(suite)
-    out = {"random": random_metrics(suite.move_value, suite.value)}
+    out = {"random": random_metrics(suite.move_value, suite.value, suite.wld)}
     keys = torch.arange(len(suite), dtype=torch.int64, device=suite.me.device)
     for d in minimax_depths:
         a, _, _ = minimax.best_moves(suite.me, suite.opp, int(d), suite.size, seed=suite.seed, keys=keys)
-        out[f"minimax{int(d)}"] = move_metrics(suite.move_value, suite.value, a.long().cpu().numpy())
+        out[f"minimax{int(d)}"] = move_metrics(suite.move_value, suite.value, a.long().cpu().numpy(), suite.wld)
     return out
 
 
 def solve_stats(suite: Suite) -> dict:
     solve_suite(suite)
-    return {"ms": suite.solve_ms, "nodes": int(suite.nodes.sum()), "max_nodes": int(suite.nodes.max())}
+    return {"solve": "wld" if suite.wld else "exact", "ms": suite.solve_ms, "nodes": int(suite.nodes.sum()),
+            "max_nodes": int(suite.nodes.max())}
 
 
 def main(argv=None):
@@ -204,6 +217,8 @@ def main(argv=None):
     ap.add_argument("--size", type=int, default=8)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--leaves", type=int, default=4, help="virtual-loss descents per tree and iteration of the search")
+    ap.add_argument("--wld", action="store_true", help="solve for win / draw / loss only (cheaper; the move scores are "
+                                                       "wld_accuracy alone)")
     args = ap.parse_args(argv)
     from . import train
 
@@ -211,7 +226,9 @@ def main(argv=None):
     depths = [minimax.check_depth(x) for x in args.minimax.split(",") if x.strip()]
     if args.empties > minimax.SOLVE_MAX_EMPTIES:
         raise SystemExit(f"--empties must be at most {minimax.SOLVE_MAX_EMPTIES}")
-    suite = solve_suite(positions(args.positions, args.empties, args.size, args.seed))
+    suite = positions(args.positions, args.empties, args.size, args.seed)
+    suite.wld = args.wld
+    solve_suite(suite)
     out = {"size": args.size, "empties": args.empties, "positions": len(suite), "seed": args.seed, "leaves": args.leaves,
            "solve": solve_stats(suite), "baselines": baselines(suite, depths), "checkpoints": {}}
     for path in args.checkpoints:

@@ -18,7 +18,9 @@ empty squares against the exact solver (``betazero_b200.endgame``), at 0 simulat
 adds ``eval_endgame``; the suite is drawn and solved once per run.  With ``--endgame-empties E`` self-play hands every game to
 the exact solver once a searched move leaves at most E empty squares, and runs a solver phase every ``--endgame-every``
 plies (``selfplay.BatchedSelfPlay``); the line then has an ``endgame`` entry with the solver's counts and the time of its
-phases.
+phases.  ``--endgame-solve wld`` runs the win/draw/loss solver for both instead of the exact one (cheaper; the handover's
+pi is then uniform over the moves that keep the result, and ``eval_endgame`` reports ``wld_accuracy`` only); both
+entries name the solver.
 """
 from __future__ import annotations
 
@@ -40,7 +42,8 @@ def default_args(**over) -> SimpleNamespace:
     """the command line's defaults as a namespace (for callers that drive iterations from Python: bench.py, tests)"""
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
-                        reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None, endgame_empties=0, endgame_every=8)
+                        reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None, endgame_empties=0, endgame_every=8,
+                        endgame_solve="exact")
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -65,13 +68,16 @@ class LoopState:
             minimax.check_depth(em)
             if eg == 0:
                 raise ValueError("eval_minimax plays --eval-games games: set eval_games > 0")
+        solve = selfplay.check_endgame_solve(getattr(args, "endgame_solve", "exact"))
         self.endgame_suite = None  # --eval-endgame: drawn and solved once per run (rank 0)
         ee = getattr(args, "eval_endgame", None)
         if ee is not None:
             if not 1 <= int(ee) <= minimax.SOLVE_MAX_EMPTIES:
                 raise ValueError(f"eval_endgame must be in 1 .. {minimax.SOLVE_MAX_EMPTIES} empty squares; got {ee}")
             if rank == 0:
-                self.endgame_suite = endgame.solve_suite(endgame.positions(ENDGAME_POSITIONS, int(ee), args.size, args.seed))
+                self.endgame_suite = endgame.positions(ENDGAME_POSITIONS, int(ee), args.size, args.seed)
+                self.endgame_suite.wld = solve == "wld"
+                endgame.solve_suite(self.endgame_suite)
         self.model = net.make_net(args.net, hidden=args.hidden, seed=args.seed)
         self.master = net.make_net(args.net, hidden=args.hidden, seed=args.seed, dtype=torch.float32)  # fp32 master weights
         self.opt = torch.optim.Adam(self.master.parameters(), lr=args.lr)  # the reference's optimiser family (SL/train.py:87)
@@ -86,7 +92,7 @@ class LoopState:
                                            n_leaves=args.leaves, reuse=bool(getattr(args, "reuse", False)),
                                            graph_unroll=min(16, max(1, args.sims // args.leaves - 1)),
                                            endgame_empties=int(getattr(args, "endgame_empties", 0)),
-                                           endgame_every=int(getattr(args, "endgame_every", 8)))
+                                           endgame_every=int(getattr(args, "endgame_every", 8)), endgame_solve=solve)
         self.sp.prepare()
 
     @torch.no_grad()
@@ -160,7 +166,7 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["replay_gather"]["busbw_GBps"] = gather_info["gathered_bytes"] * (world - 1) / world / sec / 1e9
         line["weight_broadcast_busbw_GBps"] = nbytes / (ms["weight_broadcast"] * 1e-3) / 1e9
     if sp.eg is not None:
-        line["endgame"] = {"empties": sp.endgame_empties, "every": sp.endgame_every,
+        line["endgame"] = {"solve": sp.endgame_solve, "empties": sp.endgame_empties, "every": sp.endgame_every,
                            "games": stats["endgame_games"] - eg_stats0["endgame_games"],
                            "plies": stats["endgame_plies"] - eg_stats0["endgame_plies"],
                            "pending": stats["endgame_pending"],
@@ -183,7 +189,8 @@ def run_iteration(st: LoopState, it: int) -> dict:
     if st.endgame_suite is not None:
         t_eval = time.perf_counter()
         r = endgame.evaluate(st.model, st.endgame_suite, (0, args.sims), args.leaves)
-        line["eval_endgame"] = {"empties": r["empties"], "positions": r["positions"], "budgets": r["budgets"],
+        line["eval_endgame"] = {"solve": "wld" if st.endgame_suite.wld else "exact", "empties": r["empties"],
+                                "positions": r["positions"], "budgets": r["budgets"],
                                 "random": r["baselines"]["random"], "ms": (time.perf_counter() - t_eval) * 1e3}
     if caught:
         line["warnings"] = [str(w.message) for w in caught]
@@ -243,6 +250,9 @@ def main():
                          "empty squares (1 .. 20; 0 = off): perfect play and exact z labels for the end of every game")
     ap.add_argument("--endgame-every", type=int, default=d.endgame_every, metavar="K",
                     help="with --endgame-empties: run a solver phase on the queued games every K plies")
+    ap.add_argument("--endgame-solve", choices=selfplay.ENDGAME_SOLVES, default=d.endgame_solve,
+                    help="the solver of --endgame-empties and --eval-endgame: exact (the final margin) or wld (win / "
+                         "draw / loss only: cheaper; handover pi uniform over the moves that keep the result)")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

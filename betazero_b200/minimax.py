@@ -5,7 +5,8 @@ is oracle/minimax_ref.py, the semantics are in include/betazero_b200.h).
     action, value, nodes = best_moves(me, opp, depth=4, size=8, seed=0, keys=game_keys)
 
 ``solve`` is the exact endgame solver (``bz_endgame_solve``): the perfect player's move and every move's final disc
-difference for positions with at most 20 empty squares.
+difference for positions with at most 20 empty squares.  ``wld=True`` asks only for win, draw or loss
+(``bz_endgame_solve_wld``): the signs of those values, from a cheaper search.
 
     action, value, move_value, nodes = solve(me, opp, size=8)
 """
@@ -68,14 +69,19 @@ def best_moves(me: torch.Tensor, opp: torch.Tensor, depth, size: int = 8, seed: 
 SOLVE_MAX_EMPTIES = 20  # BZ_SOLVE_MAX_EMPTIES
 
 
-def solve(me: torch.Tensor, opp: torch.Tensor, size: int = 8):
+def solve(me: torch.Tensor, opp: torch.Tensor, size: int = 8, wld: bool = False):
     """The exact endgame value of every mover-relative root (me, opp: int64 CUDA tensors holding uint64 bitboards) with
     at most 20 empty squares (``bz_endgame_solve``; the definition is oracle/endgame_ref.py).
 
     Returns CUDA tensors (action uint8 [n]: the first best move, row*8 + col, 64 = a forced pass, 255 = game over;
     value int8 [n]: the final disc difference for the mover under perfect play, empty squares to nobody; move_value int8
     [n, 65]: the value of every legal move for the mover, the pass at 64, -128 for an action that is not legal; nodes
-    int64 [n]: positions the search entered).  ``ValueError`` for a root with more than 20 empties (one device read)."""
+    int64 [n]: positions the search entered).  ``ValueError`` for a root with more than 20 empties (one device read).
+
+    ``wld=True`` (``bz_endgame_solve_wld``): win / draw / loss only -- value and move_value are the signs of the exact
+    ones (-128 still marks an action that is not legal), and action is the first move in cell order that keeps the
+    result (generally not the exact solve's action).  It searches a null window with fastest-first move ordering, so
+    it enters fewer nodes."""
     if size not in (4, 6, 8):
         raise ValueError("size must be 4, 6 or 8 (Reversi)")
     n = me.numel()
@@ -93,7 +99,7 @@ def solve(me: torch.Tensor, opp: torch.Tensor, size: int = 8):
     nodes = torch.empty(n, dtype=torch.int64, device=dev)
     L = _lib.load()
     ws = torch.empty(max(int(L.bz_endgame_workspace_bytes(n)), 16), dtype=torch.uint8, device=dev)
-    _lib.check(L.bz_endgame_solve(_lib.dptr(me), _lib.dptr(opp), n, int(size), _lib.dptr(ws), _lib.dptr(action),
-                                  _lib.dptr(value), _lib.dptr(move_value), _lib.dptr(nodes), _lib.stream_ptr()),
-               "bz_endgame_solve")
+    name = "bz_endgame_solve_wld" if wld else "bz_endgame_solve"
+    _lib.check(getattr(L, name)(_lib.dptr(me), _lib.dptr(opp), n, int(size), _lib.dptr(ws), _lib.dptr(action),
+                                _lib.dptr(value), _lib.dptr(move_value), _lib.dptr(nodes), _lib.stream_ptr()), name)
     return action, value, move_value, nodes

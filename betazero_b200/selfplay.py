@@ -12,7 +12,9 @@ Endgame handover (opt-in, ``endgame_empties=E``): a game whose searched move lea
 device-side queue and its slot restarts; every ``endgame_every`` plies the exact solver plays every queued game to its end
 (bz_selfplay_advance_endgame, bz_selfplay_endgame_play).  Its records up to the handover are those the game has without
 the feature, the solver's records carry pi uniform over the optimal moves, and every z is the exact outcome of the
-handover position.
+handover position.  ``endgame_solve="wld"`` hands the games to the win/draw/loss solver instead (bz_selfplay_endgame_play_wld):
+cheaper, with the same z, but pi is uniform over every move that keeps the result rather than over the moves that
+maximise the final margin -- a label with less information, which is why the exact solver stays the default.
 """
 from __future__ import annotations
 
@@ -26,6 +28,7 @@ from .mcts import BatchedMCTS, TreePools
 
 N_ACTIONS = 65
 SOLVE_MAX_EMPTIES = 20  # BZ_SOLVE_MAX_EMPTIES
+ENDGAME_SOLVES = ("exact", "wld")
 
 
 def check_endgame_empties(empties, board_size: int) -> int:
@@ -36,15 +39,23 @@ def check_endgame_empties(empties, board_size: int) -> int:
     return e
 
 
+def check_endgame_solve(solve) -> str:
+    """"exact" (bz_selfplay_endgame_play) or "wld" (bz_selfplay_endgame_play_wld)"""
+    if solve not in ENDGAME_SOLVES:
+        raise ValueError(f"endgame_solve must be one of {ENDGAME_SOLVES}; got {solve!r}")
+    return solve
+
+
 class BatchedSelfPlay:
     def __init__(self, n_games: int, n_sims: int, evaluator, board_size: int = 8, c_puct: float = 1.25,
                  temp_plies: int = 0, seed: int = 0, replay_cap: int | None = None, rank: int = 0, world: int = 1,
                  arena_units: int | None = None, use_graph: bool = True, graph_unroll: int = 16,
                  dirichlet_alpha: float = 0.0, dirichlet_eps: float = 0.25, n_leaves: int = 1, device="cuda",
                  one_launch: bool | None = None, reuse: bool = False, endgame_empties: int = 0, endgame_every: int = 8,
-                 endgame_cap: int | None = None):
+                 endgame_cap: int | None = None, endgame_solve: str = "exact"):
         self.n_games, self.n_sims, self.board_size = int(n_games), int(n_sims), int(board_size)
         self.endgame_empties = check_endgame_empties(endgame_empties, board_size)
+        self.endgame_solve = check_endgame_solve(endgame_solve)
         self.endgame_every = int(endgame_every)
         if self.endgame_every < 1:
             raise ValueError(f"endgame_every must be >= 1; got {endgame_every}")
@@ -149,15 +160,15 @@ class BatchedSelfPlay:
             self.endgame_play()
 
     def endgame_play(self) -> None:
-        """One solver phase: every game in the endgame queue is played to its end by the exact solver and flushed to the
-        replay buffer (a fixed number of launches, no host synchronisation).  ``advance`` calls it every
-        ``endgame_every`` plies."""
+        """One solver phase: every game in the endgame queue is played to its end by the exact solver (or the
+        win/draw/loss solver, ``endgame_solve="wld"``) and flushed to the replay buffer (a fixed number of launches, no
+        host synchronisation).  ``advance`` calls it every ``endgame_every`` plies."""
         if self.eg is None:
             raise RuntimeError("endgame_play needs endgame_empties > 0")
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
-        _lib.check(self._L.bz_selfplay_endgame_play(self._ref, self._eg_ref, _lib.dptr(self.eg_workspace),
-                                                    _lib.stream_ptr()), "bz_selfplay_endgame_play")
+        name = "bz_selfplay_endgame_play_wld" if self.endgame_solve == "wld" else "bz_selfplay_endgame_play"
+        _lib.check(getattr(self._L, name)(self._ref, self._eg_ref, _lib.dptr(self.eg_workspace), _lib.stream_ptr()), name)
         t1.record()
         self._eg_events.append((t0, t1))
         self.launches += 6 * 2 * self.endgame_empties  # per solver ply: the solve's four kernels, the move, the compaction

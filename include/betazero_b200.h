@@ -390,6 +390,12 @@ int bz_selfplay_advance_endgame(const bz_selfplay_state *st, const bz_selfplay_e
  * workspace: bz_selfplay_endgame_workspace_bytes(cap) bytes, 16-byte aligned. */
 int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
                              bz_stream_t stream);
+/* bz_selfplay_endgame_play with the win/draw/loss solve (bz_endgame_solve_wld): the move is the first move that keeps
+ * the result, and pi is 1/k on each of the k moves that keep it (not on the moves that maximise the final margin).
+ * Every z equals the z of bz_selfplay_endgame_play: the sign of the handover position's exact value.  Same state,
+ * workspace and refusals. */
+int bz_selfplay_endgame_play_wld(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
+                                 bz_stream_t stream);
 int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap);
 
 /* ------------------------------------------------------------------------------------------
@@ -512,6 +518,16 @@ int64_t bz_minimax_workspace_bytes(int64_t n);
 int bz_endgame_solve(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
                      int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream);
 int64_t bz_endgame_workspace_bytes(int64_t n);
+/* Win/draw/loss solve: the signs of bz_endgame_solve's results, not the final margin (the definition is solve_wld in
+ * oracle/endgame_ref.py).  move_value: sign(-value(child)) in {-1, 0, 1} of every legal move, -128 for an action that
+ * is not legal; value[i]: their maximum, or the sign of the disc difference of a finished game; action[i]: the first
+ * move in cell order whose sign is the value (the reference's strict ">" on the signs; generally not bz_endgame_solve's
+ * action), 64 when the mover must pass, 255 when the game is over; nodes: as for bz_endgame_solve, at most plain
+ * negamax's count.  The search is alpha-beta with the null window (-1, 1) on the same items, with the moves of nodes
+ * that have many empty squares tried fastest first (fewest legal replies for the opponent).  Same arguments, workspace,
+ * refusals and treatment of roots with too many empties as bz_endgame_solve. */
+int bz_endgame_solve_wld(const uint64_t *me, const uint64_t *opp, int64_t n, int size, void *workspace, uint8_t *action,
+                         int8_t *value, int8_t *move_value, int64_t *nodes, bz_stream_t stream);
 
 /* Philox4x32-10 of (seed, game_id, ply): the u32 the move sampler draws (for tests). */
 int bz_philox_u32(uint64_t seed, const int64_t *game_id, const int32_t *ply, uint32_t *out, int64_t n,
