@@ -1,9 +1,10 @@
-// The policy/value MLP of mlp.cu on CTA PAIRS: tcgen05.mma.cta_group::2, all weights resident in shared memory.
+// The policy/value MLP on CTA PAIRS (pair_net.cuh): tcgen05.mma.cta_group::2, all weights resident in shared memory.
 //
-// Why a second kernel: at the self-play batch (4096 leaves) the net is a latency chain, not a throughput problem.
-// With one CTA per 128 leaves (mlp.cu) a hidden layer costs 16 MMAs x 128 clk (M = 128, N = 256 on one SM) plus
-// the epilogue of 128 x 256 accumulators (bias, ReLU, bf16, swizzled st.shared: ~1 us), and the next layer's 128 KB of
-// weights can only be fetched once the previous ones have been consumed (they do not fit beside the activations).
+// Why pairs: at the self-play batch (4096 leaves) the net is a latency chain, not a throughput problem.  With one CTA
+// per 128 leaves (profiles/experiments/mlp_onecta.cu) a hidden layer costs 16 MMAs x 128 clk (M = 128, N = 256 on one
+// SM) plus the epilogue of 128 x 256 accumulators (bias, ReLU, bf16, swizzled st.shared: ~1 us), and the next layer's
+// 128 KB of weights can only be fetched once the previous ones have been consumed (they do not fit beside the
+// activations).
 // Two CTAs of a cluster sharing one 128-leaf tile halve all three terms:
 //   * the pair executes ONE M = 128, N = 256 MMA per K step (64 leaves per SM): 64 clk instead of 128;
 //   * each SM converts only its own 64 x 256 accumulators;
@@ -15,32 +16,12 @@
 //
 // TMEM layout of a cta_group::2, M = 128 accumulator (PTX ISA "Data path layout organisation", 2x2 atom): in each
 // CTA, row m (0..63) and column n live at lane m + 64 * (n / (N/2)), column n % (N/2).
-//
-// Numerics are those of mlp.cu (bf16 operands, fp32 accumulate, fp32 bias, ReLU, bf16 round per layer).
-#include <cuda_bf16.h>
-
-#include "common.cuh"
-#include "umma.cuh"
+#include "pair_net.cuh"
 
 namespace bz {
 namespace {
 
-constexpr int kPairRows = 128;   // leaves per CTA pair == UMMA M
-constexpr int kCtaRows = 64;     // leaves per CTA
-constexpr int kIn = 128;
-constexpr int kHidden = 256;
-constexpr int kHeadRows = 80;    // 65 logits + value, padded to a legal UMMA N
-constexpr int kOutStride = 72;
 constexpr int kThreads = 512;    // 16 warps: 4 per TMEM lane quadrant x 4 groups of 32 accumulator columns
-constexpr int kSlabA = kCtaRows * 128;            // one 64-element K slab of A: 64 rows x 128 B
-constexpr int kSmemA = 4 * kSlabA;                // 32 KB
-constexpr int kSlabW = (kHidden / 2) * 128;       // hidden layers: this CTA's 128 weight rows x 128 B
-constexpr int kSlabHead = (kHeadRows / 2) * 128;  // head: 40 rows x 128 B
-constexpr int kW0 = 2 * kSlabW, kW1 = 4 * kSlabW, kW2 = 4 * kSlabW, kW3 = 4 * kSlabHead;
-constexpr int kSmemW = kW0 + kW1 + kW2 + kW3;     // 180 KB: this CTA's half of every layer
-constexpr int kNumBias = 3 * kHidden + kHeadRows;
-constexpr int kSmemBias = kNumBias * 4;
-constexpr int kImgRank = kSmemW + kSmemBias;      // one rank's slice of the weight image: its weights, then all biases (fp32)
 constexpr int kSmemTotal = kSmemA + kSmemW + kSmemBias + 128 + 1024;
 constexpr int kTmemCols = 128;
 
@@ -52,13 +33,6 @@ __device__ long long g_pair_trace[64];
 #define PAIR_TRACE(i) do { } while (0)
 #define PAIR_TRACE2(i) do { } while (0)
 #endif
-
-struct PairParams {
-    const __nv_bfloat16 *x;   // [B, 128]
-    const uint8_t *wimg;      // [2 ranks][kImgRank]: each rank's half of W1, W2, W3, W_head in the shared-memory layout + all biases (fp32)
-    __nv_bfloat16 *out;       // [B, 72]
-    int B;
-};
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pair_kernel(const PairParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -79,8 +53,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);  // provably warp-uniform
     const int lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
-    const int row0 = (int)(blockIdx.x >> 1) * kPairRows + (int)rank * kCtaRows;
+    const int row0 = (int)(blockIdx.x >> 1) * kTileRows + (int)rank * kCtaRows;
     const int valid_rows = max(0, min(kCtaRows, p.B - row0));
+    const uint8_t *img = p.wimg + (size_t)rank * kImgRank;
 
     // ---- prologue: nothing here depends on the previous kernel (it overlaps its tail under PDL) ----
     if (warp == 0) {
@@ -96,11 +71,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         // First in the queue: what layer 0 needs (this CTA's half of W1, the biases).  An SM ingests ~64 B/clk from
         // L2, so the order of the copies is the order in which the layers can start.
-        const uint8_t *src = p.wimg + (size_t)rank * kImgRank;
-        mbar_expect_tx(bar0, kW0);
-        bulk_load(sW, src, kW0, bar0);
-        mbar_expect_tx(bias_bar, kSmemBias);
-        bulk_load(sW + kSmemW, src + kSmemW, kSmemBias, bias_bar);
+        load_layer(sW, img, 0, bar0);
+        load_biases(sW + kSmemW, img, bias_bar);
     }
 
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -110,21 +82,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
     pdl_wait();
     pdl_launch_dependents();
     PAIR_TRACE(1);
-    for (int i = threadIdx.x; i < kCtaRows * (kIn / 8); i += kThreads) {
-        const int r = i >> 4, c = i & 15;
-        const bool ok = r < valid_rows;
-        cp_async16(sA + (uint32_t)(c >> 3) * kSlabA + (uint32_t)r * 128u + (uint32_t)(((c & 7) ^ (r & 7)) << 4),
-                   p.x + (size_t)(ok ? row0 + r : 0) * kIn + c * 8, ok);
-    }
+    load_x_rows(sA, p.x, row0, p.B, threadIdx.x, kThreads);
     if (threadIdx.x == 32) {  // behind the x copies: this CTA's half of the other three layers, one bulk copy per layer
-        const uint8_t *src = p.wimg + (size_t)rank * kImgRank;
-        const uint32_t bytes[4] = {kW0, kW1, kW2, kW3};
-        uint32_t off = kW0;
-        for (int l = 1; l < 4; ++l) {
-            mbar_expect_tx(bar0 + 8u * l, bytes[l]);
-            bulk_load(sW + off, src + off, bytes[l], bar0 + 8u * l);
-            off += bytes[l];
-        }
+        for (int l = 1; l < 4; ++l) load_layer(sW + layer_off(l), img, l, bar0 + 8u * l);
     }
     PAIR_TRACE(25);
     cluster_wait();
@@ -137,14 +97,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
     const int q = warp & 3, g = warp >> 2;
     const int r = (q & 1) * 32 + lane;                                // accumulator row of this thread
     const uint32_t trow = tmem + ((uint32_t)(q * 32) << 16);          // TMEM lanes of this warp
-    constexpr uint32_t kDescLo = 1u << 16, kDescHi32 = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);  // umma_desc, as 32-bit halves
-    uint32_t woff = 0;
 
 #pragma unroll 1
     for (int layer = 0; layer < 4; ++layer) {
-        const int K = layer == 0 ? kIn : kHidden;
-        const int N = layer == 3 ? kHeadRows : kHidden;
-        const uint32_t slabW = layer == 3 ? kSlabHead : kSlabW;
         // this warp's part of the A operand (generic-proxy stores) -> visible to the tensor cores of the pair;
         // its accumulator reads of the previous layer are complete.  One arrival per warp on the leader's barrier.
         PAIR_TRACE2(31 + 4 * layer);
@@ -164,28 +119,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
             mbar_wait_cluster(ready_bar, (uint32_t)(layer & 1));
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             PAIR_TRACE(5 + 5 * layer);
-            const uint32_t idesc = umma_idesc(kPairRows, N);
-            const uint32_t elected = elect_one();
-            const uint32_t nk = (uint32_t)K / 16;
-            // ONE elected-thread region for the layer, descriptors as 32-bit halves: the compiler keeps and advances them
-            // in uniform registers (an `if (elected)` around every MMA costs ~7 R2UR moves per instruction)
-            if (elected) {
-                const uint32_t tmem_u = tmem;
-#pragma unroll 4
-                for (uint32_t k = 0; k < nk; ++k) {
-                    const uint32_t off = k >> 2, kk = (k & 3) * 32u;
-                    const uint32_t alo = kDescLo | (((sA + off * kSlabA + kk) >> 4) & 0x3FFFu);
-                    const uint32_t blo = kDescLo | (((sW + woff + off * slabW + kk) >> 4) & 0x3FFFu);
-                    umma_bf16_pair_lohi(tmem_u, alo, blo, kDescHi32, idesc, k > 0);
-                }
-                asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(mma_bar),
-                             "h"((uint16_t)3)
-                             : "memory");
-            }
+            pair_issue_layer(elect_one(), tmem, sA, sW + layer_off(layer), layer, mma_bar);
             __syncwarp();
             PAIR_TRACE(6 + 5 * layer);
         }
-        woff += (uint32_t)(K / 64) * slabW;
         if (layer == 0) mbar_wait(bias_bar, 0);
         const float *bias = sBias + layer * kHidden;
         // this thread's 32 accumulator columns: logical columns (q / 2) * 128 + g * 32 ..; their biases are fetched
@@ -204,21 +141,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
             uint32_t acc[32];
             tmem_ld32(trow + (uint32_t)(g * 32), acc);
             PAIR_TRACE2(30 + 4 * layer);
-            uint32_t packed[16];
 #pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                packed[2 * j] = pack_relu_bf16(add2(acc[4 * j], acc[4 * j + 1], bv[j].x, bv[j].y));
-                packed[2 * j + 1] = pack_relu_bf16(add2(acc[4 * j + 2], acc[4 * j + 3], bv[j].z, bv[j].w));
-            }
-            const uint32_t rowbase = sA + (uint32_t)(c0 >> 6) * kSlabA + (uint32_t)r * 128u;
-            const int j0 = (c0 & 63) >> 3;
-#pragma unroll
-            for (int qq = 0; qq < 4; ++qq) {
-                const uint32_t dst = rowbase + (uint32_t)(((j0 + qq) ^ (r & 7)) << 4);
-                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(packed[4 * qq]), "r"(packed[4 * qq + 1]),
-                             "r"(packed[4 * qq + 2]), "r"(packed[4 * qq + 3])
-                             : "memory");
-            }
+            for (int qq = 0; qq < 4; ++qq) st_shared_v4(a_chunk(sA, r, (c0 >> 3) + qq), hidden_chunk(acc + 8 * qq, bv + 2 * qq));
         } else {
             // head: N = 80 -> 40 TMEM columns per lane half; 72 output columns (65 logits, value, padding).
             // The cluster barrier that guards the TMEM release is signalled as soon as the accumulators are in
@@ -268,22 +192,6 @@ extern "C" int bz_mlp_pair_debug_trace(long long *host_out) {
 extern "C" int64_t bz_mlp_pair_image_bytes(void) { return 2 * (int64_t)kImgRank; }
 
 extern "C" int bz_mlp_forward_pair(const void *x_bf16, const void *weight_image_pair, void *out_bf16, int64_t n, bz_stream_t stream) {
-    if (n < 0 || (n && (!x_bf16 || !weight_image_pair || !out_bf16))) return BZ_ERR_ARG;
-    if (!aligned16(x_bf16) || !aligned16(weight_image_pair) || !aligned16(out_bf16)) return BZ_ERR_UNALIGNED;
-    if (n == 0) return BZ_OK;
     static bool configured[64] = {};
-    {
-        cudaError_t e = allow_dynamic_smem(mlp_pair_kernel, kSmemTotal, configured);
-        if (e != cudaSuccess) return cuda_rc(e);
-    }
-    PairParams p = {};
-    p.x = (const __nv_bfloat16 *)x_bf16;
-    p.wimg = (const uint8_t *)weight_image_pair;
-    p.out = (__nv_bfloat16 *)out_bf16;
-    p.B = (int)n;
-    const unsigned pairs = (unsigned)((n + kPairRows - 1) / kPairRows);
-    cudaError_t e = launch_kernel(mlp_pair_kernel, dim3(2 * pairs), dim3(kThreads), (size_t)kSmemTotal, as_stream(stream),
-                                  pdl_enabled(), p);
-    if (e != cudaSuccess) return cuda_rc(e);
-    return launch_rc();
+    return launch_pair_mlp(mlp_pair_kernel, kTileRows, kThreads, kSmemTotal, configured, x_bf16, weight_image_pair, out_bf16, n, stream);
 }

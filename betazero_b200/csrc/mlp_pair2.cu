@@ -14,32 +14,15 @@
 //   region A: layer 1's half (64 KB, fetched behind the input) -> after both tiles' layer-1 MMAs: the head's half (20 KB)
 // so every layer's weights are requested a full layer before they are needed.
 // Same weight image (bz_mlp_pair_image_bytes), numerics and results as bz_mlp_forward_pair.
-#include <cuda_bf16.h>
-
-#include "common.cuh"
-#include "umma.cuh"
+#include "pair_net.cuh"
 
 namespace bz {
 namespace {
 
-constexpr int kTileRows = 128;   // leaves per tile == UMMA M
-constexpr int kPairRows = 256;   // leaves per CTA pair (two tiles)
-constexpr int kCtaRows = 64;     // leaves per CTA and tile
-constexpr int kIn = 128;
-constexpr int kHidden = 256;
-constexpr int kHeadRows = 80;
-constexpr int kOutStride = 72;
+constexpr int kPairRows = 2 * kTileRows;  // leaves per CTA pair (two tiles)
 constexpr int kEpiWarps = 16;    // epilogue: 4 warps per TMEM lane quadrant x 4 groups of 32 accumulator columns
 constexpr int kThreads = (kEpiWarps + 2) * 32;  // + the control warp + the loader warp
-constexpr int kSlabA = kCtaRows * 128;            // one 64-element K slab of one tile's A operand: 64 rows x 128 B
-constexpr int kSmemA = 4 * kSlabA;                // 32 KB per tile
-constexpr int kSlabW = (kHidden / 2) * 128;
-constexpr int kSlabHead = (kHeadRows / 2) * 128;
-constexpr int kW0 = 2 * kSlabW, kW1 = 4 * kSlabW, kW2 = 4 * kSlabW, kW3 = 4 * kSlabHead;
 constexpr int kRegion = 4 * kSlabW;               // 64 KB: one recycled weight region
-constexpr int kNumBias = 3 * kHidden + kHeadRows;
-constexpr int kSmemBias = kNumBias * 4;
-constexpr int kImgRank = kW0 + kW1 + kW2 + kW3 + kSmemBias;  // the image of bz_mlp_forward_pair
 constexpr int kSmemTotal = 2 * kSmemA + 2 * kRegion + kSmemBias + 256 + 1024;
 constexpr int kTmemCols = 256;                    // 2 tiles x 128 columns
 
@@ -51,14 +34,7 @@ __device__ long long g_pair2_trace[96];
 #define P2_TRACE(i) do { } while (0)
 #endif
 
-struct Pair2Params {
-    const __nv_bfloat16 *x;
-    const uint8_t *wimg;
-    __nv_bfloat16 *out;
-    int B;
-};
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pair2_kernel(const Pair2Params p) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pair2_kernel(const PairParams p) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;  // identical in both CTAs: the MMA uses the leader's descriptors for both
@@ -105,10 +81,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
     // All bulk copies come from the loader WARP: a releasing remote arrive (control warp) otherwise waits for the bulk
     // copies its own warp has in flight (+0.8 us per handshake, whichever lane issued them).
     if (loader && lane == 0) {
-        mbar_expect_tx(bar0, kW0);  // layer 0's half -> region B, first in the queue
-        bulk_load(sRegB, wsrc, kW0, bar0);
-        mbar_expect_tx(bias_bar, kSmemBias);
-        bulk_load(sRegA + 2 * kRegion, wsrc + kW0 + kW1 + kW2 + kW3, kSmemBias, bias_bar);  // the bias array behind the regions
+        load_layer(sRegB, wsrc, 0, bar0);  // layer 0's half -> region B, first in the queue
+        load_biases(sRegA + 2 * kRegion, wsrc, bias_bar);  // the bias array behind the regions
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     cluster_arrive();  // both CTAs: barriers initialised, TMEM allocated; completes while the x copies are in flight
@@ -118,16 +92,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
     pdl_launch_dependents();
     if (warp < kEpiWarps) {
         // both tiles' rows of this CTA: tile t, rank r -> rows pair_row0 + t * 128 + r * 64 ..
-        for (int i = threadIdx.x; i < 2 * kCtaRows * (kIn / 8); i += kEpiWarps * 32) {
-            const int t = i >> 10, rr = (i >> 4) & 63, c = i & 15;
-            const int row = pair_row0 + t * kTileRows + (int)rank * kCtaRows + rr;
-            const bool ok = row < p.B;
-            cp_async16(sA + (uint32_t)t * kSmemA + (uint32_t)(c >> 3) * kSlabA + (uint32_t)rr * 128u + (uint32_t)(((c & 7) ^ (rr & 7)) << 4),
-                       p.x + (size_t)(ok ? row : 0) * kIn + c * 8, ok);
-        }
+        for (int t = 0; t < 2; ++t)
+            load_x_rows(sA + (uint32_t)t * kSmemA, p.x, pair_row0 + t * kTileRows + (int)rank * kCtaRows, p.B, threadIdx.x, kEpiWarps * 32);
     } else if (loader && lane == 0) {  // behind the x copies: layer 1's half -> region A
-        mbar_expect_tx(bar0 + 8u, kW1);
-        bulk_load(sRegA, wsrc + kW0, kW1, bar0 + 8u);
+        load_layer(sRegA, wsrc, 1, bar0 + 8u);
     }
     cluster_wait();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -136,16 +104,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
 
     if (control) {
         // ================= control warp (converged; one elected lane per tcgen05 instruction) =================
-        constexpr uint32_t kDescLo = 1u << 16, kDescHi32 = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);  // umma_desc, as 32-bit halves
         const uint32_t elected = elect_one();
 #pragma unroll 1
         for (int layer = 0; layer < 4; ++layer) {
-            const int K = layer == 0 ? kIn : kHidden;
-            const int N = layer == 3 ? kHeadRows : kHidden;
-            const uint32_t slabW = layer == 3 ? kSlabHead : kSlabW;
             const uint32_t sWl = (layer & 1) ? sRegA : sRegB;  // layers 0, 2 read region B; layers 1, 3 region A
             const uint32_t par = (uint32_t)(layer & 1);
-            const uint32_t idesc = umma_idesc(kTileRows, N);
 #pragma unroll 1
             for (int t = 0; t < 2; ++t) {
                 mbar_wait(local_bar(t), par);                       // this CTA's 16 epilogue warps have stored tile t's operand
@@ -158,22 +121,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
                     mbar_wait_cluster(ready_bar(t), par);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     P2_TRACE(2 + 8 * layer + 4 * t);
-                    const uint32_t nk = (uint32_t)K / 16;
-                    const uint32_t sAt = sA + (uint32_t)t * kSmemA, dcol = tmem + (uint32_t)t * 128u;
-                    // ONE elected-thread region per tile and layer, descriptors as 32-bit halves (uniform registers)
-                    if (elected) {
-#pragma unroll 4
-                        for (uint32_t k = 0; k < nk; ++k) {
-                            const uint32_t off = k >> 2, kk = (k & 3) * 32u;
-                            const uint32_t alo = kDescLo | (((sAt + off * kSlabA + kk) >> 4) & 0x3FFFu);
-                            const uint32_t blo = kDescLo | (((sWl + off * slabW + kk) >> 4) & 0x3FFFu);
-                            umma_bf16_pair_lohi(dcol, alo, blo, kDescHi32, idesc, k > 0);
-                        }
-                        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                                         mma_bar(t)),
-                                     "h"((uint16_t)3)
-                                     : "memory");
-                    }
+                    pair_issue_layer(elected, tmem + (uint32_t)t * 128u, sA + (uint32_t)t * kSmemA, sWl, layer, mma_bar(t));
                     __syncwarp();
                     P2_TRACE(3 + 8 * layer + 4 * t);
                 }
@@ -187,13 +135,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
             mbar_wait(mma_bar(0), (uint32_t)(layer & 1));
             mbar_wait(mma_bar(1), (uint32_t)(layer & 1));
             if (lane == 0) {
-                if (layer == 0) {
-                    mbar_expect_tx(bar0 + 16u, kW2);
-                    bulk_load(sRegB, wsrc + kW0 + kW1, kW2, bar0 + 16u);
-                } else {
-                    mbar_expect_tx(bar0 + 24u, kW3);
-                    bulk_load(sRegA, wsrc + kW0 + kW1 + kW2, kW3, bar0 + 24u);
-                }
+                if (layer == 0) load_layer(sRegB, wsrc, 2, bar0 + 16u);
+                else load_layer(sRegA, wsrc, 3, bar0 + 24u);
             }
             __syncwarp();
         }
@@ -232,21 +175,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) mlp_pai
                 if (layer < 3) {
                     uint32_t acc[32];
                     tmem_ld32(tcol + (uint32_t)(g * 32), acc);
-                    uint32_t packed[16];
 #pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        packed[2 * j] = pack_relu_bf16(add2(acc[4 * j], acc[4 * j + 1], bv[j].x, bv[j].y));
-                        packed[2 * j + 1] = pack_relu_bf16(add2(acc[4 * j + 2], acc[4 * j + 3], bv[j].z, bv[j].w));
-                    }
-                    const uint32_t rowbase = sA + (uint32_t)t * kSmemA + (uint32_t)(c0 >> 6) * kSlabA + (uint32_t)r * 128u;
-                    const int j0 = (c0 & 63) >> 3;
-#pragma unroll
-                    for (int qq = 0; qq < 4; ++qq) {
-                        const uint32_t dst = rowbase + (uint32_t)(((j0 + qq) ^ (r & 7)) << 4);
-                        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(packed[4 * qq]), "r"(packed[4 * qq + 1]),
-                                     "r"(packed[4 * qq + 2]), "r"(packed[4 * qq + 3])
-                                     : "memory");
-                    }
+                    for (int qq = 0; qq < 4; ++qq)
+                        st_shared_v4(a_chunk(sA + (uint32_t)t * kSmemA, r, (c0 >> 3) + qq), hidden_chunk(acc + 8 * qq, bv + 2 * qq));
                     // this warp's part of tile t's next operand -> visible to the tensor cores; its accumulator reads are done
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -304,22 +235,6 @@ extern "C" int bz_mlp_pair2_debug_trace(long long *host_out) {
 #endif
 
 extern "C" int bz_mlp_forward_pair2(const void *x_bf16, const void *weight_image_pair, void *out_bf16, int64_t n, bz_stream_t stream) {
-    if (n < 0 || (n && (!x_bf16 || !weight_image_pair || !out_bf16))) return BZ_ERR_ARG;
-    if (!aligned16(x_bf16) || !aligned16(weight_image_pair) || !aligned16(out_bf16)) return BZ_ERR_UNALIGNED;
-    if (n == 0) return BZ_OK;
     static bool configured[64] = {};
-    {
-        cudaError_t e = allow_dynamic_smem(mlp_pair2_kernel, kSmemTotal, configured);
-        if (e != cudaSuccess) return cuda_rc(e);
-    }
-    Pair2Params p = {};
-    p.x = (const __nv_bfloat16 *)x_bf16;
-    p.wimg = (const uint8_t *)weight_image_pair;
-    p.out = (__nv_bfloat16 *)out_bf16;
-    p.B = (int)n;
-    const unsigned pairs = (unsigned)((n + kPairRows - 1) / kPairRows);
-    cudaError_t e = launch_kernel(mlp_pair2_kernel, dim3(2 * pairs), dim3(kThreads), (size_t)kSmemTotal, as_stream(stream),
-                                  pdl_enabled(), p);
-    if (e != cudaSuccess) return cuda_rc(e);
-    return launch_rc();
+    return launch_pair_mlp(mlp_pair2_kernel, kPairRows, kThreads, kSmemTotal, configured, x_bf16, weight_image_pair, out_bf16, n, stream);
 }

@@ -1,6 +1,6 @@
-// tcgen05 / TMEM / mbarrier / bulk-copy building blocks shared by the MLP kernels (mlp.cu, mlp_pair.cu): inline PTX
-// for sm_100a.  Descriptor encodings follow the PTX ISA "tcgen05 shared memory descriptor" / "instruction
-// descriptor" tables.
+// tcgen05 / TMEM / mbarrier / bulk-copy building blocks of the net's kernels (pair_net.cuh; the single-CTA helpers are
+// those of profiles/experiments/mlp_onecta.cu): inline PTX for sm_100a.  Descriptor encodings follow the PTX ISA
+// "tcgen05 shared memory descriptor" / "instruction descriptor" tables.
 #pragma once
 #include <cstdint>
 #include <cuda_bf16.h>
@@ -20,6 +20,9 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr) {
     d |= (uint64_t)2 << 61;
     return d;
 }
+// umma_desc as 32-bit halves (umma_bf16_pair_lohi): LBO = 1 in the low word beside the address; SBO, version and
+// SWIZZLE_128B in the high word, the same for every operand
+constexpr uint32_t kDescLo = 1u << 16, kDescHi32 = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);
 
 // instruction descriptor for kind::f16: D = F32, A = B = BF16, both K-major, shape M x N
 __device__ __forceinline__ uint32_t umma_idesc(int M, int N) {
@@ -65,18 +68,13 @@ __device__ __forceinline__ void mbar_wait_parked(uint32_t bar, uint32_t parity) 
             : "r"(bar), "r"(parity), "r"(20000u)
             : "memory");
         if (done) return;
-#ifdef BZ_PARK_NS
-        __nanosleep(BZ_PARK_NS);
-#endif
     }
     __trap();
 }
 
-// Short waits beside working warps: poll, but yield the issue slot for BZ_NAP_NS between polls (measured on the final
+// Short waits beside working warps: poll, but yield the issue slot for kNapNs between polls (measured on the final
 // one-launch kernel: 20 / 40 / 100 ns all +0.7 % from the start position, +0.3 % in the bench region, against a plain spin)
-#ifndef BZ_NAP_NS
-#define BZ_NAP_NS 32
-#endif
+constexpr unsigned kNapNs = 32;
 __device__ __forceinline__ void mbar_wait_nap(uint32_t bar, uint32_t parity) {
     for (uint32_t spin = 0; spin < (1u << 26); ++spin) {
         uint32_t done;
@@ -86,7 +84,7 @@ __device__ __forceinline__ void mbar_wait_nap(uint32_t bar, uint32_t parity) {
             : "r"(bar), "r"(parity)
             : "memory");
         if (done) return;
-        if (BZ_NAP_NS > 0) __nanosleep(BZ_NAP_NS);
+        __nanosleep(kNapNs);
     }
     __trap();
 }
@@ -121,12 +119,16 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint4 v) {
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+
 __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
     const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
     return *reinterpret_cast<const uint32_t *>(&v);
 }
 
-// ---- CTA pairs (clusters of 2, tcgen05 cta_group::2): used by mlp_pair.cu and mlp_pair2.cu -------------------------
+// ---- CTA pairs (clusters of 2, tcgen05 cta_group::2): the net of pair_net.cuh ---------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));

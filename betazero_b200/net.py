@@ -95,19 +95,21 @@ class PolicyValueMLP(nn.Module):
         self._head_full = (hw, hb)
         self._head = (hw[: self.raw_width], hb[: self.raw_width])
         self._w = [m.weight.t() for m in (self.fc1, self.fc2, self.fc3)]  # views of the parameters themselves
-        if w.is_cuda and w.dtype == torch.bfloat16 and self.fc1.in_features == 128 and self.fc1.out_features == 256 \
-                and self.raw_width == 72:
+        if w.is_cuda and w.dtype == torch.bfloat16 and self._tcgen05_shape():
             ws = [self.fc1.weight, self.fc2.weight, self.fc3.weight, hw[:80]]
             bs = [self.fc1.bias, self.fc2.bias, self.fc3.bias, hb[:80]]
             keep("_image_pair", pack_mlp_pair_image(ws, bs))
         else:
             self._image_pair = None
 
+    def _tcgen05_shape(self) -> bool:
+        """the shape of the net the tcgen05 kernels implement (csrc/pair_net.cuh): 128-256-256-256-(65+1)"""
+        return self.fc1.in_features == 128 and self.fc1.out_features == 256 and self.raw_width == 72
+
     def fused_kernel_ok(self, planes: torch.Tensor) -> bool:
         """the hand-written tcgen05 kernel covers exactly the Reversi shape in bf16 on a GPU"""
         return (planes.is_cuda and planes.dtype == torch.bfloat16 and self.fc1.weight.dtype == torch.bfloat16
-                and self.fc1.in_features == 128 and self.fc1.out_features == 256 and self.raw_width == 72
-                and not self.training)
+                and self._tcgen05_shape() and not self.training)
 
     @torch.no_grad()
     def forward_raw(self, planes: torch.Tensor, out: torch.Tensor | None = None, fused: bool | str | None = None) -> torch.Tensor:
