@@ -1,7 +1,7 @@
 """The policy/value net, bit for bit: exactly representable nets against a float64 reference.
 
 An "exact net" has weights and biases that are small integers times a power of two per layer, with sparse rows, and is
-fed 0/1 planes.  `check_exact` proves, on the data of each test, that every partial sum of every layer is then an
+fed 0/1 planes (the tic-tac-toe net of test_gpu_logits_path.py: 0/+-1 cells).  `check_exact` proves, on the data of each test, that every partial sum of every layer is then an
 integer multiple of the layer's grid unit u far below 2^24 u: the fp32 accumulators of the tensor cores hold the exact
 sum whatever the summation order, and every bf16 the kernels write must equal the float64 sum rounded to nearest even.
 So the tcgen05 MLP kernels (`bz_mlp_forward_pair` / `_pair2`) and the copy of the net inside the one-launch search
@@ -31,15 +31,17 @@ def _sparse_ints(rows, cols, nnz, wmax, g):
     return torch.zeros(rows, cols, dtype=torch.float64).scatter_(1, pos, val.double())
 
 
-def exact_net(seed, nnz=(24, 16, 16, 16), wmax=(7, 7, 3, 3), bias=(64, 64, 64, 64), shifts=(0, 0, 0, 12), device="cpu"):
-    """A bf16 PolicyValueMLP 128-256-256-256-(65+1) whose layer l (fc1, fc2, fc3, head) has nnz[l] nonzero weights per
-    row, integers in +-[1, wmax[l]], integer biases in [-bias[l], bias[l]], all times 2^-shifts[l].  The value row is
-    the head's 66th row.  The default head shift keeps the logits within about +-20 on Reversi positions."""
+def exact_net(seed, nnz=(24, 16, 16, 16), wmax=(7, 7, 3, 3), bias=(64, 64, 64, 64), shifts=(0, 0, 0, 12), device="cpu",
+              n_in=128, n_actions=N_ACTIONS):
+    """A bf16 PolicyValueMLP n_in-256-256-256-(n_actions+1) (default: the Reversi net 128-256-256-256-(65+1)) whose
+    layer l (fc1, fc2, fc3, head) has nnz[l] nonzero weights per row, integers in +-[1, wmax[l]], integer biases in
+    [-bias[l], bias[l]], all times 2^-shifts[l].  The value row is the head's last row.  The default head shift keeps
+    the logits within about +-20 on Reversi positions."""
     from betazero_b200 import net
 
     g = torch.Generator().manual_seed(seed)
-    m = net.PolicyValueMLP(128, 256, N_ACTIONS)
-    shapes = ((256, 128), (256, 256), (256, 256), (N_ACTIONS + 1, 256))
+    m = net.PolicyValueMLP(n_in, 256, n_actions)
+    shapes = ((256, n_in), (256, 256), (256, 256), (n_actions + 1, 256))
     params = []
     for l, (rows, cols) in enumerate(shapes):
         W = _sparse_ints(rows, cols, nnz[l], wmax[l], g) * 2.0 ** -shifts[l]
@@ -50,10 +52,10 @@ def exact_net(seed, nnz=(24, 16, 16, 16), wmax=(7, 7, 3, 3), bias=(64, 64, 64, 6
             fc.weight.copy_(W)
             fc.bias.copy_(b)
         W, b = params[3]
-        m.policy.weight.copy_(W[:N_ACTIONS])
-        m.policy.bias.copy_(b[:N_ACTIONS])
-        m.value.weight.copy_(W[N_ACTIONS:])
-        m.value.bias.copy_(b[N_ACTIONS:])
+        m.policy.weight.copy_(W[:n_actions])
+        m.policy.bias.copy_(b[:n_actions])
+        m.value.weight.copy_(W[n_actions:])
+        m.value.bias.copy_(b[n_actions:])
     return m.to(device=device, dtype=torch.bfloat16).eval()
 
 
@@ -107,7 +109,7 @@ def check_exact(net, planes):
     Rounding a multiple of u to bf16 gives a multiple of u again, so the next layer's input grid is u."""
     a = planes.reshape(planes.shape[0], -1).double()
     u_a = 1.0
-    assert torch.equal(a, (a == 1).double()), "the planes must be 0/1"
+    assert torch.equal(a.abs(), (a.abs() == 1).double()), "the planes must be 0/1 (tic-tac-toe: 0/+-1)"
     pre = []
     for l, (W, b) in enumerate(_layers(net)):
         u = min(_unit(W) * u_a, _unit(b))  # every product and the bias are integer multiples of u
