@@ -115,6 +115,18 @@ __device__ __forceinline__ void apply_legal(uint64_t &me, uint64_t &opp, unsigne
     }
 }
 
+// the cell of the k-th set bit of m in ascending cell order (k < popcount(m))
+__device__ __forceinline__ unsigned kth_bit(uint64_t m, int k) {
+    for (; k > 0; --k) m &= m - 1;
+    return (unsigned)(__ffsll((long long)m) - 1);
+}
+
+// a move drawn from the legal moves m (m != 0) by the 32-bit draw u: the k-th legal move in ascending cell order,
+// k = floor(u * moves / 2^32)
+__device__ __forceinline__ unsigned pick_move(uint64_t m, uint32_t u) {
+    return kth_bit(m, (int)(((uint64_t)u * (uint64_t)__popcll(m)) >> 32));
+}
+
 // ---- group-cooperative forms (tree kernels: a group of G lanes owns one board) -------------------
 // The 8 ray directions are spread over 8 lanes of the group instead of being computed serially by
 // every lane: group lane d handles shift {1,7,8,9}[d & 3]; lanes 4..7 work on the bit-reversed

@@ -14,11 +14,15 @@
 // at depths 3 - 6 on 4096 mid-game roots (DESIGN.md section 7).
 //
 // The endgame solver (bz_endgame_solve; definition: oracle/endgame_ref.py) searches to the end of the game with
-// negamax and passes, split at two plies; it has its own prep, search and finish kernels and shares the workspace
-// layout, the scan, item_root and the hand-out (take_item) with the minimax search.  Its win/draw/loss form
-// (bz_endgame_solve_wld) is the same kernels instantiated with kWld: a null window and fastest-first move ordering.
-// Self-play's endgame queue (selfplay.cu) runs the same kernels with its root count read from device memory
-// (endgame_launch_live).
+// passes, split at two plies; it has its own prep and finish kernels and shares the workspace layout, the scan and the
+// item search with minimax.  Its win/draw/loss form (bz_endgame_solve_wld) is the same kernels instantiated with kWld:
+// a null window and fastest-first move ordering.  Self-play's endgame queue (selfplay.cu) runs the same kernels with
+// its root count read from device memory (endgame_launch_live).
+//
+// The item search (search_kernel) is one negamax loop for both solvers, with a struct per solver for what differs.
+// Minimax in negamax form visits the reference's nodes: its value at depth d is (-1)^d times the value for the mover, a
+// min node's beta update is the negamax alpha update on the negated window, and the initial best differs only at a node
+// without children, which the node rule ends first.
 #include "bitboard.cuh"
 #include "common.cuh"
 #include "minimax.cuh"
@@ -27,7 +31,6 @@ namespace bz {
 namespace {
 
 constexpr int kD0 = 1;  // absolute depth of a work item's first node: a root move's child
-constexpr int kLevels = BZ_MINIMAX_MAX_DEPTH + 1;
 constexpr int kInf = 127;      // the value of +-inf
 constexpr int kWindow = 128;   // the full window (-128, 128) holds every value, +-inf included
 constexpr int kSlots = 64;     // per root in the workspace's value array: more than any position's move count
@@ -74,16 +77,10 @@ __device__ __forceinline__ int root_depth(const MinimaxRoots &R, int64_t i, uint
     return d <= BZ_MINIMAX_MAX_DEPTH ? d : kSkip;  // a net entrant's tree
 }
 
-__device__ __forceinline__ unsigned kth_bit(uint64_t m, int k) {
-    for (; k > 0; --k) m &= m - 1;
-    return (unsigned)(__ffsll((long long)m) - 1);
-}
-
 // the reference's random.choice(moves) (reversi_players.py:42-43), reproducibly: Philox keyed by 2^32 + the game key,
-// counter = discs on the board; the k-th legal move in ascending cell order, k = floor(u * moves / 2^32)
+// counter = discs on the board
 __device__ __forceinline__ unsigned random_move(uint64_t seed, uint64_t key, uint64_t me, uint64_t opp, uint64_t m) {
-    const uint32_t u = philox_u32(seed, (1ull << 32) + key, (uint32_t)__popcll(me | opp));
-    return kth_bit(m, (int)(((uint64_t)u * (uint64_t)__popcll(m)) >> 32));
+    return pick_move(m, philox_u32(seed, (1ull << 32) + key, (uint32_t)__popcll(me | opp)));
 }
 
 __global__ void __launch_bounds__(256) minimax_prep_kernel(const MinimaxRoots R, uint64_t seed, uint64_t cells, Workspace W,
@@ -175,98 +172,6 @@ __device__ __forceinline__ bool take_item(const Workspace &W, int64_t n, unsigne
     return true;
 }
 
-__global__ void __launch_bounds__(kSearchThreads) minimax_search_kernel(const MinimaxRoots R, uint64_t cells, Workspace W) {
-    const unsigned total = W.counter[1];
-    // the stack of the item's search: level k holds the node at absolute depth kD0 + k
-    uint64_t s_me[kLevels], s_opp[kLevels], s_rem[kLevels];
-    int s_best[kLevels], s_alpha[kLevels], s_beta[kLevels];
-    int k = -1;  // level of the node being searched; -1: no item
-    int depth = 0, v = 0;
-    int64_t root = 0;
-    unsigned slot = 0, nodes = 0;
-    bool leaf = false;
-
-    // enter the node (me, opp) at level k: a leaf sets v, an inner node its moves and initial best
-    auto enter = [&](uint64_t me, uint64_t opp) {
-        const int d = kD0 + k;
-        const bool maxing = (d & 1) == 0;
-        s_me[k] = me;
-        s_opp[k] = opp;
-        const int ev = maxing ? __popcll(me) - __popcll(opp) : __popcll(opp) - __popcll(me);
-        if (d >= depth) {
-            v = ev;
-            leaf = true;
-            return;
-        }
-        const uint64_t m = legal_mask(me, opp, cells);
-        if (m == 0) {  // game over: evaluate; otherwise the loop over no moves returns the initial -inf / +inf
-            v = legal_mask(opp, me, cells) == 0 ? ev : (maxing ? -kInf : kInf);
-            leaf = true;
-            return;
-        }
-        s_rem[k] = m;
-        s_best[k] = maxing ? -kInf : kInf;
-        leaf = false;
-    };
-
-    while (true) {
-        if (k < 0) {
-            if (!take_item(W, R.n, total, root, slot)) break;
-            uint64_t key;
-            depth = root_depth(R, root, key);
-            uint64_t me = R.me[root], opp = R.opp[root];
-            slot -= W.offset[root];
-            BZ_CHECK(slot < (unsigned)kSlots, 63);  // value slot
-            k = 0;
-            nodes = 1;
-            s_alpha[0] = -kWindow;
-            s_beta[0] = kWindow;
-            apply_legal(me, opp, kth_bit(legal_mask(me, opp, cells), (int)slot));
-            enter(me, opp);
-        } else if (!leaf) {  // descend into the next move of level k, row-major
-            const uint64_t rem = s_rem[k];
-            const uint64_t x = rem & (0ull - rem);
-            s_rem[k] = rem ^ x;
-            uint64_t me = s_me[k], opp = s_opp[k];
-            apply_legal(me, opp, (unsigned)(__ffsll((long long)x) - 1));
-            BZ_CHECK(k + 1 < kLevels, 64);  // stack level
-            s_alpha[k + 1] = s_alpha[k];
-            s_beta[k + 1] = s_beta[k];
-            ++k;
-            ++nodes;
-            enter(me, opp);
-        }
-        if (!leaf) continue;
-        // return v to the parents until one has a move left to search
-        while (true) {
-            if (k == 0) {
-                BZ_CHECK(root * kSlots + slot < R.n * kSlots, 65);  // value slot
-                W.vals[root * kSlots + slot] = (int8_t)v;
-                atomicAdd(&W.nodes[root], (unsigned long long)nodes);
-                k = -1;
-                break;
-            }
-            --k;
-            const bool maxing = ((kD0 + k) & 1) == 0;
-            int best = s_best[k];
-            if (maxing) {
-                if (v > best) best = v;
-                if (best > s_alpha[k]) s_alpha[k] = best;
-            } else {
-                if (v < best) best = v;
-                if (best < s_beta[k]) s_beta[k] = best;
-            }
-            s_best[k] = best;
-            if (s_alpha[k] >= s_beta[k] || s_rem[k] == 0) {
-                v = best;
-                continue;
-            }
-            leaf = false;
-            break;
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256) minimax_finish_kernel(const MinimaxRoots R, uint64_t seed, uint64_t cells, Workspace W,
                                                              uint8_t *action, int8_t *value, int64_t *nodes,
                                                              int64_t *nodes_total) {
@@ -304,7 +209,7 @@ __global__ void __launch_bounds__(256) minimax_finish_kernel(const MinimaxRoots 
 // one work item, and so is a root move whose child must pass or is finished; one thread searches it with alpha-beta in
 // row-major order and the full window, so the item's value is exact.  move_value[a] is the minimum over a's items
 // (atomicMin into the workspace), and the finish kernel takes the first maximum.  A root that must pass has the pass as
-// its one move.  Workspace, scan, item_root and the persistent hand-out are those of the minimax search.
+// its one move.  Workspace, scan and the item search are those of minimax.
 //
 // The win/draw/loss solve (kWld; bz_endgame_solve_wld) runs the same items with the null window (-1, 1): fail-soft, an
 // item's value v >= 1 is a win, v <= -1 a loss and 0 an exact draw, so clamped to [-1, 1] it is the sign of the exact
@@ -392,16 +297,22 @@ __global__ void __launch_bounds__(256) endgame_prep_kernel(const uint64_t *me_, 
     W.offset[i] = cnt;
 }
 
-template <bool kWld>
-__global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const uint64_t *me_, const uint64_t *opp_,
-                                                                        int64_t n, uint64_t cells, Workspace W) {
+// ---- the item search of both solvers --------------------------------------------------------------------------------
+// Fail-soft alpha-beta negamax of one item per thread from the item's first node.  S supplies what differs between the
+// solvers: kLevels (the stack depth), kOrdered (fastest first at nodes with at least kOrderEmpties empties), roots(),
+// first() (the item's first node and window (-w, w), or false and the value of an item whose game is over: the prep
+// kernel entered its node), node() (the node rule: kLeaf and the value for the node's mover, kInner and the moves, or
+// kPass and the opponent's moves) and store() (the value of the item's first node, for its mover).
+enum NodeKind { kInner, kLeaf, kPass };
+
+template <class S>
+__global__ void __launch_bounds__(kSearchThreads) search_kernel(const S s, Workspace W) {
     const unsigned total = W.counter[1];
-    int *const mv = reinterpret_cast<int *>(W.vals);
     // the stack of the item's search: level k holds the node k plies below the item's first node; a node whose mover
     // must pass is held as the position after the pass, with bit k of `passed` set and its window negated
-    uint64_t s_me[kSolveLevels], s_opp[kSolveLevels], s_rem[kSolveLevels];
-    int s_best[kSolveLevels], s_alpha[kSolveLevels], s_beta[kSolveLevels];
-    // kWld: a level with bit k of `ordered` set descends in the order of s_order[k] (order_moves' keys), from s_cur[k]
+    uint64_t s_me[S::kLevels], s_opp[S::kLevels], s_rem[S::kLevels];
+    int s_best[S::kLevels], s_alpha[S::kLevels], s_beta[S::kLevels];
+    // S::kOrdered: a level with bit k of `ordered` set descends in the order of s_order[k] from s_cur[k] (order_moves)
     uint16_t s_order[kOrderLevels][kOrderMoves];
     uint8_t s_cur[kOrderLevels];
     unsigned ordered = 0;
@@ -409,28 +320,27 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
     int k = -1;  // level of the node being searched; -1: no item
     int v = 0;
     int64_t root = 0;
-    unsigned slot = 0, move = 0;
+    unsigned slot = 0;
+    typename S::Item it;
     unsigned long long nodes = 0;
     bool leaf = false;
 
-    // enter the node (me, opp) at level k with the window (alpha, beta): a finished game sets v, any other node its moves
+    // enter the node (me, opp) at level k with the window (alpha, beta): a leaf sets v, any other node its moves
     auto enter = [&](uint64_t me, uint64_t opp, int alpha, int beta) {
         ++nodes;
         passed &= ~(1u << k);
-        uint64_t m = legal_mask(me, opp, cells);
-        if (m == 0) {
-            const uint64_t mo = legal_mask(opp, me, cells);
-            if (mo == 0) {  // game over: the disc difference, empty squares to nobody
-                v = __popcll(me) - __popcll(opp);
-                leaf = true;
-                return;
-            }
+        uint64_t m = 0;
+        const NodeKind kind = s.node(me, opp, k, it, m, v);
+        if (kind == kLeaf) {
+            leaf = true;
+            return;
+        }
+        if (kind == kPass) {
             ++nodes;  // the position after the pass
             passed |= 1u << k;
             const uint64_t t = me;
             me = opp;
             opp = t;
-            m = mo;
             const int a = alpha;
             alpha = -beta;
             beta = -a;
@@ -441,10 +351,10 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
         s_best[k] = -kWindow;
         s_alpha[k] = alpha;
         s_beta[k] = beta;
-        if constexpr (kWld) {
+        if constexpr (S::kOrdered) {
             ordered &= ~(1u << k);
-            if (k < kOrderLevels && solve_empties(me, opp, cells) >= kOrderEmpties) {
-                order_moves(me, opp, m, cells, s_order[k]);
+            if (k < kOrderLevels && solve_empties(me, opp, s.cells) >= kOrderEmpties) {
+                order_moves(me, opp, m, s.cells, s_order[k]);
                 s_cur[k] = 0;
                 ordered |= 1u << k;
             }
@@ -454,42 +364,24 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
 
     while (true) {
         if (k < 0) {
-            if (!take_item(W, n, total, root, slot)) break;
+            if (!take_item(W, s.roots(), total, root, slot)) break;
             slot -= W.offset[root];
-            const uint64_t me = me_[root], opp = opp_[root], m = legal_mask(me, opp, cells);
-            const int moves = m ? __popcll(m) : 1;
-            uint64_t cme = 0, copp = 0, cm = 0;
             nodes = 0;
             k = 0;
-            unsigned r = slot;
-            for (int j = 0; j < moves; ++j) {  // the root move of the item, and the reply's index r
-                move = root_move(me, opp, m, j, cme, copp);
-                cm = legal_mask(cme, copp, cells);
-                const unsigned c = cm ? (unsigned)__popcll(cm) : 1u;
-                if (r < c) break;
-                r -= c;
-            }
-            BZ_CHECK(r < (cm ? (unsigned)__popcll(cm) : 1u), 71);  // reply
-            constexpr int w = kWld ? 1 : kWindow;  // the null window, or the full one
-            if (cm) {
-                apply_legal(cme, copp, kth_bit(cm, (int)r));
-                enter(cme, copp, -w, w);
-            } else if (legal_mask(copp, cme, cells)) {
-                enter(copp, cme, -w, w);  // the child passes: the item is the position after the pass
-            } else {
-                v = __popcll(copp) - __popcll(cme);  // the child's game is over: the root mover's count
-                leaf = true;
-            }
+            uint64_t me = 0, opp = 0;
+            int w = 0;
+            if (s.first(root, slot, it, me, opp, w, v)) enter(me, opp, -w, w);
+            else leaf = true;
         } else if (!leaf) {  // descend into the next move of level k: row-major, or in the level's order
             const uint64_t rem = s_rem[k];
             uint64_t x = rem & (0ull - rem);
-            if constexpr (kWld) {
+            if constexpr (S::kOrdered) {
                 if ((ordered >> k) & 1u) x = 1ull << (s_order[k][s_cur[k]++] & 63u);
             }
             s_rem[k] = rem ^ x;
             uint64_t me = s_me[k], opp = s_opp[k];
             apply_legal(me, opp, (unsigned)(__ffsll((long long)x) - 1));
-            BZ_CHECK(k + 1 < kSolveLevels, 72);  // stack level: a disc per level, at most BZ_SOLVE_MAX_EMPTIES
+            BZ_CHECK(k + 1 < S::kLevels, 64);  // stack level
             const int alpha = s_alpha[k], beta = s_beta[k];
             ++k;
             enter(me, opp, -beta, -alpha);
@@ -498,10 +390,7 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
         // return v, the value of level k's node for its mover, to the parents until one has a move left to search
         while (true) {
             if (k == 0) {
-                // the item's first node belongs to the root's mover: a move's value is its items' minimum
-                BZ_CHECK(root * kMoveSlots + move < n * kMoveSlots, 73);  // move value slot
-                if constexpr (kWld) v = v > 1 ? 1 : (v < -1 ? -1 : v);  // a bound beyond the null window: its sign
-                atomicMin(&mv[root * kMoveSlots + move], v);
+                s.store(W, root, slot, it, v);
                 if (nodes) atomicAdd(&W.nodes[root], nodes);
                 k = -1;
                 break;
@@ -521,6 +410,102 @@ __global__ void __launch_bounds__(kSearchThreads) endgame_search_kernel(const ui
         }
     }
 }
+
+// minimax: the item of root move `slot` is that move's child, the opponent's node, searched to the root's depth
+struct MinimaxItems {
+    static constexpr int kLevels = BZ_MINIMAX_MAX_DEPTH + 1;
+    static constexpr bool kOrdered = false;
+    struct Item { int depth; };
+    MinimaxRoots R;
+    uint64_t cells;
+
+    __device__ __forceinline__ int64_t roots() const { return R.n; }
+
+    __device__ __forceinline__ bool first(int64_t root, unsigned slot, Item &it, uint64_t &me, uint64_t &opp, int &w,
+                                          int &) const {
+        uint64_t key;
+        it.depth = root_depth(R, root, key);
+        me = R.me[root];
+        opp = R.opp[root];
+        BZ_CHECK(slot < (unsigned)kSlots, 63);  // value slot
+        apply_legal(me, opp, kth_bit(legal_mask(me, opp, cells), (int)slot));
+        w = kWindow;
+        return true;
+    }
+
+    // at the depth limit the disc difference; without a move the disc difference if the game is over, otherwise -inf:
+    // the reference's search does not pass, its loop over no moves returns the initial -inf (for the mover)
+    __device__ __forceinline__ NodeKind node(uint64_t me, uint64_t opp, int k, const Item &it, uint64_t &m,
+                                             int &v) const {
+        v = __popcll(me) - __popcll(opp);
+        if (kD0 + k >= it.depth) return kLeaf;
+        m = legal_mask(me, opp, cells);
+        if (m) return kInner;
+        if (legal_mask(opp, me, cells)) v = -kInf;
+        return kLeaf;
+    }
+
+    __device__ __forceinline__ void store(const Workspace &W, int64_t root, unsigned slot, const Item &, int v) const {
+        BZ_CHECK(root * kSlots + slot < R.n * kSlots, 65);  // value slot
+        W.vals[root * kSlots + slot] = (int8_t)-v;  // the root mover's view of the opponent's node
+    }
+};
+
+// the endgame solver: the item is a (root move, reply) decoded from its index, or a root move whose child must pass or
+// is finished; kWld: the null window and move ordering
+template <bool kWld>
+struct EndgameItems {
+    static constexpr int kLevels = kSolveLevels;
+    static constexpr bool kOrdered = kWld;
+    struct Item { unsigned move; };  // the root move
+    const uint64_t *root_me, *root_opp;
+    int64_t n;
+    uint64_t cells;
+
+    __device__ __forceinline__ int64_t roots() const { return n; }
+
+    __device__ __forceinline__ bool first(int64_t root, unsigned slot, Item &it, uint64_t &me, uint64_t &opp, int &w,
+                                          int &v) const {
+        const uint64_t rme = root_me[root], ropp = root_opp[root], m = legal_mask(rme, ropp, cells);
+        const int moves = m ? __popcll(m) : 1;
+        uint64_t cme = 0, copp = 0, cm = 0;
+        unsigned r = slot;
+        for (int j = 0; j < moves; ++j) {  // the root move of the item, and the reply's index r
+            it.move = root_move(rme, ropp, m, j, cme, copp);
+            cm = legal_mask(cme, copp, cells);
+            const unsigned c = cm ? (unsigned)__popcll(cm) : 1u;
+            if (r < c) break;
+            r -= c;
+        }
+        BZ_CHECK(r < (cm ? (unsigned)__popcll(cm) : 1u), 71);  // reply
+        if (!cm && !legal_mask(copp, cme, cells)) {
+            v = __popcll(copp) - __popcll(cme);  // the child's game is over: the root mover's count
+            return false;
+        }
+        apply_legal(cme, copp, cm ? kth_bit(cm, (int)r) : 64u);  // the child passes: the item is the position after it
+        me = cme;
+        opp = copp;
+        w = kWld ? 1 : kWindow;  // the null window, or the full one
+        return true;
+    }
+
+    // a finished game: the disc difference, empty squares to nobody; no move: a pass
+    __device__ __forceinline__ NodeKind node(uint64_t me, uint64_t opp, int, const Item &, uint64_t &m, int &v) const {
+        m = legal_mask(me, opp, cells);
+        if (m) return kInner;
+        m = legal_mask(opp, me, cells);
+        if (m) return kPass;
+        v = __popcll(me) - __popcll(opp);
+        return kLeaf;
+    }
+
+    // the item's first node belongs to the root's mover: a move's value is its items' minimum
+    __device__ __forceinline__ void store(const Workspace &W, int64_t root, unsigned, const Item &it, int v) const {
+        BZ_CHECK(root * kMoveSlots + it.move < n * kMoveSlots, 73);  // move value slot
+        if constexpr (kWld) v = v > 1 ? 1 : (v < -1 ? -1 : v);  // a bound beyond the null window: its sign
+        atomicMin(reinterpret_cast<int *>(W.vals) + root * kMoveSlots + it.move, v);
+    }
+};
 
 template <bool kLive>
 __global__ void __launch_bounds__(256) endgame_finish_kernel(const uint64_t *me_, const uint64_t *opp_, int64_t n,
@@ -569,7 +554,7 @@ int minimax_launch(const MinimaxRoots &R, uint64_t seed, int size, void *workspa
     const unsigned blocks = (unsigned)((R.n + 255) / 256);
     minimax_prep_kernel<<<blocks, 256, 0, stream>>>(R, seed, cells, W, action, value);
     minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, R.n);
-    minimax_search_kernel<<<persistent_grid(R.n * 32, kSearchThreads, 8), kSearchThreads, 0, stream>>>(R, cells, W);
+    search_kernel<<<persistent_grid(R.n * 32, kSearchThreads, 8), kSearchThreads, 0, stream>>>(MinimaxItems{R, cells}, W);
     minimax_finish_kernel<<<blocks, 256, 0, stream>>>(R, seed, cells, W, action, value, nodes, nodes_total);
     return launch_rc();
 }
@@ -589,8 +574,8 @@ void endgame_kernels(const uint64_t *me, const uint64_t *opp, int64_t n, const i
     const unsigned blocks = (unsigned)((n + 255) / 256);
     endgame_prep_kernel<kLive, kWld><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, live);
     minimax_scan_kernel<<<1, 1024, 0, stream>>>(W, n);  // the roots past *live have no items: no item maps to them
-    endgame_search_kernel<kWld><<<persistent_grid(n * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(me, opp, n,
-                                                                                                         cells, W);
+    search_kernel<<<persistent_grid(n * 64, kSearchThreads, 8), kSearchThreads, 0, stream>>>(
+        EndgameItems<kWld>{me, opp, n, cells}, W);
     endgame_finish_kernel<kLive><<<blocks, 256, 0, stream>>>(me, opp, n, cells, W, action, value, move_value, nodes,
                                                              live);
 }

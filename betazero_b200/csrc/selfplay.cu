@@ -464,14 +464,7 @@ __global__ void __launch_bounds__(256) match_init_kernel(const bz_match_state S,
     while (!over && ply < S.opening_plies && ply < BZ_MATCH_MAX_PLIES) {
         const uint64_t m = legal_mask(me, opp, cells);
         unsigned action = 64u;  // pass: the mover has no move (the game is not over, so the opponent has one)
-        if (m) {
-            // the k-th legal move in ascending cell order, k = floor(u32 * moves / 2^32)
-            const uint32_t r = philox_u32(S.seed, pair_id, (uint32_t)ply);
-            int k = (int)(((uint64_t)r * (uint64_t)__popcll(m)) >> 32);
-            uint64_t b = m;
-            for (; k > 0; --k) b &= b - 1;
-            action = (unsigned)(__ffsll((long long)b) - 1);
-        }
+        if (m) action = pick_move(m, philox_u32(S.seed, pair_id, (uint32_t)ply));
         BZ_CHECK(ply >= 0 && ply < BZ_MATCH_MAX_PLIES, 31);  // move row
         mv[ply] = (uint8_t)action;
         apply_legal(me, opp, action);

@@ -1,6 +1,9 @@
 """Shared test helpers: the reference's episode loops restated without prints, and an oracle-side
 MCTS player (oracle/mcts_ref.py on the C-restated boards) with the reference's player interface."""
+import ctypes
+
 import numpy as np
+import pytest
 
 from oracle import mcts_ref as mr
 from oracle import pyoracle as po
@@ -67,3 +70,19 @@ class OracleMCTSPlayer:
         if cnt.sum() == 0 or (not self.is_ttt and a == 64):
             return None, None
         return (a // 3, a % 3) if self.is_ttt else (a >> 3, a & 7)
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _minimax_bounds_checks():
+    """a -DBZ_BOUNDS_CHECK library: the violation record of the minimax and solver kernels (minimax.cu has its own) must
+    stay empty.  Imported by the test modules of those kernels."""
+    yield
+    import torch
+
+    from betazero_b200 import _lib
+
+    if _lib._lib is not None and hasattr(_lib._lib, "bz_debug_checks_minimax"):
+        torch.cuda.synchronize()
+        rec = (ctypes.c_int * 4)()
+        assert _lib._lib.bz_debug_checks_minimax(rec) == 0
+        assert rec[3] == 0, f"check {rec[0]} failed in block {rec[1]}, thread {rec[2]} ({rec[3]} violations)"

@@ -8,20 +8,9 @@ import numpy as np
 import pytest
 import torch
 
+from helpers import _minimax_bounds_checks  # noqa: F401
+
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _minimax_bounds_checks():
-    """a -DBZ_BOUNDS_CHECK library: the violation record of the minimax and solver kernels must stay empty"""
-    yield
-    from betazero_b200 import _lib
-
-    if _lib._lib is not None and hasattr(_lib._lib, "bz_debug_checks_minimax"):
-        torch.cuda.synchronize()
-        rec = (ctypes.c_int * 4)()
-        assert _lib._lib.bz_debug_checks_minimax(rec) == 0
-        assert rec[3] == 0, f"check {rec[0]} failed in block {rec[1]}, thread {rec[2]} ({rec[3]} violations)"
 
 
 def _dev(x):
