@@ -57,6 +57,16 @@ class BzSelfplayEndgameState(C.Structure):
     N_SCALARS = 4
 
 
+class BzSelfplayResignState(C.Structure):
+    """Mirror of ``bz_selfplay_resign_state`` (include/betazero_b200.h)."""
+
+    _fields_ = [
+        ("threshold", C.c_float), ("reserved", C.c_int32), ("audit_below", C.c_uint64),
+        ("hist_q", ptr), ("eg_hist_q", ptr), ("rp_q", ptr), ("counters", ptr),
+    ]
+    N_SCALARS = 3
+
+
 class BzMatchState(C.Structure):
     """Mirror of ``bz_match_state`` (include/betazero_b200.h)."""
 
@@ -83,6 +93,7 @@ _I64, _INT, _U64, _F = C.c_int64, C.c_int, C.c_uint64, C.c_float
 _PP = C.POINTER(BzTreePools)
 _SP = C.POINTER(BzSelfplayState)
 _EP = C.POINTER(BzSelfplayEndgameState)
+_RP = C.POINTER(BzSelfplayResignState)
 _MP = C.POINTER(BzMatchState)
 _TP = C.POINTER(BzTournamentState)
 SIGNATURES = {
@@ -117,6 +128,8 @@ SIGNATURES = {
     "bz_selfplay_endgame_play": [_SP, _EP, ptr, ptr],
     "bz_selfplay_endgame_play_wld": [_SP, _EP, ptr, ptr],
     "bz_selfplay_endgame_workspace_bytes": [_I64],
+    "bz_selfplay_advance_resign": [_SP, _EP, _RP, _PP, ptr, ptr],
+    "bz_selfplay_endgame_play_resign": [_SP, _EP, _RP, ptr, _INT, ptr],
     "bz_match_init": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
     "bz_tournament_layout": [_TP, ptr],

@@ -35,13 +35,26 @@ __device__ __forceinline__ void restart_slot(const bz_selfplay_state &S, int s, 
     S.game_id[s] = gid + S.id_stride;
 }
 
-// a warp: the game `gid` has ended at (me, opp), seen by the side to move after `player`'s last move; score it and copy
-// its nrec history rows, block `block` of max_plies rows in hist_*, to the replay buffer (whole or not at all); lane 0 counts
+// the result of a game that has ended at (me, opp), seen by the side to move after `player`'s last move (get_score: more
+// discs wins); absolute: +1 X, -1 O, 0 draw
+__device__ __forceinline__ int disc_winner(uint64_t me, uint64_t opp, int player) {
+    const int cm = __popcll(me), co = __popcll(opp);
+    return ((cm > co) - (cm < co)) * (-player);
+}
+
+// game g is audited (never resigns) iff philox_u32(seed, g, 0xFFFFFFFF) < audit_below: the counter is never a ply
+__device__ __forceinline__ bool resign_audited(uint64_t seed, int64_t gid, uint64_t audit_below) {
+    return (uint64_t)philox_u32(seed, (uint64_t)gid, 0xFFFFFFFFu) < audit_below;
+}
+
+// a warp: the game `gid` has ended with `winner` (absolute: +1 X, -1 O, 0 draw); copy its nrec history rows, block `block`
+// of max_plies rows in hist_*, to the replay buffer (whole or not at all); lane 0 counts.  kResign: the q rows (hist_q)
+// go to R->rp_q as well, and an audited game is counted in R->counters[1].
+template <bool kResign = false>
 __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uint64_t *hist_me, const uint64_t *hist_opp,
                                            const int8_t *hist_player, const float *hist_pi, int block, int max_plies,
-                                           int nrec, int64_t gid, uint64_t me, uint64_t opp, int player, int lane) {
-    const int cm = __popcll(me), co = __popcll(opp);
-    const int winner = ((cm > co) - (cm < co)) * (-player);  // absolute: +1 X, -1 O, 0 draw
+                                           int nrec, int64_t gid, int winner, int lane,
+                                           const bz_selfplay_resign_state *R = nullptr, const float *hist_q = nullptr) {
     // counters[0] = rows COMMITTED to the replay buffer: a game reserves its rows with a compare-and-swap and takes
     // nothing when it does not fit, so [0, counters[0]) never contains a row that no game wrote
     unsigned long long rb = ~0ull;  // ~0: no room, the game is dropped (counted in counters[5])
@@ -58,6 +71,9 @@ __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uin
         atomicAdd(&S.counters[1], 1ull);
         atomicAdd(&S.counters[3 + winner], 1ull);
         atomicAdd(&S.counters[6], 1ull);
+        if constexpr (kResign) {
+            if (resign_audited(S.seed, gid, R->audit_below)) atomicAdd(&R->counters[1], 1ull);
+        }
     }
     rb = __shfl_sync(kFull, rb, 0);
     __syncwarp();  // the record written above is visible to the copying lanes
@@ -70,6 +86,7 @@ __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uin
             S.rp_z[rb + r] = (int8_t)(winner * hist_player[h0 + r]);
             S.rp_game[rb + r] = gid;
             S.rp_ply[rb + r] = (int16_t)r;
+            if constexpr (kResign) R->rp_q[rb + r] = hist_q[h0 + r];
         }
         const int64_t nf = (int64_t)nrec * A;  // pi rows are contiguous in both buffers
         const float *src = hist_pi + h0 * A;
@@ -82,9 +99,11 @@ __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uin
 
 // a warp: move the game of slot s -- (me, opp) with `player` to move, nrec history rows -- to the next free entry of the
 // endgame queue, its rows to the entry's history block (row == entry: the queue fills from an empty state between solver
-// phases); false, and counted, when the queue is full
+// phases); false, and counted, when the queue is full.  kResign: the q rows go to R->eg_hist_q as well.
+template <bool kResign>
 __device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_selfplay_endgame_state &EG, int s, int lane,
-                                         uint64_t me, uint64_t opp, int player, int nrec, int64_t gid) {
+                                         uint64_t me, uint64_t opp, int player, int nrec, int64_t gid,
+                                         const bz_selfplay_resign_state *R) {
     int q = -1;
     if (lane == 0) {
         int cur = *EG.count;
@@ -108,6 +127,7 @@ __device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_se
         EG.hist_opp[dst + r] = S.hist_opp[src + r];
         EG.hist_player[dst + r] = S.hist_player[src + r];
         EG.hist_action[dst + r] = S.hist_action[src + r];
+        if constexpr (kResign) R->eg_hist_q[dst + r] = R->hist_q[src + r];
     }
     const int64_t nf = (int64_t)nrec * A;
     for (int64_t i = lane; i < nf; i += 32) EG.hist_pi[dst * A + i] = S.hist_pi[src * A + i];
@@ -124,12 +144,27 @@ __device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_se
     return true;
 }
 
+// a warp: the most visited root action, lowest action id on ties (players.py:92-98 applied to visit counts); lane i holds
+// edge i (Ne, act), edge 32 is held uniformly (N32, act32)
+__device__ __forceinline__ unsigned greedy_action(int Ne, unsigned act, int N32, unsigned act32, int n, int lane) {
+    unsigned key = (lane < n && Ne > 0) ? (((unsigned)Ne << 7) | (127u - act)) : 0u;
+    if (n > 32 && N32 > 0) {
+        const unsigned k32 = ((unsigned)N32 << 7) | (127u - act32);
+        key = k32 > key ? k32 : key;
+    }
+    key = __reduce_max_sync(kFull, key);
+    return 127u - (key & 127u);
+}
+
 // a warp per game slot: the move from the root visit counts, the record, the move applied, the terminal test; a finished
 // game is flushed and its slot restarts.  kEndgame: a game whose move leaves EG->empties empties or fewer for the first
-// time goes to the endgame queue instead (and its slot restarts) when the queue has room.
-template <bool kEndgame>
+// time goes to the endgame queue instead (and its slot restarts) when the queue has room.  kResign: the ply's q (W / N of
+// the most visited root edge, the mover's view) is recorded, and a game that is not audited resigns when q < threshold:
+// the record is kept, the mover loses, the game is flushed and the slot restarts before the move is applied.
+template <bool kEndgame, bool kResign = false>
 __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const bz_tree_pools &P, uint8_t *action_out,
-                                             uint64_t cells, const bz_selfplay_endgame_state *EG, int s, int lane) {
+                                             uint64_t cells, const bz_selfplay_endgame_state *EG, int s, int lane,
+                                             const bz_selfplay_resign_state *R = nullptr) {
 
     // root statistics: lane i holds edge i (ascending action id); a 33rd edge is read uniformly
     const uint32_t rmeta = P.root_meta[s];
@@ -151,6 +186,26 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
     uint64_t me = S.me[s], opp = S.opp[s];
     const int player = S.player[s];
 
+    // --- q of the ply (kResign): W / N of the greedy pick a*, whether or not the move is sampled; NaN without visits ----
+    [[maybe_unused]] unsigned best = 0u;
+    [[maybe_unused]] float q = __int_as_float(0x7FC00000);
+    if constexpr (kResign) {
+        if (n > 0 && total > 0) {
+            best = greedy_action(Ne, act, N32, act32, n, lane);
+            const unsigned hit = __ballot_sync(kFull, lane < n && act == best);
+            const int src = hit ? __ffs(hit) - 1 : 0;
+            float w = 0.f;
+            if (hit && lane == src) w = __uint_as_float(blk[BZ_NODE_HEADER_WORDS + n + lane]);
+            w = __shfl_sync(kFull, w, src);
+            int nb = __shfl_sync(kFull, Ne, src);
+            if (!hit) {  // a* is edge 32
+                w = __uint_as_float(blk[BZ_NODE_HEADER_WORDS + n + 32]);
+                nb = N32;
+            }
+            q = __fdiv_rn(w, (float)nb);
+        }
+    }
+
     // --- choose the move -------------------------------------------------------------------
     unsigned action;
     if (n == 0 || total == 0) {
@@ -169,15 +224,10 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
         }
         const unsigned hit = __ballot_sync(kFull, lane < n && cum > target);
         action = hit ? __shfl_sync(kFull, act, __ffs(hit) - 1) : act32;
+    } else if constexpr (kResign) {
+        action = best;
     } else {
-        // most visited, lowest action id on ties (players.py:92-98 applied to visit counts)
-        unsigned key = (lane < n && Ne > 0) ? (((unsigned)Ne << 7) | (127u - act)) : 0u;
-        if (n > 32 && N32 > 0) {
-            const unsigned k32 = ((unsigned)N32 << 7) | (127u - act32);
-            key = k32 > key ? k32 : key;
-        }
-        key = __reduce_max_sync(kFull, key);
-        action = 127u - (key & 127u);
+        action = greedy_action(Ne, act, N32, act32, n, lane);
     }
 
     // --- record (board, pi, player, action) in the slot's history -----------------------------
@@ -196,6 +246,20 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
         S.hist_player[h] = (int8_t)player;
         S.hist_action[h] = (uint8_t)action;
         if (action_out) action_out[s] = (uint8_t)action;
+        if constexpr (kResign) R->hist_q[h] = q;
+    }
+
+    // --- resignation (kResign): before the move is applied, so before the handover test; NaN never compares below -----
+    if constexpr (kResign) {
+        if (q < R->threshold && !resign_audited(S.seed, gid, R->audit_below)) {
+            flush_game<true>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, ply + 1, gid, -player,
+                             lane, R, R->hist_q);
+            if (lane == 0) {
+                atomicAdd(&R->counters[0], 1ull);
+                restart_slot(S, s, gid);
+            }
+            return;
+        }
     }
 
     // --- apply, terminal test -----------------------------------------------------------------
@@ -208,7 +272,7 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
             // the first position at E empties or fewer (the move placed a disc): a game the full queue refuses is not
             // offered again and is searched to its end
             if (__popcll(cells) - __popcll(me | opp) <= EG->empties && EG->empties < __popcll(cells) - __popcll(occupied) &&
-                handover(S, *EG, s, lane, me, opp, -player, nrec, gid)) {
+                handover<kResign>(S, *EG, s, lane, me, opp, -player, nrec, gid, R)) {
                 if (lane == 0) restart_slot(S, s, gid);
                 return;
             }
@@ -224,7 +288,8 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
     }
 
     // --- finished: score, flush the history to the replay buffer, restart the slot ----------------
-    flush_game(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, nrec, gid, me, opp, player, lane);
+    flush_game<kResign>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, nrec, gid,
+                        disc_winner(me, opp, player), lane, R, kResign ? R->hist_q : nullptr);
     if (lane == 0) restart_slot(S, s, gid);
 }
 
@@ -243,12 +308,26 @@ __global__ void __launch_bounds__(kThreads)
     advance_slot<true>(S, P, action_out, cells, &EG, s, threadIdx.x & 31);
 }
 
+// kEndgame = false: EG is not read
+template <bool kEndgame>
+__global__ void __launch_bounds__(kThreads)
+    selfplay_advance_resign_kernel(const bz_selfplay_state S, const bz_tree_pools P, uint8_t *action_out, uint64_t cells,
+                                   const __grid_constant__ bz_selfplay_endgame_state EG,
+                                   const __grid_constant__ bz_selfplay_resign_state R) {
+    const int s = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (s >= S.n_games) return;
+    advance_slot<kEndgame, true>(S, P, action_out, cells, &EG, s, threadIdx.x & 31, &R);
+}
+
 // ---- the endgame queue: one solver ply of every pending game -----------------------------------------------------------
 // a warp per entry i < count: record the position with pi = 1/k on each of the k moves whose value is the root value
-// (a forced pass: one-hot on 64), play the solver's first best move, flush a finished game (ply = -1 marks the entry)
+// (a forced pass: one-hot on 64), play the solver's first best move, flush a finished game (ply = -1 marks the entry).
+// kResign: the record's q is NaN, and the flush carries the q rows (R->eg_hist_q) to the replay buffer.
+template <bool kResign>
 __global__ void __launch_bounds__(kThreads)
     endgame_ply_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_endgame_state EG,
-                       const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value, uint64_t cells) {
+                       const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value, uint64_t cells,
+                       const __grid_constant__ bz_selfplay_resign_state R) {
     const int i = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
     if (i >= *EG.count) return;
     const int lane = threadIdx.x & 31;
@@ -272,6 +351,7 @@ __global__ void __launch_bounds__(kThreads)
         EG.hist_opp[h] = opp;
         EG.hist_player[h] = (int8_t)player;
         EG.hist_action[h] = (uint8_t)action;
+        if constexpr (kResign) R.eg_hist_q[h] = __int_as_float(0x7FC00000);
         atomicAdd(&EG.counters[1], 1ull);
     }
     apply_legal(me, opp, action);  // the next mover's view
@@ -287,8 +367,8 @@ __global__ void __launch_bounds__(kThreads)
         }
         return;
     }
-    flush_game(S, EG.hist_me, EG.hist_opp, EG.hist_player, EG.hist_pi, b, EG.max_plies, nrec, gid, me, opp, player,
-               lane);
+    flush_game<kResign>(S, EG.hist_me, EG.hist_opp, EG.hist_player, EG.hist_pi, b, EG.max_plies, nrec, gid,
+                        disc_winner(me, opp, player), lane, &R, R.eg_hist_q);
     if (lane == 0) {
         EG.ply[i] = -1;
         atomicAdd(&EG.counters[3], 1ull);
@@ -693,6 +773,14 @@ int check_endgame(const bz_selfplay_state *s, const bz_selfplay_endgame_state *e
     return BZ_OK;
 }
 
+int check_resign(const bz_selfplay_endgame_state *e, const bz_selfplay_resign_state *r) {
+    if (!r) return BZ_ERR_ARG;
+    if (!(r->threshold >= -1.0f && r->threshold <= 1.0f)) return BZ_ERR_ARG;  // NaN fails both
+    if (r->audit_below > (1ull << 32)) return BZ_ERR_ARG;
+    if (!r->hist_q || !r->rp_q || !r->counters || (e && !r->eg_hist_q)) return BZ_ERR_ARG;
+    return BZ_OK;
+}
+
 int check_state(const bz_selfplay_state *s) {
     if (!s) return BZ_ERR_ARG;
     if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
@@ -747,6 +835,31 @@ int bz_selfplay_advance_endgame(const bz_selfplay_state *st, const bz_selfplay_e
     return launch_rc();
 }
 
+int bz_selfplay_advance_resign(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                               const bz_selfplay_resign_state *rs, const bz_tree_pools *pools, uint8_t *action_out,
+                               bz_stream_t stream) {
+    int rc = check_state(st);
+    if (rc != BZ_OK) return rc;
+    if (eg && (rc = check_endgame(st, eg)) != BZ_OK) return rc;
+    rc = check_resign(eg, rs);
+    if (rc != BZ_OK) return rc;
+    if (!pools || pools->game != BZ_GAME_REVERSI || pools->n_trees != st->n_games || pools->board_size != st->board_size ||
+        !pools->root_meta || !pools->arena)
+        return BZ_ERR_ARG;
+    if (st->n_games == 0) return BZ_OK;
+    const unsigned grid = (st->n_games + kWarpsPerCta - 1) / kWarpsPerCta;
+    const uint64_t cells = cell_mask(st->board_size);
+    if (eg) {
+        selfplay_advance_resign_kernel<true><<<grid, kThreads, 0, as_stream(stream)>>>(*st, *pools, action_out, cells, *eg,
+                                                                                      *rs);
+    } else {
+        const bz_selfplay_endgame_state none = {};
+        selfplay_advance_resign_kernel<false><<<grid, kThreads, 0, as_stream(stream)>>>(*st, *pools, action_out, cells, none,
+                                                                                       *rs);
+    }
+    return launch_rc();
+}
+
 // the solve's workspace, then its action [cap], value [cap] and move values [cap, 65], each 16-byte aligned
 static int64_t endgame_play_align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
 
@@ -756,12 +869,14 @@ int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap) {
            endgame_play_align16(cap * A);
 }
 
-static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace, bool wld,
-                        bz_stream_t stream) {
+// rs: NULL without resignation
+static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                        const bz_selfplay_resign_state *rs, void *workspace, bool wld, bz_stream_t stream) {
     int rc = check_state(st);
     if (rc != BZ_OK) return rc;
     rc = check_endgame(st, eg);
     if (rc != BZ_OK) return rc;
+    if (rs && (rc = check_resign(eg, rs)) != BZ_OK) return rc;
     if (!workspace) return BZ_ERR_ARG;
     if (!aligned16(workspace)) return BZ_ERR_UNALIGNED;
     const int64_t cap = eg->cap;
@@ -775,8 +890,13 @@ static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_s
         rc = endgame_launch_live(eg->me, eg->opp, cap, eg->count, st->board_size, workspace, action, value, move_value, wld,
                                  s);
         if (rc != BZ_OK) return rc;
-        endgame_ply_kernel<<<(unsigned)((cap + kWarpsPerCta - 1) / kWarpsPerCta), kThreads, 0, s>>>(*st, *eg, action, value,
-                                                                                                    move_value, cells);
+        const unsigned grid = (unsigned)((cap + kWarpsPerCta - 1) / kWarpsPerCta);
+        if (rs) {
+            endgame_ply_kernel<true><<<grid, kThreads, 0, s>>>(*st, *eg, action, value, move_value, cells, *rs);
+        } else {
+            const bz_selfplay_resign_state none = {};
+            endgame_ply_kernel<false><<<grid, kThreads, 0, s>>>(*st, *eg, action, value, move_value, cells, none);
+        }
         endgame_compact_kernel<<<1, 1024, 0, s>>>(*eg);
         rc = launch_rc();
         if (rc != BZ_OK) return rc;
@@ -786,12 +906,18 @@ static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_s
 
 int bz_selfplay_endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
                              bz_stream_t stream) {
-    return endgame_play(st, eg, workspace, false, stream);
+    return endgame_play(st, eg, nullptr, workspace, false, stream);
 }
 
 int bz_selfplay_endgame_play_wld(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg, void *workspace,
                                  bz_stream_t stream) {
-    return endgame_play(st, eg, workspace, true, stream);
+    return endgame_play(st, eg, nullptr, workspace, true, stream);
+}
+
+int bz_selfplay_endgame_play_resign(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                    const bz_selfplay_resign_state *rs, void *workspace, int wld, bz_stream_t stream) {
+    if (!rs) return BZ_ERR_ARG;
+    return endgame_play(st, eg, rs, workspace, wld != 0, stream);
 }
 
 int bz_match_init(const bz_match_state *st, bz_stream_t stream) {

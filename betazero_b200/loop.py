@@ -20,7 +20,11 @@ the exact solver once a searched move leaves at most E empty squares, and runs a
 plies (``selfplay.BatchedSelfPlay``); the line then has an ``endgame`` entry with the solver's counts and the time of its
 phases.  ``--endgame-solve wld`` runs the win/draw/loss solver for both instead of the exact one (cheaper; the handover's
 pi is then uniform over the moves that keep the result, and ``eval_endgame`` reports ``wld_accuracy`` only); both
-entries name the solver.
+entries name the solver.  With ``--resign V`` a self-play game that is not audited resigns at its first searched ply whose
+q (W / N of the most visited root edge) is below V (-1: audit only); ``--resign-audit F`` games never resign and measure
+the false positives, and ``--resign-fp P`` sets the next iteration's threshold from this iteration's gathered audited
+games (``resign.calibrate``: the same on every rank, since every rank gathers the same replay).  The line then has a
+``resign`` entry, and the checkpoint's ``extra`` holds the next threshold, which ``--resume`` restores.
 """
 from __future__ import annotations
 
@@ -35,7 +39,7 @@ from types import SimpleNamespace
 import torch
 
 from . import dist as bzd
-from . import endgame, match, mcts, minimax, net, selfplay, train
+from . import endgame, match, mcts, minimax, net, resign, selfplay, train
 
 
 def default_args(**over) -> SimpleNamespace:
@@ -43,7 +47,7 @@ def default_args(**over) -> SimpleNamespace:
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
                         reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None, endgame_empties=0, endgame_every=8,
-                        endgame_solve="exact")
+                        endgame_solve="exact", resign=None, resign_audit=0.1, resign_fp=None)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -81,10 +85,21 @@ class LoopState:
         self.model = net.make_net(args.net, hidden=args.hidden, seed=args.seed)
         self.master = net.make_net(args.net, hidden=args.hidden, seed=args.seed, dtype=torch.float32)  # fp32 master weights
         self.opt = torch.optim.Adam(self.master.parameters(), lr=args.lr)  # the reference's optimiser family (SL/train.py:87)
+        # resignation: --resign V, or -1 (audit only) when only --resign-fp is given; None = off
+        threshold, fp = getattr(args, "resign", None), getattr(args, "resign_fp", None)
+        if fp is not None and not float(fp) >= 0.0:
+            raise ValueError(f"resign_fp must be a false-positive rate >= 0; got {fp}")
+        if threshold is None and fp is not None:
+            threshold = -1.0
+        if threshold is not None:
+            threshold = resign.check_threshold(threshold)
         self.first_iteration = 0
         if args.resume:
             self.first_iteration = train.load_checkpoint(args.resume, self.master, self.opt)
             self._publish()
+            kept = torch.load(args.resume, map_location="cpu", weights_only=True).get("extra", {}).get("resign_threshold")
+            if threshold is not None and kept is not None:
+                threshold = resign.check_threshold(kept)
         self.evaluator = (mcts.FusedNetEvaluator(self.model) if hasattr(self.model, "forward_raw")
                           else mcts.NetEvaluator(self.model))
         self.sp = selfplay.BatchedSelfPlay(args.games, args.sims, self.evaluator, board_size=args.size,
@@ -92,7 +107,8 @@ class LoopState:
                                            n_leaves=args.leaves, reuse=bool(getattr(args, "reuse", False)),
                                            graph_unroll=min(16, max(1, args.sims // args.leaves - 1)),
                                            endgame_empties=int(getattr(args, "endgame_empties", 0)),
-                                           endgame_every=int(getattr(args, "endgame_every", 8)), endgame_solve=solve)
+                                           endgame_every=int(getattr(args, "endgame_every", 8)), endgame_solve=solve,
+                                           resign_threshold=threshold, resign_audit=float(getattr(args, "resign_audit", 0.1)))
         self.sp.prepare()
 
     @torch.no_grad()
@@ -116,6 +132,7 @@ def run_iteration(st: LoopState, it: int) -> dict:
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
     torch.cuda.synchronize()
     eg_ms0, eg_stats0 = (sp.endgame_ms(), sp.stats()) if sp.eg is not None else (0.0, None)
+    rs_stats0, rs_threshold = (sp.stats(), sp.resign_threshold) if sp.rs is not None else (None, None)
     t0 = time.perf_counter()
     ev[0].record()
     for _ in range(args.plies):
@@ -128,6 +145,18 @@ def run_iteration(st: LoopState, it: int) -> dict:
     gather_info = dict(bzd.last_gather)
     ev[2].record()
     n = replay["me"].shape[0]
+    resign_line = None
+    if sp.rs is not None:
+        # the audited games of the gathered replay: every rank holds the same records, so every rank computes the same
+        # false-positive rate and the same next threshold
+        recs = resign.with_audit(replay, args.seed, sp.resign_audit)
+        fp_target = getattr(args, "resign_fp", None)
+        if fp_target is not None:
+            sp.set_resign_threshold(resign.calibrate(recs, float(fp_target), keep=rs_threshold))
+        n_games = int(torch.unique(replay["game"]).numel()) if n else 0
+        resign_line = {"threshold": rs_threshold, "next_threshold": sp.resign_threshold, "audit": sp.resign_audit,
+                       "fp_target": fp_target, "fp": resign.false_positive_rate(recs, rs_threshold),
+                       "audited_games": resign.audited_games(recs), "plies_per_game": n / n_games if n_games else None}
     # --eval-games: the net that played this iteration's self-play, to be matched against the trained one
     snapshot = copy.deepcopy(st.model) if getattr(args, "eval_games", 0) and rank == 0 else None
     losses = []
@@ -172,6 +201,10 @@ def run_iteration(st: LoopState, it: int) -> dict:
                            "pending": stats["endgame_pending"],
                            "overflow": stats["endgame_overflow"] - eg_stats0["endgame_overflow"],
                            "ms": sp.endgame_ms() - eg_ms0}
+    if resign_line is not None:
+        resign_line["resigned_local"] = stats["resigned"] - rs_stats0["resigned"]
+        resign_line["audited_local"] = stats["audited"] - rs_stats0["audited"]
+        line["resign"] = resign_line
     if snapshot is not None:
         t_eval = time.perf_counter()
         r = match.BatchedMatch(st.model, snapshot, args.eval_games, args.sims, n_leaves=args.leaves, board_size=args.size,
@@ -196,8 +229,10 @@ def run_iteration(st: LoopState, it: int) -> dict:
         line["warnings"] = [str(w.message) for w in caught]
     if args.checkpoint and rank == 0:
         path = checkpoint_path(args.checkpoint, it)
-        train.save_checkpoint(path, st.master, st.opt, iteration=it + 1,
-                              extra={"games_per_gpu": args.games, "sims_per_move": args.sims, "world": world})
+        extra = {"games_per_gpu": args.games, "sims_per_move": args.sims, "world": world}
+        if sp.rs is not None:
+            extra["resign_threshold"] = sp.resign_threshold
+        train.save_checkpoint(path, st.master, st.opt, iteration=it + 1, extra=extra)
         line["checkpoint"] = path
     return line
 
@@ -253,6 +288,14 @@ def main():
     ap.add_argument("--endgame-solve", choices=selfplay.ENDGAME_SOLVES, default=d.endgame_solve,
                     help="the solver of --endgame-empties and --eval-endgame: exact (the final margin) or wld (win / "
                          "draw / loss only: cheaper; handover pi uniform over the moves that keep the result)")
+    ap.add_argument("--resign", type=float, default=d.resign, metavar="V",
+                    help="a self-play game that is not audited resigns at its first searched ply whose q (W / N of the "
+                         "most visited root edge, the mover's view) is below V (-1 .. 1; -1 = audit only; default off)")
+    ap.add_argument("--resign-audit", type=float, default=d.resign_audit, metavar="F",
+                    help="with --resign: the fraction of games that never resign and measure its false positives")
+    ap.add_argument("--resign-fp", type=float, default=d.resign_fp, metavar="P",
+                    help="set the threshold after every iteration from its audited games: the largest one whose "
+                         "false-positive rate stays at most P (switches resignation on, from --resign or -1)")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

@@ -15,6 +15,13 @@ the feature, the solver's records carry pi uniform over the optimal moves, and e
 handover position.  ``endgame_solve="wld"`` hands the games to the win/draw/loss solver instead (bz_selfplay_endgame_play_wld):
 cheaper, with the same z, but pi is uniform over every move that keeps the result rather than over the moves that
 maximise the final margin -- a label with less information, which is why the exact solver stays the default.
+
+Resignation (opt-in, ``resign_threshold=v``): a game that is not audited resigns at its first searched ply whose q -- W / N
+of the most visited root edge, the mover's view -- is below v; the ply is recorded, the mover loses and the slot
+restarts (bz_selfplay_advance_resign).  A fraction ``resign_audit`` of the games (by a Philox draw on the game id) never
+resigns: they measure how often resigning would have been wrong (``resign.false_positive_rate``, ``resign.calibrate``).
+Every record then carries its ply's q (NaN for solver-played plies) and ``drain_replay`` returns it as "q".  The
+threshold can change between plies (``set_resign_threshold``): the state is passed by value at every launch.
 """
 from __future__ import annotations
 
@@ -23,7 +30,8 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import BzSelfplayEndgameState, BzSelfplayState
+from . import resign as _resign
+from ._lib import BzSelfplayEndgameState, BzSelfplayResignState, BzSelfplayState
 from .mcts import BatchedMCTS, TreePools
 
 N_ACTIONS = 65
@@ -52,8 +60,13 @@ class BatchedSelfPlay:
                  arena_units: int | None = None, use_graph: bool = True, graph_unroll: int = 16,
                  dirichlet_alpha: float = 0.0, dirichlet_eps: float = 0.25, n_leaves: int = 1, device="cuda",
                  one_launch: bool | None = None, reuse: bool = False, endgame_empties: int = 0, endgame_every: int = 8,
-                 endgame_cap: int | None = None, endgame_solve: str = "exact"):
+                 endgame_cap: int | None = None, endgame_solve: str = "exact", resign_threshold: float | None = None,
+                 resign_audit: float = 0.1):
         self.n_games, self.n_sims, self.board_size = int(n_games), int(n_sims), int(board_size)
+        self.resign_audit = float(resign_audit)
+        self._audit_below = _resign.audit_below(resign_audit)
+        if resign_threshold is not None:
+            resign_threshold = _resign.check_threshold(resign_threshold)
         self.endgame_empties = check_endgame_empties(endgame_empties, board_size)
         self.endgame_solve = check_endgame_solve(endgame_solve)
         self.endgame_every = int(endgame_every)
@@ -110,6 +123,9 @@ class BatchedSelfPlay:
         self._eg_ms = 0.0
         if self.endgame_empties:
             self._init_endgame()
+        self.rs = None
+        if resign_threshold is not None:
+            self._init_resign(resign_threshold)
 
     def _init_endgame(self) -> None:
         Q, dev = self.endgame_cap, self.device
@@ -134,6 +150,31 @@ class BatchedSelfPlay:
         self.eg = g
         self._eg_ref = C.byref(g)
 
+    def _init_resign(self, threshold: float) -> None:
+        dev = self.device
+        self.hist_q = torch.empty(max(self.n_games, 1) * self.max_plies, dtype=torch.float32, device=dev)
+        self.eg_hist_q = (torch.empty(self.endgame_cap * self.max_plies, dtype=torch.float32, device=dev)
+                          if self.eg is not None else None)
+        self.rp_q = torch.empty(max(self.replay_cap, 1), dtype=torch.float32, device=dev)
+        self.resign_counters = torch.zeros(2, dtype=torch.int64, device=dev)
+        r = BzSelfplayResignState()
+        r.threshold, r.audit_below = threshold, self._audit_below
+        r.hist_q, r.rp_q, r.counters = self.hist_q.data_ptr(), self.rp_q.data_ptr(), self.resign_counters.data_ptr()
+        r.eg_hist_q = self.eg_hist_q.data_ptr() if self.eg_hist_q is not None else None
+        self.rs = r
+        self._rs_ref = C.byref(r)
+
+    @property
+    def resign_threshold(self) -> float | None:
+        """the threshold of the next plies (float32), None when resignation is off"""
+        return None if self.rs is None else float(self.rs.threshold)
+
+    def set_resign_threshold(self, v: float) -> None:
+        """a new threshold in [-1, 1] for the following plies (resignation must have been switched on)"""
+        if self.rs is None:
+            raise RuntimeError("set_resign_threshold needs BatchedSelfPlay(resign_threshold=...)")
+        self.rs.threshold = _resign.check_threshold(v)
+
     # -- one lockstep ply for every game ----------------------------------------------------------
     def search(self) -> None:
         if (self.mcts.use_graph and self.mcts._graph is None and not self.mcts.one_launch
@@ -147,6 +188,16 @@ class BatchedSelfPlay:
         self._moves += 1
 
     def advance(self) -> None:
+        if self.rs is not None:
+            _lib.check(self._L.bz_selfplay_advance_resign(self._ref, self._eg_ref if self.eg is not None else None,
+                                                          self._rs_ref, self.pools._ref, _lib.dptr(self.last_action),
+                                                          _lib.stream_ptr()), "bz_selfplay_advance_resign")
+            self.launches += 1
+            if self.eg is not None:
+                self._advances += 1
+                if self._advances % self.endgame_every == 0:
+                    self.endgame_play()
+            return
         if self.eg is None:
             _lib.check(self._L.bz_selfplay_advance(self._ref, self.pools._ref, _lib.dptr(self.last_action),
                                                    _lib.stream_ptr()), "bz_selfplay_advance")
@@ -167,8 +218,14 @@ class BatchedSelfPlay:
             raise RuntimeError("endgame_play needs endgame_empties > 0")
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
-        name = "bz_selfplay_endgame_play_wld" if self.endgame_solve == "wld" else "bz_selfplay_endgame_play"
-        _lib.check(getattr(self._L, name)(self._ref, self._eg_ref, _lib.dptr(self.eg_workspace), _lib.stream_ptr()), name)
+        if self.rs is not None:
+            name = "bz_selfplay_endgame_play_resign"
+            _lib.check(self._L.bz_selfplay_endgame_play_resign(self._ref, self._eg_ref, self._rs_ref,
+                                                               _lib.dptr(self.eg_workspace), int(self.endgame_solve == "wld"),
+                                                               _lib.stream_ptr()), name)
+        else:
+            name = "bz_selfplay_endgame_play_wld" if self.endgame_solve == "wld" else "bz_selfplay_endgame_play"
+            _lib.check(getattr(self._L, name)(self._ref, self._eg_ref, _lib.dptr(self.eg_workspace), _lib.stream_ptr()), name)
         t1.record()
         self._eg_events.append((t0, t1))
         self.launches += 6 * 2 * self.endgame_empties  # per solver ply: the solve's four kernels, the move, the compaction
@@ -199,6 +256,9 @@ class BatchedSelfPlay:
         eg = self.eg_counters.cpu().tolist() if self.eg is not None else [0, 0, 0, 0]
         out.update({"endgame_games": eg[3], "endgame_plies": eg[1],
                     "endgame_pending": int(self.eg_count.item()) if self.eg is not None else 0, "endgame_overflow": eg[2]})
+        # resignation: games resigned, audited games finished (both 0 when it is off)
+        rc = self.resign_counters.cpu().tolist() if self.rs is not None else [0, 0]
+        out.update({"resigned": rc[0], "audited": rc[1]})
         return out
 
     def drain_replay(self) -> dict:
@@ -217,6 +277,8 @@ class BatchedSelfPlay:
             "pi": self.rp_pi[: n * N_ACTIONS].view(n, N_ACTIONS).clone(),
             "z": self.rp_z[:n].clone(), "game": self.rp_game[:n].clone(), "ply": self.rp_ply[:n].clone(),
         }
+        if self.rs is not None:
+            out["q"] = self.rp_q[:n].clone()  # q of the record's ply (NaN for solver-played plies)
         self.counters[0] = 0
         return out
 

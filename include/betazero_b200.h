@@ -398,6 +398,40 @@ int bz_selfplay_endgame_play_wld(const bz_selfplay_state *st, const bz_selfplay_
                                  bz_stream_t stream);
 int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap);
 
+/* Resignation (opt-in): a self-play game whose search has called the result stops early.
+ * q of a searched ply: a* is the most visited root action, lowest action id on ties (the greedy pick, also on plies
+ * that sample the move); q = float32(W[a*]) / float32(N[a*]) with one correctly rounded division, the mover's view
+ * (the value is negated before it is added to the edge into a node).  A root with no visits has q = NaN.
+ * Game g is AUDITED iff bz_philox_u32(seed, g, 0xFFFFFFFF) < audit_below (the counter is never a ply, so the draw is
+ * independent of move sampling); an audited game never resigns.  A searched ply of a game that is not audited RESIGNS
+ * iff q < threshold (float32 compare; -1 never fires): the position is recorded as always (board, pi, action), the
+ * mover loses (winner = -player), the game is flushed like a finished game (z = winner * player for every record) and
+ * the slot restarts.  The move is not played; action_out holds the picked action.  Resignation is checked before the
+ * move is applied, so before the endgame handover test of the same ply; solver-played plies never resign.
+ * Every replay record carries its ply's q in rp_q (NaN for solver-played records).  Oracle:
+ * oracle/selfplay_resign_ref.py. */
+typedef struct bz_selfplay_resign_state {
+    float threshold;      /* in [-1, 1] */
+    int32_t reserved;
+    uint64_t audit_below; /* 0 .. 2^32: floor(fraction * 2^32) */
+    float *hist_q;        /* [n_games * max_plies]: q of the slot's history rows */
+    float *eg_hist_q;     /* [eg->cap * max_plies]: q of the endgame queue's history blocks; NULL without a handover */
+    float *rp_q;          /* [replay_cap]: q of the replay records */
+    /* device uint64 [2]: 0 games resigned, 1 audited games finished (flushed, or dropped by a full replay buffer) */
+    unsigned long long *counters;
+} bz_selfplay_resign_state;
+
+/* bz_selfplay_advance (eg NULL) or bz_selfplay_advance_endgame (eg given) with resignation.  counters start at zero
+ * (the caller zeroes them once).  BZ_ERR_ARG: what those refuse, a NULL rs, a NaN threshold or one outside [-1, 1],
+ * audit_below > 2^32, a NULL hist_q, rp_q or counters, a NULL eg_hist_q when eg is given. */
+int bz_selfplay_advance_resign(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                               const bz_selfplay_resign_state *rs, const bz_tree_pools *pools, uint8_t *action_out,
+                               bz_stream_t stream);
+/* bz_selfplay_endgame_play (wld = 0) or bz_selfplay_endgame_play_wld (wld != 0) with the q rows carried through: a
+ * solver ply's q is NaN.  Same refusals as bz_selfplay_advance_resign with eg given, and those of the solver phase. */
+int bz_selfplay_endgame_play_resign(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                    const bz_selfplay_resign_state *rs, void *workspace, int wld, bz_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
  * the same launches; a net-versus-net match is the tournament of two entrants and the one pairing (0, 1).  Game pair i
