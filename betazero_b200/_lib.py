@@ -67,6 +67,17 @@ class BzSelfplayResignState(C.Structure):
     N_SCALARS = 3
 
 
+class BzSelfplayCapState(C.Structure):
+    """Mirror of ``bz_selfplay_cap_state`` (include/betazero_b200.h)."""
+
+    _fields_ = [
+        ("full_below", C.c_uint64), ("n_trees", C.c_int32), ("reserved", C.c_int32),
+        ("tree_of_slot", ptr), ("root_me", ptr), ("root_opp", ptr), ("pair_entrant", ptr),
+        ("hist_full", ptr), ("eg_hist_full", ptr), ("rp_full", ptr), ("counters", ptr),
+    ]
+    N_SCALARS = 3
+
+
 class BzMatchState(C.Structure):
     """Mirror of ``bz_match_state`` (include/betazero_b200.h)."""
 
@@ -94,6 +105,7 @@ _PP = C.POINTER(BzTreePools)
 _SP = C.POINTER(BzSelfplayState)
 _EP = C.POINTER(BzSelfplayEndgameState)
 _RP = C.POINTER(BzSelfplayResignState)
+_CP = C.POINTER(BzSelfplayCapState)
 _MP = C.POINTER(BzMatchState)
 _TP = C.POINTER(BzTournamentState)
 SIGNATURES = {
@@ -120,6 +132,7 @@ SIGNATURES = {
     "bz_mcts_root_edges": [_PP, ptr, ptr, ptr, ptr],
     "bz_mcts_best_action": [_PP, ptr, ptr],
     "bz_mcts_root_noise": [_PP, ptr, _F, ptr],
+    "bz_mcts_root_noise_entrant": [_PP, ptr, _F, ptr, _INT, ptr],
     "bz_mcts_reroot": [_PP, ptr, ptr, ptr, ptr, _INT, ptr, ptr],
     "bz_hash_eval": [ptr, ptr, _U64, _INT, ptr, ptr, _I64, ptr],
     "bz_selfplay_init": [_SP, _I64, ptr],
@@ -130,6 +143,9 @@ SIGNATURES = {
     "bz_selfplay_endgame_workspace_bytes": [_I64],
     "bz_selfplay_advance_resign": [_SP, _EP, _RP, _PP, ptr, ptr],
     "bz_selfplay_endgame_play_resign": [_SP, _EP, _RP, ptr, _INT, ptr],
+    "bz_selfplay_cap_layout": [_SP, _CP, ptr],
+    "bz_selfplay_advance_cap": [_SP, _EP, _RP, _CP, _PP, ptr, ptr],
+    "bz_selfplay_endgame_play_cap": [_SP, _EP, _RP, _CP, ptr, _INT, ptr],
     "bz_match_init": [_MP, ptr],
     "bz_match_advance": [_MP, _PP, ptr],
     "bz_tournament_layout": [_TP, ptr],

@@ -47,14 +47,22 @@ __device__ __forceinline__ bool resign_audited(uint64_t seed, int64_t gid, uint6
     return (uint64_t)philox_u32(seed, (uint64_t)gid, 0xFFFFFFFFu) < audit_below;
 }
 
+// the ply `ply` of game `gid` is searched with the full budget iff philox_u32(seed, gid, 0x80000000 | ply) < full_below:
+// the counter is never a ply (< 128) and never the audit draw's 0xFFFFFFFF
+__device__ __forceinline__ bool cap_full(uint64_t seed, int64_t gid, int ply, uint64_t full_below) {
+    return (uint64_t)philox_u32(seed, (uint64_t)gid, 0x80000000u | (uint32_t)ply) < full_below;
+}
+
 // a warp: the game `gid` has ended with `winner` (absolute: +1 X, -1 O, 0 draw); copy its nrec history rows, block `block`
 // of max_plies rows in hist_*, to the replay buffer (whole or not at all); lane 0 counts.  kResign: the q rows (hist_q)
-// go to R->rp_q as well, and an audited game is counted in R->counters[1].
-template <bool kResign = false>
+// go to R->rp_q as well, and an audited game is counted in R->counters[1].  kCap: the flag rows (hist_full) go to
+// Cs->rp_full.
+template <bool kResign = false, bool kCap = false>
 __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uint64_t *hist_me, const uint64_t *hist_opp,
                                            const int8_t *hist_player, const float *hist_pi, int block, int max_plies,
                                            int nrec, int64_t gid, int winner, int lane,
-                                           const bz_selfplay_resign_state *R = nullptr, const float *hist_q = nullptr) {
+                                           const bz_selfplay_resign_state *R = nullptr, const float *hist_q = nullptr,
+                                           const bz_selfplay_cap_state *Cs = nullptr, const uint8_t *hist_full = nullptr) {
     // counters[0] = rows COMMITTED to the replay buffer: a game reserves its rows with a compare-and-swap and takes
     // nothing when it does not fit, so [0, counters[0]) never contains a row that no game wrote
     unsigned long long rb = ~0ull;  // ~0: no room, the game is dropped (counted in counters[5])
@@ -87,6 +95,7 @@ __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uin
             S.rp_game[rb + r] = gid;
             S.rp_ply[rb + r] = (int16_t)r;
             if constexpr (kResign) R->rp_q[rb + r] = hist_q[h0 + r];
+            if constexpr (kCap) Cs->rp_full[rb + r] = hist_full[h0 + r];
         }
         const int64_t nf = (int64_t)nrec * A;  // pi rows are contiguous in both buffers
         const float *src = hist_pi + h0 * A;
@@ -99,11 +108,12 @@ __device__ __forceinline__ void flush_game(const bz_selfplay_state &S, const uin
 
 // a warp: move the game of slot s -- (me, opp) with `player` to move, nrec history rows -- to the next free entry of the
 // endgame queue, its rows to the entry's history block (row == entry: the queue fills from an empty state between solver
-// phases); false, and counted, when the queue is full.  kResign: the q rows go to R->eg_hist_q as well.
-template <bool kResign>
+// phases); false, and counted, when the queue is full.  kResign: the q rows go to R->eg_hist_q as well.  kCap: the flag
+// rows go to Cs->eg_hist_full.
+template <bool kResign, bool kCap = false>
 __device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_selfplay_endgame_state &EG, int s, int lane,
                                          uint64_t me, uint64_t opp, int player, int nrec, int64_t gid,
-                                         const bz_selfplay_resign_state *R) {
+                                         const bz_selfplay_resign_state *R, const bz_selfplay_cap_state *Cs = nullptr) {
     int q = -1;
     if (lane == 0) {
         int cur = *EG.count;
@@ -128,6 +138,7 @@ __device__ __forceinline__ bool handover(const bz_selfplay_state &S, const bz_se
         EG.hist_player[dst + r] = S.hist_player[src + r];
         EG.hist_action[dst + r] = S.hist_action[src + r];
         if constexpr (kResign) R->eg_hist_q[dst + r] = R->hist_q[src + r];
+        if constexpr (kCap) Cs->eg_hist_full[dst + r] = Cs->hist_full[src + r];
     }
     const int64_t nf = (int64_t)nrec * A;
     for (int64_t i = lane; i < nf; i += 32) EG.hist_pi[dst * A + i] = S.hist_pi[src * A + i];
@@ -160,16 +171,23 @@ __device__ __forceinline__ unsigned greedy_action(int Ne, unsigned act, int N32,
 // game is flushed and its slot restarts.  kEndgame: a game whose move leaves EG->empties empties or fewer for the first
 // time goes to the endgame queue instead (and its slot restarts) when the queue has room.  kResign: the ply's q (W / N of
 // the most visited root edge, the mover's view) is recorded, and a game that is not audited resigns when q < threshold:
-// the record is kept, the mover loses, the game is flushed and the slot restarts before the move is applied.
-template <bool kEndgame, bool kResign = false>
+// the record is kept, the mover loses, the game is flushed and the slot restarts before the move is applied.  kCap: the
+// search of slot s is tree Cs->tree_of_slot[s] of the pools, and the ply's flag (full or fast) goes to Cs->hist_full.
+template <bool kEndgame, bool kResign = false, bool kCap = false>
 __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const bz_tree_pools &P, uint8_t *action_out,
                                              uint64_t cells, const bz_selfplay_endgame_state *EG, int s, int lane,
-                                             const bz_selfplay_resign_state *R = nullptr) {
+                                             const bz_selfplay_resign_state *R = nullptr,
+                                             const bz_selfplay_cap_state *Cs = nullptr) {
 
     // root statistics: lane i holds edge i (ascending action id); a 33rd edge is read uniformly
-    const uint32_t rmeta = P.root_meta[s];
+    int tree = s;
+    if constexpr (kCap) {
+        tree = Cs->tree_of_slot[s];
+        BZ_CHECK(tree >= 0 && tree < P.n_trees, 26);  // tree of the slot
+    }
+    const uint32_t rmeta = P.root_meta[tree];
     const int n = (int)((rmeta >> BZ_META_N_SHIFT) & 63u);
-    const uint32_t *blk = P.arena + (int64_t)s * P.arena_units * 8 + (int64_t)(rmeta >> BZ_META_OFF_SHIFT) * 8;
+    const uint32_t *blk = P.arena + (int64_t)tree * P.arena_units * 8 + (int64_t)(rmeta >> BZ_META_OFF_SHIFT) * 8;
     int Ne = 0, N32 = 0;
     unsigned act = 127u, act32 = 127u;
     if (lane < n) {
@@ -247,13 +265,14 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
         S.hist_action[h] = (uint8_t)action;
         if (action_out) action_out[s] = (uint8_t)action;
         if constexpr (kResign) R->hist_q[h] = q;
+        if constexpr (kCap) Cs->hist_full[h] = (uint8_t)cap_full(S.seed, gid, ply, Cs->full_below);
     }
 
     // --- resignation (kResign): before the move is applied, so before the handover test; NaN never compares below -----
     if constexpr (kResign) {
         if (q < R->threshold && !resign_audited(S.seed, gid, R->audit_below)) {
-            flush_game<true>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, ply + 1, gid, -player,
-                             lane, R, R->hist_q);
+            flush_game<true, kCap>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, ply + 1, gid,
+                                   -player, lane, R, R->hist_q, Cs, kCap ? Cs->hist_full : nullptr);
             if (lane == 0) {
                 atomicAdd(&R->counters[0], 1ull);
                 restart_slot(S, s, gid);
@@ -272,7 +291,7 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
             // the first position at E empties or fewer (the move placed a disc): a game the full queue refuses is not
             // offered again and is searched to its end
             if (__popcll(cells) - __popcll(me | opp) <= EG->empties && EG->empties < __popcll(cells) - __popcll(occupied) &&
-                handover<kResign>(S, *EG, s, lane, me, opp, -player, nrec, gid, R)) {
+                handover<kResign, kCap>(S, *EG, s, lane, me, opp, -player, nrec, gid, R, Cs)) {
                 if (lane == 0) restart_slot(S, s, gid);
                 return;
             }
@@ -288,8 +307,9 @@ __device__ __forceinline__ void advance_slot(const bz_selfplay_state &S, const b
     }
 
     // --- finished: score, flush the history to the replay buffer, restart the slot ----------------
-    flush_game<kResign>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, nrec, gid,
-                        disc_winner(me, opp, player), lane, R, kResign ? R->hist_q : nullptr);
+    flush_game<kResign, kCap>(S, S.hist_me, S.hist_opp, S.hist_player, S.hist_pi, s, S.max_plies, nrec, gid,
+                              disc_winner(me, opp, player), lane, R, kResign ? R->hist_q : nullptr, Cs,
+                              kCap ? Cs->hist_full : nullptr);
     if (lane == 0) restart_slot(S, s, gid);
 }
 
@@ -319,18 +339,28 @@ __global__ void __launch_bounds__(kThreads)
     advance_slot<kEndgame, true>(S, P, action_out, cells, &EG, s, threadIdx.x & 31, &R);
 }
 
+// kEndgame = false: EG is not read; kResign = false: R is not read
+template <bool kEndgame, bool kResign>
+__global__ void __launch_bounds__(kThreads)
+    selfplay_advance_cap_kernel(const bz_selfplay_state S, const bz_tree_pools P, uint8_t *action_out, uint64_t cells,
+                                const __grid_constant__ bz_selfplay_endgame_state EG,
+                                const __grid_constant__ bz_selfplay_resign_state R,
+                                const __grid_constant__ bz_selfplay_cap_state Cs) {
+    const int s = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (s >= S.n_games) return;
+    advance_slot<kEndgame, kResign, true>(S, P, action_out, cells, &EG, s, threadIdx.x & 31, &R, &Cs);
+}
+
 // ---- the endgame queue: one solver ply of every pending game -----------------------------------------------------------
 // a warp per entry i < count: record the position with pi = 1/k on each of the k moves whose value is the root value
 // (a forced pass: one-hot on 64), play the solver's first best move, flush a finished game (ply = -1 marks the entry).
-// kResign: the record's q is NaN, and the flush carries the q rows (R->eg_hist_q) to the replay buffer.
-template <bool kResign>
-__global__ void __launch_bounds__(kThreads)
-    endgame_ply_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_endgame_state EG,
-                       const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value, uint64_t cells,
-                       const __grid_constant__ bz_selfplay_resign_state R) {
-    const int i = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
-    if (i >= *EG.count) return;
-    const int lane = threadIdx.x & 31;
+// kResign: the record's q is NaN, and the flush carries the q rows (R->eg_hist_q) to the replay buffer.  kCap: the
+// record's flag is 1 (an exact label), and the flush carries the flag rows (Cs->eg_hist_full).
+template <bool kResign, bool kCap>
+__device__ __forceinline__ void endgame_ply(const bz_selfplay_state &S, const bz_selfplay_endgame_state &EG, int i,
+                                            int lane, const uint8_t *solve_action, const int8_t *solve_value,
+                                            const int8_t *move_value, uint64_t cells, const bz_selfplay_resign_state *R,
+                                            const bz_selfplay_cap_state *Cs) {
     const int ply = EG.ply[i], player = EG.player[i], b = EG.row[i];
     const int64_t gid = EG.game_id[i];
     uint64_t me = EG.me[i], opp = EG.opp[i];
@@ -351,7 +381,8 @@ __global__ void __launch_bounds__(kThreads)
         EG.hist_opp[h] = opp;
         EG.hist_player[h] = (int8_t)player;
         EG.hist_action[h] = (uint8_t)action;
-        if constexpr (kResign) R.eg_hist_q[h] = __int_as_float(0x7FC00000);
+        if constexpr (kResign) R->eg_hist_q[h] = __int_as_float(0x7FC00000);
+        if constexpr (kCap) Cs->eg_hist_full[h] = 1;
         atomicAdd(&EG.counters[1], 1ull);
     }
     apply_legal(me, opp, action);  // the next mover's view
@@ -367,12 +398,34 @@ __global__ void __launch_bounds__(kThreads)
         }
         return;
     }
-    flush_game<kResign>(S, EG.hist_me, EG.hist_opp, EG.hist_player, EG.hist_pi, b, EG.max_plies, nrec, gid,
-                        disc_winner(me, opp, player), lane, &R, R.eg_hist_q);
+    flush_game<kResign, kCap>(S, EG.hist_me, EG.hist_opp, EG.hist_player, EG.hist_pi, b, EG.max_plies, nrec, gid,
+                              disc_winner(me, opp, player), lane, R, R->eg_hist_q, Cs, kCap ? Cs->eg_hist_full : nullptr);
     if (lane == 0) {
         EG.ply[i] = -1;
         atomicAdd(&EG.counters[3], 1ull);
     }
+}
+
+template <bool kResign>
+__global__ void __launch_bounds__(kThreads)
+    endgame_ply_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_endgame_state EG,
+                       const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value, uint64_t cells,
+                       const __grid_constant__ bz_selfplay_resign_state R) {
+    const int i = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (i >= *EG.count) return;
+    endgame_ply<kResign, false>(S, EG, i, threadIdx.x & 31, solve_action, solve_value, move_value, cells, &R, nullptr);
+}
+
+// kResign = false: R is not read
+template <bool kResign>
+__global__ void __launch_bounds__(kThreads)
+    endgame_ply_cap_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_endgame_state EG,
+                           const uint8_t *solve_action, const int8_t *solve_value, const int8_t *move_value,
+                           uint64_t cells, const __grid_constant__ bz_selfplay_resign_state R,
+                           const __grid_constant__ bz_selfplay_cap_state Cs) {
+    const int i = blockIdx.x * kWarpsPerCta + (threadIdx.x >> 5);
+    if (i >= *EG.count) return;
+    endgame_ply<kResign, true>(S, EG, i, threadIdx.x & 31, solve_action, solve_value, move_value, cells, &R, &Cs);
 }
 
 // one CTA: the live entries (ply >= 0) of [0, count) to the front, in order; count = their number.  In place: a chunk's
@@ -740,6 +793,93 @@ __global__ void __launch_bounds__(kLayoutThreads) tournament_layout_kernel(const
     }
 }
 
+// ---- self-play with randomized search budgets ----------------------------------------------------------------------------
+// one CTA: a two-key stable partition of the slots -- full slots (cap_full) to trees [0, n_full) in slot order, fast slots
+// to [fast0, fast0 + n_fast) in slot order, fast0 = n_full rounded up to a CTA pair (56 trees); empty boards (a finished
+// game: the search expands nothing there) on the padding [n_full, fast0) and after the fast range.  Ranks: ballots inside
+// a warp, the per-warp counts scanned by warp 0, a running base per key across the 512-slot chunks.  512 threads: the
+// Philox draw and the two running bases fit in registers without a spill.
+constexpr int kCapLayoutThreads = 512, kCapLayoutWarps = kCapLayoutThreads / 32;
+__global__ void __launch_bounds__(kCapLayoutThreads)
+    selfplay_cap_layout_kernel(const bz_selfplay_state S, const __grid_constant__ bz_selfplay_cap_state Cs) {
+    __shared__ unsigned wfull[kCapLayoutWarps], wfast[kCapLayoutWarps];  // [warp]: slots of the chunk, then the warp's first rank
+    __shared__ unsigned sum_full, sum_fast;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    // pass 1: full slots
+    unsigned mine = 0;
+    for (int s = tid; s < S.n_games; s += kCapLayoutThreads)
+        mine += cap_full(S.seed, S.game_id[s], S.ply[s], Cs.full_below);
+    mine = __reduce_add_sync(kFull, mine);
+    if (lane == 0) wfull[w] = mine;
+    __syncthreads();
+    if (w == 0) {
+        const unsigned v = __reduce_add_sync(kFull, lane < kCapLayoutWarps ? wfull[lane] : 0u);
+        if (lane == 0) sum_full = v;
+    }
+    __syncthreads();
+    const int n_full = (int)sum_full, n_fast = S.n_games - n_full;
+    const int fast0 = (n_full + kPairTrees - 1) / kPairTrees * kPairTrees;
+    // pass 2: trees of the slots
+    int base_full = 0, base_fast = fast0;
+    for (int s0 = 0; s0 < S.n_games; s0 += kCapLayoutThreads) {
+        const int s = s0 + tid;
+        const bool live = s < S.n_games;
+        const bool full = live && cap_full(S.seed, S.game_id[s], S.ply[s], Cs.full_below);
+        const unsigned bf = __ballot_sync(kFull, full), bs = __ballot_sync(kFull, live && !full);
+        __syncthreads();  // the previous chunk's ranks have been read
+        if (lane == 0) {
+            wfull[w] = __popc(bf);
+            wfast[w] = __popc(bs);
+        }
+        __syncthreads();
+        if (w == 0) {
+            const unsigned vf = lane < kCapLayoutWarps ? wfull[lane] : 0u, vs = lane < kCapLayoutWarps ? wfast[lane] : 0u;
+            unsigned inf = vf, ins = vs;
+            for (int d = 1; d < 32; d <<= 1) {
+                const unsigned uf = __shfl_up_sync(kFull, inf, d), us = __shfl_up_sync(kFull, ins, d);
+                if (lane >= d) {
+                    inf += uf;
+                    ins += us;
+                }
+            }
+            if (lane < kCapLayoutWarps) {
+                wfull[lane] = inf - vf;
+                wfast[lane] = ins - vs;
+            }
+            if (lane == 31) {
+                sum_full = inf;
+                sum_fast = ins;
+            }
+        }
+        __syncthreads();
+        if (live) {
+            const unsigned below = (1u << lane) - 1u;
+            const int t = full ? base_full + (int)(wfull[w] + __popc(bf & below))
+                               : base_fast + (int)(wfast[w] + __popc(bs & below));
+            BZ_CHECK(t >= 0 && t < Cs.n_trees && (full ? t < n_full : t >= fast0 && t < fast0 + n_fast), 27);  // tree row
+            Cs.tree_of_slot[s] = t;
+            Cs.root_me[t] = S.me[s];
+            Cs.root_opp[t] = S.opp[s];
+        }
+        base_full += (int)sum_full;
+        base_fast += (int)sum_fast;
+    }
+    for (int t = n_full + tid; t < fast0; t += kCapLayoutThreads) {
+        Cs.root_me[t] = 0ull;
+        Cs.root_opp[t] = 0ull;
+    }
+    for (int t = fast0 + n_fast + tid; t < Cs.n_trees; t += kCapLayoutThreads) {
+        Cs.root_me[t] = 0ull;
+        Cs.root_opp[t] = 0ull;
+    }
+    const int n_pairs = (Cs.n_trees + kPairTrees - 1) / kPairTrees;
+    for (int q = tid; q < n_pairs; q += kCapLayoutThreads) Cs.pair_entrant[q] = q * kPairTrees < fast0 ? 0 : 1;
+    if (tid == 0) {
+        Cs.counters[0] += (unsigned long long)n_full;
+        Cs.counters[1] += (unsigned long long)n_fast;
+    }
+}
+
 int check_match(const bz_match_state *s) {
     if (!s) return BZ_ERR_ARG;
     if (!(s->board_size == 4 || s->board_size == 6 || s->board_size == 8)) return BZ_ERR_ARG;
@@ -778,6 +918,16 @@ int check_resign(const bz_selfplay_endgame_state *e, const bz_selfplay_resign_st
     if (!(r->threshold >= -1.0f && r->threshold <= 1.0f)) return BZ_ERR_ARG;  // NaN fails both
     if (r->audit_below > (1ull << 32)) return BZ_ERR_ARG;
     if (!r->hist_q || !r->rp_q || !r->counters || (e && !r->eg_hist_q)) return BZ_ERR_ARG;
+    return BZ_OK;
+}
+
+int check_cap(const bz_selfplay_state *s, const bz_selfplay_endgame_state *e, const bz_selfplay_cap_state *c) {
+    if (!c) return BZ_ERR_ARG;
+    if (c->full_below > (1ull << 32)) return BZ_ERR_ARG;
+    if (c->n_trees < s->n_games + kPairTrees - 1) return BZ_ERR_ARG;
+    if (!c->tree_of_slot || !c->root_me || !c->root_opp || !c->pair_entrant || !c->hist_full || !c->rp_full ||
+        !c->counters || (e && !c->eg_hist_full))
+        return BZ_ERR_ARG;
     return BZ_OK;
 }
 
@@ -869,14 +1019,16 @@ int64_t bz_selfplay_endgame_workspace_bytes(int64_t cap) {
            endgame_play_align16(cap * A);
 }
 
-// rs: NULL without resignation
+// rs: NULL without resignation; cs: NULL without randomized budgets
 static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
-                        const bz_selfplay_resign_state *rs, void *workspace, bool wld, bz_stream_t stream) {
+                        const bz_selfplay_resign_state *rs, void *workspace, bool wld, bz_stream_t stream,
+                        const bz_selfplay_cap_state *cs = nullptr) {
     int rc = check_state(st);
     if (rc != BZ_OK) return rc;
     rc = check_endgame(st, eg);
     if (rc != BZ_OK) return rc;
     if (rs && (rc = check_resign(eg, rs)) != BZ_OK) return rc;
+    if (cs && (rc = check_cap(st, eg, cs)) != BZ_OK) return rc;
     if (!workspace) return BZ_ERR_ARG;
     if (!aligned16(workspace)) return BZ_ERR_UNALIGNED;
     const int64_t cap = eg->cap;
@@ -891,7 +1043,15 @@ static int endgame_play(const bz_selfplay_state *st, const bz_selfplay_endgame_s
                                  s);
         if (rc != BZ_OK) return rc;
         const unsigned grid = (unsigned)((cap + kWarpsPerCta - 1) / kWarpsPerCta);
-        if (rs) {
+        if (cs) {
+            const bz_selfplay_resign_state none = {};
+            if (rs) {
+                endgame_ply_cap_kernel<true><<<grid, kThreads, 0, s>>>(*st, *eg, action, value, move_value, cells, *rs, *cs);
+            } else {
+                endgame_ply_cap_kernel<false><<<grid, kThreads, 0, s>>>(*st, *eg, action, value, move_value, cells, none,
+                                                                       *cs);
+            }
+        } else if (rs) {
             endgame_ply_kernel<true><<<grid, kThreads, 0, s>>>(*st, *eg, action, value, move_value, cells, *rs);
         } else {
             const bz_selfplay_resign_state none = {};
@@ -918,6 +1078,53 @@ int bz_selfplay_endgame_play_resign(const bz_selfplay_state *st, const bz_selfpl
                                     const bz_selfplay_resign_state *rs, void *workspace, int wld, bz_stream_t stream) {
     if (!rs) return BZ_ERR_ARG;
     return endgame_play(st, eg, rs, workspace, wld != 0, stream);
+}
+
+int bz_selfplay_endgame_play_cap(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                 const bz_selfplay_resign_state *rs, const bz_selfplay_cap_state *cs, void *workspace,
+                                 int wld, bz_stream_t stream) {
+    if (!cs) return BZ_ERR_ARG;
+    return endgame_play(st, eg, rs, workspace, wld != 0, stream, cs);
+}
+
+int bz_selfplay_cap_layout(const bz_selfplay_state *st, const bz_selfplay_cap_state *cs, bz_stream_t stream) {
+    int rc = check_state(st);
+    if (rc != BZ_OK) return rc;
+    rc = check_cap(st, nullptr, cs);
+    if (rc != BZ_OK) return rc;
+    selfplay_cap_layout_kernel<<<1, kCapLayoutThreads, 0, as_stream(stream)>>>(*st, *cs);
+    return launch_rc();
+}
+
+int bz_selfplay_advance_cap(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                            const bz_selfplay_resign_state *rs, const bz_selfplay_cap_state *cs,
+                            const bz_tree_pools *pools, uint8_t *action_out, bz_stream_t stream) {
+    int rc = check_state(st);
+    if (rc != BZ_OK) return rc;
+    if (eg && (rc = check_endgame(st, eg)) != BZ_OK) return rc;
+    if (rs && (rc = check_resign(eg, rs)) != BZ_OK) return rc;
+    rc = check_cap(st, eg, cs);
+    if (rc != BZ_OK) return rc;
+    if (!pools || pools->game != BZ_GAME_REVERSI || pools->n_trees != cs->n_trees || pools->board_size != st->board_size ||
+        !pools->root_meta || !pools->arena)
+        return BZ_ERR_ARG;
+    if (st->n_games == 0) return BZ_OK;
+    const unsigned grid = (st->n_games + kWarpsPerCta - 1) / kWarpsPerCta;
+    const uint64_t cells = cell_mask(st->board_size);
+    const bz_selfplay_endgame_state no_eg = {};
+    const bz_selfplay_resign_state no_rs = {};
+    const cudaStream_t s = as_stream(stream);
+    if (eg && rs) {
+        selfplay_advance_cap_kernel<true, true><<<grid, kThreads, 0, s>>>(*st, *pools, action_out, cells, *eg, *rs, *cs);
+    } else if (eg) {
+        selfplay_advance_cap_kernel<true, false><<<grid, kThreads, 0, s>>>(*st, *pools, action_out, cells, *eg, no_rs, *cs);
+    } else if (rs) {
+        selfplay_advance_cap_kernel<false, true><<<grid, kThreads, 0, s>>>(*st, *pools, action_out, cells, no_eg, *rs, *cs);
+    } else {
+        selfplay_advance_cap_kernel<false, false><<<grid, kThreads, 0, s>>>(*st, *pools, action_out, cells, no_eg, no_rs,
+                                                                           *cs);
+    }
+    return launch_rc();
 }
 
 int bz_match_init(const bz_match_state *st, bz_stream_t stream) {

@@ -24,7 +24,11 @@ entries name the solver.  With ``--resign V`` a self-play game that is not audit
 q (W / N of the most visited root edge) is below V (-1: audit only); ``--resign-audit F`` games never resign and measure
 the false positives, and ``--resign-fp P`` sets the next iteration's threshold from this iteration's gathered audited
 games (``resign.calibrate``: the same on every rank, since every rank gathers the same replay).  The line then has a
-``resign`` entry, and the checkpoint's ``extra`` holds the next threshold, which ``--resume`` restores.
+``resign`` entry, and the checkpoint's ``extra`` holds the next threshold, which ``--resume`` restores.  With
+``--fast-sims N`` a fraction ``--full-fraction P`` of the self-play plies (a Philox draw per ply) is searched with
+``--sims`` and every other ply with N simulations (randomized search budgets); training batches are drawn from the full
+plies' records only, after the resignation calibration, which uses every record.  The line then has a ``cap`` entry,
+and the checkpoint's ``extra`` holds both settings.
 """
 from __future__ import annotations
 
@@ -47,7 +51,8 @@ def default_args(**over) -> SimpleNamespace:
     a = SimpleNamespace(games=4096, sims=800, leaves=4, plies=70, size=8, iterations=1, train_steps=8, batch=4096, lr=1e-4,
                         temp_plies=8, net="mlp", hidden=256, seed=0, train_on_rank0=False, checkpoint=None, resume=None,
                         reuse=False, eval_games=0, eval_minimax=None, eval_endgame=None, endgame_empties=0, endgame_every=8,
-                        endgame_solve="exact", resign=None, resign_audit=0.1, resign_fp=None)
+                        endgame_solve="exact", resign=None, resign_audit=0.1, resign_fp=None, fast_sims=None,
+                        full_fraction=0.25)
     for k, v in over.items():
         if not hasattr(a, k):
             raise TypeError(f"unknown loop argument {k!r}")
@@ -108,7 +113,9 @@ class LoopState:
                                            graph_unroll=min(16, max(1, args.sims // args.leaves - 1)),
                                            endgame_empties=int(getattr(args, "endgame_empties", 0)),
                                            endgame_every=int(getattr(args, "endgame_every", 8)), endgame_solve=solve,
-                                           resign_threshold=threshold, resign_audit=float(getattr(args, "resign_audit", 0.1)))
+                                           resign_threshold=threshold, resign_audit=float(getattr(args, "resign_audit", 0.1)),
+                                           fast_sims=getattr(args, "fast_sims", None),
+                                           full_fraction=float(getattr(args, "full_fraction", 0.25)))
         self.sp.prepare()
 
     @torch.no_grad()
@@ -133,6 +140,7 @@ def run_iteration(st: LoopState, it: int) -> dict:
     torch.cuda.synchronize()
     eg_ms0, eg_stats0 = (sp.endgame_ms(), sp.stats()) if sp.eg is not None else (0.0, None)
     rs_stats0, rs_threshold = (sp.stats(), sp.resign_threshold) if sp.rs is not None else (None, None)
+    cap_stats0 = sp.stats() if sp.cs is not None else None
     t0 = time.perf_counter()
     ev[0].record()
     for _ in range(args.plies):
@@ -157,13 +165,19 @@ def run_iteration(st: LoopState, it: int) -> dict:
         resign_line = {"threshold": rs_threshold, "next_threshold": sp.resign_threshold, "audit": sp.resign_audit,
                        "fp_target": fp_target, "fp": resign.false_positive_rate(recs, rs_threshold),
                        "audited_games": resign.audited_games(recs), "plies_per_game": n / n_games if n_games else None}
+    # randomized budgets: the policy targets of fast plies come from cheap searches, so the batches are drawn from the
+    # full records only (after the calibration above, which uses every record)
+    train_rows = torch.nonzero(replay["full"]).squeeze(1) if sp.cs is not None and n else None
+    n_train = int(train_rows.numel()) if train_rows is not None else n
     # --eval-games: the net that played this iteration's self-play, to be matched against the trained one
     snapshot = copy.deepcopy(st.model) if getattr(args, "eval_games", 0) and rank == 0 else None
     losses = []
-    if n and (not args.train_on_rank0 or rank == 0):
+    if n_train and (not args.train_on_rank0 or rank == 0):
         g = torch.Generator(device="cuda").manual_seed(args.seed * 1000 + it)
         for k in range(args.train_steps):
-            idx = torch.randint(0, n, (min(args.batch, n),), device="cuda", generator=g)
+            idx = torch.randint(0, n_train, (min(args.batch, n_train),), device="cuda", generator=g)
+            if train_rows is not None:
+                idx = train_rows[idx]
             planes, pi, z = train.make_batch(replay, idx, size=args.size, augment_seed=args.seed + 31 * it + k)
             losses.append(train.train_step(st.master, st.opt, planes, pi, z)["loss"])
         st._publish()
@@ -183,7 +197,7 @@ def run_iteration(st: LoopState, it: int) -> dict:
         "sims_per_sec_per_gpu": args.games * args.sims * args.plies / (ms["selfplay"] * 1e-3),
         "replay_records_gathered": int(n), "local_records": int(shard["me"].shape[0]),
         "games_finished_local": stats["games"], "records_dropped_local": stats["dropped"],
-        "train_steps": len(losses), "train_batch": min(args.batch, int(n)) if n else 0,
+        "train_steps": len(losses), "train_batch": min(args.batch, n_train) if n_train else 0,
         "loss_first_last": [losses[0], losses[-1]] if losses else None,
         "broadcast_bytes": nbytes, "replay_gather": gather_info,
     }
@@ -205,6 +219,11 @@ def run_iteration(st: LoopState, it: int) -> dict:
         resign_line["resigned_local"] = stats["resigned"] - rs_stats0["resigned"]
         resign_line["audited_local"] = stats["audited"] - rs_stats0["audited"]
         line["resign"] = resign_line
+    if sp.cs is not None:
+        line["cap"] = {"full_fraction": sp.full_fraction, "fast_sims": sp.fast_sims,
+                       "full_plies_local": stats["full_plies"] - cap_stats0["full_plies"],
+                       "fast_plies_local": stats["fast_plies"] - cap_stats0["fast_plies"],
+                       "records_trained_on": n_train, "games_finished_local": stats["games"] - cap_stats0["games"]}
     if snapshot is not None:
         t_eval = time.perf_counter()
         r = match.BatchedMatch(st.model, snapshot, args.eval_games, args.sims, n_leaves=args.leaves, board_size=args.size,
@@ -232,6 +251,8 @@ def run_iteration(st: LoopState, it: int) -> dict:
         extra = {"games_per_gpu": args.games, "sims_per_move": args.sims, "world": world}
         if sp.rs is not None:
             extra["resign_threshold"] = sp.resign_threshold
+        if sp.cs is not None:
+            extra["fast_sims"], extra["full_fraction"] = sp.fast_sims, sp.full_fraction
         train.save_checkpoint(path, st.master, st.opt, iteration=it + 1, extra=extra)
         line["checkpoint"] = path
     return line
@@ -296,6 +317,11 @@ def main():
     ap.add_argument("--resign-fp", type=float, default=d.resign_fp, metavar="P",
                     help="set the threshold after every iteration from its audited games: the largest one whose "
                          "false-positive rate stays at most P (switches resignation on, from --resign or -1)")
+    ap.add_argument("--fast-sims", type=int, default=d.fast_sims, metavar="N",
+                    help="randomized search budgets: plies that are not full are searched with N simulations (a "
+                         "multiple of --leaves, 2 * leaves .. --sims; default off); only full plies are trained on")
+    ap.add_argument("--full-fraction", type=float, default=d.full_fraction, metavar="P",
+                    help="with --fast-sims: the fraction of plies searched with --sims (a Philox draw per ply)")
     ap.add_argument("--checkpoint", default=None, help="write a state_dict checkpoint (master weights + Adam state) here "
                                                        "after every iteration (rank 0); SL/train.py:204-214.  A {iteration} "
                                                        "in the path is replaced by the iteration number, so every "

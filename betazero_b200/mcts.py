@@ -407,15 +407,22 @@ class BatchedMCTS:
         self.evaluate()
         self.expand_backup()
 
-    def add_root_noise(self) -> None:
+    def add_root_noise(self, pair_entrant: torch.Tensor | None = None, entrant: int = 0) -> None:
         """P_root <- (1 - eps) P + eps Dirichlet(alpha) over the root's legal moves (bz_mcts_root_noise).
-        Gamma(alpha, 1) samples come from torch (plumbing); the kernel normalises over the legal edges."""
+        Gamma(alpha, 1) samples come from torch (plumbing); the kernel normalises over the legal edges.  With
+        ``pair_entrant`` (uint8 per CTA pair of 56 trees) only the trees of the pairs of ``entrant`` get the noise
+        (bz_mcts_root_noise_entrant)."""
         p = self.pools
         shape = (max(p.n_trees, 1), p.n_actions)
         alpha = torch.full(shape, self.dirichlet_alpha, dtype=torch.float32, device=p.device)
         noise = torch._standard_gamma(alpha, generator=self._noise_gen).clamp_min_(1e-30)
-        _lib.check(self._L.bz_mcts_root_noise(p._ref, _lib.dptr(noise), self.dirichlet_eps, _lib.stream_ptr()),
-                   "bz_mcts_root_noise")
+        if pair_entrant is None:
+            _lib.check(self._L.bz_mcts_root_noise(p._ref, _lib.dptr(noise), self.dirichlet_eps, _lib.stream_ptr()),
+                       "bz_mcts_root_noise")
+        else:
+            _lib.check(self._L.bz_mcts_root_noise_entrant(p._ref, _lib.dptr(noise), self.dirichlet_eps,
+                                                          _lib.dptr(pair_entrant), int(entrant), _lib.stream_ptr()),
+                       "bz_mcts_root_noise_entrant")
         self.launches += 1
 
     def prepare(self) -> None:

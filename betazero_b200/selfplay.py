@@ -22,21 +22,61 @@ restarts (bz_selfplay_advance_resign).  A fraction ``resign_audit`` of the games
 resigns: they measure how often resigning would have been wrong (``resign.false_positive_rate``, ``resign.calibrate``).
 Every record then carries its ply's q (NaN for solver-played plies) and ``drain_replay`` returns it as "q".  The
 threshold can change between plies (``set_resign_threshold``): the state is passed by value at every launch.
+
+Randomized search budgets (opt-in, ``fast_sims=n``; KataGo's playout cap randomization): a ply of game g at ply t is full
+iff a Philox draw on (seed, g, 0x80000000 | t) falls below ``full_fraction``; a full ply is searched with ``n_sims``, any
+other ply with ``fast_sims``, both from a fresh tree.  Every record carries ``full`` (solver-played records are full) and
+``drain_replay`` returns it as "full": the policy target of a fast ply comes from a cheap search and is not trained on,
+its z is the game's.  Each ply runs bz_selfplay_cap_layout (the full slots' trees first, padded to a CTA pair, then the
+fast ones), bz_mcts_reset from its roots, bz_mcts_search_fused_entrants with the two budgets, and
+bz_selfplay_advance_cap; launches made of fast pairs only end early.  Root noise, when on, perturbs full plies only.
+It needs the one-launch search and refuses tree reuse.
 """
 from __future__ import annotations
 
 import ctypes as C
 
+import math
+
 import torch
 
 from . import _lib
 from . import resign as _resign
-from ._lib import BzSelfplayEndgameState, BzSelfplayResignState, BzSelfplayState
-from .mcts import BatchedMCTS, TreePools
+from ._lib import BzSelfplayCapState, BzSelfplayEndgameState, BzSelfplayResignState, BzSelfplayState
+from .mcts import BatchedMCTS, FusedNetEvaluator, TreePools
 
 N_ACTIONS = 65
 SOLVE_MAX_EMPTIES = 20  # BZ_SOLVE_MAX_EMPTIES
 ENDGAME_SOLVES = ("exact", "wld")
+PAIR_TREES = 56  # BZ_MATCH_TREES_PER_PAIR: the trees of a CTA pair of the one-launch search
+FULL_COUNTER = 0x80000000  # the Philox counter of the full-ply draw is 0x80000000 | ply
+
+
+def full_below(fraction) -> int:
+    """floor(fraction * 2^32) for a full fraction in [0, 1]"""
+    f = float(fraction)
+    if not 0.0 <= f <= 1.0:
+        raise ValueError(f"full_fraction must be in [0, 1]; got {fraction}")
+    return int(math.floor(f * 2.0 ** 32))
+
+
+def check_fast_sims(fast_sims, n_sims: int, n_leaves: int) -> int:
+    """2 K <= fast_sims <= n_sims, a multiple of K = n_leaves"""
+    f, k = int(fast_sims), int(n_leaves)
+    if not 2 * k <= f <= int(n_sims) or f % k:
+        raise ValueError(f"fast_sims must be a multiple of n_leaves = {k} in {2 * k} .. n_sims = {n_sims}; got {fast_sims}")
+    return f
+
+
+def is_full(game_id: torch.Tensor, ply: torch.Tensor, seed: int, fraction: float) -> torch.Tensor:
+    """bool tensor: the searches of these (game id, ply) plies are full (bz_philox_u32 on the device)"""
+    L = _lib.load()
+    g = game_id.to(device="cuda", dtype=torch.int64).contiguous()
+    t = (ply.to(device="cuda", dtype=torch.int64) - FULL_COUNTER).to(torch.int32).contiguous()  # int32 bits of 0x80000000 | ply
+    out = torch.empty(g.numel(), dtype=torch.int32, device="cuda")
+    _lib.check(L.bz_philox_u32(int(seed), _lib.dptr(g), _lib.dptr(t), _lib.dptr(out), g.numel(), _lib.stream_ptr()),
+               "bz_philox_u32")
+    return (out.to(torch.int64) & 0xFFFFFFFF) < full_below(fraction)
 
 
 def check_endgame_empties(empties, board_size: int) -> int:
@@ -61,8 +101,21 @@ class BatchedSelfPlay:
                  dirichlet_alpha: float = 0.0, dirichlet_eps: float = 0.25, n_leaves: int = 1, device="cuda",
                  one_launch: bool | None = None, reuse: bool = False, endgame_empties: int = 0, endgame_every: int = 8,
                  endgame_cap: int | None = None, endgame_solve: str = "exact", resign_threshold: float | None = None,
-                 resign_audit: float = 0.1):
+                 resign_audit: float = 0.1, fast_sims: int | None = None, full_fraction: float = 0.25):
         self.n_games, self.n_sims, self.board_size = int(n_games), int(n_sims), int(board_size)
+        # randomized search budgets: checked before anything touches the GPU
+        self.fast_sims, self.full_fraction = None, float(full_fraction)
+        if fast_sims is not None:
+            self._full_below = full_below(full_fraction)
+            self.fast_sims = check_fast_sims(fast_sims, n_sims, n_leaves)
+            if n_sims % int(n_leaves):
+                raise ValueError(f"n_sims {n_sims} is not a multiple of n_leaves {n_leaves}")
+            if reuse:
+                raise ValueError("fast_sims does not combine with tree reuse: the layout gives a slot another tree from "
+                                 "ply to ply, so there is no subtree to keep")
+            if one_launch is False or int(n_leaves) not in (1, 2, 4) or not isinstance(evaluator, FusedNetEvaluator):
+                raise ValueError("fast_sims needs the one-launch search (bz_mcts_search_fused_entrants): n_leaves 1, 2 "
+                                 "or 4 and a FusedNetEvaluator on the bf16 MLP")
         self.resign_audit = float(resign_audit)
         self._audit_below = _resign.audit_below(resign_audit)
         if resign_threshold is not None:
@@ -81,11 +134,16 @@ class BatchedSelfPlay:
         # simulations per move on top of the kept ones; the default is a fresh tree per move, which the goldens pin
         self.reuse = bool(reuse)
         self._moves = 0
-        self.pools = TreePools(n_games, n_sims, board_size=board_size, c_puct=c_puct, arena_units=arena_units,
+        # randomized budgets: n_games + 55 trees, so the full range's padding to a CTA pair always fits
+        n_trees = n_games + PAIR_TREES - 1 if self.fast_sims is not None else n_games
+        self.pools = TreePools(n_trees, n_sims, board_size=board_size, c_puct=c_puct, arena_units=arena_units,
                                n_leaves=n_leaves, device=device, reuse=reuse)
         self.mcts = BatchedMCTS(self.pools, evaluator, use_graph=use_graph, graph_unroll=graph_unroll,
                                 dirichlet_alpha=dirichlet_alpha, dirichlet_eps=dirichlet_eps,
                                 noise_seed=seed * 7919 + rank, one_launch=one_launch)
+        if self.fast_sims is not None and not self.mcts.one_launch_ok():
+            raise ValueError("fast_sims needs the one-launch search (bz_mcts_search_fused_entrants): the evaluator's net "
+                             "must run through the bf16 MLP kernel path")
         self.max_plies = 128
         B, H = max(self.n_games, 1), max(self.n_games, 1) * self.max_plies
         self.replay_cap = int(replay_cap if replay_cap is not None else B * 2 * self.max_plies)
@@ -126,6 +184,9 @@ class BatchedSelfPlay:
         self.rs = None
         if resign_threshold is not None:
             self._init_resign(resign_threshold)
+        self.cs = None
+        if self.fast_sims is not None:
+            self._init_cap()
 
     def _init_endgame(self) -> None:
         Q, dev = self.endgame_cap, self.device
@@ -164,6 +225,50 @@ class BatchedSelfPlay:
         self.rs = r
         self._rs_ref = C.byref(r)
 
+    def _init_cap(self) -> None:
+        dev, T = self.device, self.pools.n_trees
+
+        def e(n, dt):
+            return torch.empty(max(n, 1), dtype=dt, device=dev)
+
+        self.tree_of_slot = e(self.n_games, torch.int32)
+        self.cap_root_me, self.cap_root_opp = e(T, torch.int64), e(T, torch.int64)
+        self.pair_entrant = e(-(-T // PAIR_TREES), torch.uint8)
+        self.hist_full = e(self.n_games * self.max_plies, torch.uint8)
+        self.eg_hist_full = e(self.endgame_cap * self.max_plies, torch.uint8) if self.eg is not None else None
+        self.rp_full = e(self.replay_cap, torch.uint8)
+        self.cap_counters = torch.zeros(2, dtype=torch.int64, device=dev)
+        c = BzSelfplayCapState()
+        c.full_below, c.n_trees = self._full_below, T
+        for name in ("tree_of_slot", "pair_entrant", "hist_full", "eg_hist_full", "rp_full"):
+            t = getattr(self, name)
+            setattr(c, name, t.data_ptr() if t is not None else None)
+        c.root_me, c.root_opp, c.counters = (self.cap_root_me.data_ptr(), self.cap_root_opp.data_ptr(),
+                                             self.cap_counters.data_ptr())
+        self.cs = c
+        self._cs_ref = C.byref(c)
+
+    def _search_cap(self) -> None:
+        """layout -> reset from the layout's roots -> the two budgets in one bz_mcts_search_fused_entrants; with root
+        noise the first iteration runs through the per-iteration kernels and the noise goes to the full pairs only"""
+        m, st = self.mcts, _lib.stream_ptr()
+        _lib.check(self._L.bz_selfplay_cap_layout(self._ref, self._cs_ref, st), "bz_selfplay_cap_layout")
+        self.launches += 1
+        m.reset(self.cap_root_me, self.cap_root_opp)
+        K = self.pools.n_leaves
+        iters = [self.n_sims // K, self.fast_sims // K]
+        if m.dirichlet_alpha > 0:
+            m.select()
+            m.evaluate()
+            m.expand_backup()
+            m.add_root_noise(self.pair_entrant, 0)
+            iters = [n - 1 for n in iters]
+        img = m.evaluator.net._image_pair.data_ptr()  # read at every ply: refresh() may rebuild the image
+        _lib.check(self._L.bz_mcts_search_fused_entrants(self.pools._ref, (C.c_void_p * 2)(img, img),
+                                                         (C.c_int32 * 2)(*iters), 2, _lib.dptr(self.pair_entrant), st),
+                   "bz_mcts_search_fused_entrants")
+        m.launches += -(-self.pools.n_trees // m.ONE_LAUNCH_MAX_TREES)  # one launch per chunk of <= 4144 trees
+
     @property
     def resign_threshold(self) -> float | None:
         """the threshold of the next plies (float32), None when resignation is off"""
@@ -177,6 +282,10 @@ class BatchedSelfPlay:
 
     # -- one lockstep ply for every game ----------------------------------------------------------
     def search(self) -> None:
+        if self.cs is not None:
+            self._search_cap()
+            self._moves += 1
+            return
         if (self.mcts.use_graph and self.mcts._graph is None and not self.mcts.one_launch
                 and self.n_sims // self.pools.n_leaves - 1 >= self.mcts.unroll):
             self.mcts.prepare()  # lazily, before the roots are set: play_move() works without an explicit prepare()
@@ -188,6 +297,17 @@ class BatchedSelfPlay:
         self._moves += 1
 
     def advance(self) -> None:
+        if self.cs is not None:
+            _lib.check(self._L.bz_selfplay_advance_cap(self._ref, self._eg_ref if self.eg is not None else None,
+                                                       self._rs_ref if self.rs is not None else None, self._cs_ref,
+                                                       self.pools._ref, _lib.dptr(self.last_action), _lib.stream_ptr()),
+                       "bz_selfplay_advance_cap")
+            self.launches += 1
+            if self.eg is not None:
+                self._advances += 1
+                if self._advances % self.endgame_every == 0:
+                    self.endgame_play()
+            return
         if self.rs is not None:
             _lib.check(self._L.bz_selfplay_advance_resign(self._ref, self._eg_ref if self.eg is not None else None,
                                                           self._rs_ref, self.pools._ref, _lib.dptr(self.last_action),
@@ -218,7 +338,12 @@ class BatchedSelfPlay:
             raise RuntimeError("endgame_play needs endgame_empties > 0")
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
-        if self.rs is not None:
+        if self.cs is not None:
+            name = "bz_selfplay_endgame_play_cap"
+            _lib.check(self._L.bz_selfplay_endgame_play_cap(self._ref, self._eg_ref, self._rs_ref if self.rs is not None
+                                                            else None, self._cs_ref, _lib.dptr(self.eg_workspace),
+                                                            int(self.endgame_solve == "wld"), _lib.stream_ptr()), name)
+        elif self.rs is not None:
             name = "bz_selfplay_endgame_play_resign"
             _lib.check(self._L.bz_selfplay_endgame_play_resign(self._ref, self._eg_ref, self._rs_ref,
                                                                _lib.dptr(self.eg_workspace), int(self.endgame_solve == "wld"),
@@ -243,8 +368,9 @@ class BatchedSelfPlay:
         self.advance()
 
     def prepare(self) -> None:
-        """capture the CUDA graph (before the first search)"""
-        self.mcts.prepare()
+        """capture the CUDA graph (before the first search); randomized budgets run the one-launch search, no graph"""
+        if self.cs is None:
+            self.mcts.prepare()
 
     # -- results ---------------------------------------------------------------------------------
     def stats(self) -> dict:
@@ -259,6 +385,9 @@ class BatchedSelfPlay:
         # resignation: games resigned, audited games finished (both 0 when it is off)
         rc = self.resign_counters.cpu().tolist() if self.rs is not None else [0, 0]
         out.update({"resigned": rc[0], "audited": rc[1]})
+        # randomized budgets: searched plies with the full budget and with the fast one (both 0 when it is off)
+        cc = self.cap_counters.cpu().tolist() if self.cs is not None else [0, 0]
+        out.update({"full_plies": cc[0], "fast_plies": cc[1]})
         return out
 
     def drain_replay(self) -> dict:
@@ -279,6 +408,8 @@ class BatchedSelfPlay:
         }
         if self.rs is not None:
             out["q"] = self.rp_q[:n].clone()  # q of the record's ply (NaN for solver-played plies)
+        if self.cs is not None:
+            out["full"] = self.rp_full[:n].clone()  # 1: a full search's (or the solver's) pi; 0: a fast search's
         self.counters[0] = 0
         return out
 

@@ -432,6 +432,56 @@ int bz_selfplay_advance_resign(const bz_selfplay_state *st, const bz_selfplay_en
 int bz_selfplay_endgame_play_resign(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
                                     const bz_selfplay_resign_state *rs, void *workspace, int wld, bz_stream_t stream);
 
+/* Randomized search budgets (opt-in; KataGo's playout cap randomization): a searched ply of game g at ply t (the slot's
+ * ply, the t that keys move sampling) is FULL iff bz_philox_u32(seed, g, 0x80000000 | t) < full_below, full_below =
+ * floor(p * 2^32) in 0 .. 2^32 (the counter is never a ply and never the audit draw's 0xFFFFFFFF).  A full ply is
+ * searched with the full budget, any other ply with the fast one; both start from a fresh tree.  Every record carries
+ * full (uint8, 1 = full) in rp_full; solver-played records are full.  Resignation and the endgame handover apply to
+ * every searched ply as without the option.
+ * Every ply: bz_selfplay_cap_layout gives each slot a tree -- the full slots first, in slot order, padded with empty
+ * boards to the next multiple of 56 trees (a CTA pair of the one-launch search), then the fast slots in slot order, then
+ * empty boards to n_trees -- and writes the roots for bz_mcts_reset and pair_entrant (0: a pair of full trees, 1: fast
+ * or trailing pairs) for bz_mcts_search_fused_entrants with the two entries {full budget, fast budget}.  Launches made
+ * of fast pairs only then end early.  Slots never go idle, so the layout needs no host read between plies.
+ * bz_selfplay_advance_cap reads slot s's search from tree tree_of_slot[s].  Oracle: oracle/selfplay_cap_ref.py. */
+typedef struct bz_selfplay_cap_state {
+    uint64_t full_below;   /* 0 .. 2^32: floor(p * 2^32) */
+    int32_t n_trees;       /* trees of the pools: >= n_games + 55 */
+    int32_t reserved;
+    int32_t *tree_of_slot; /* [n_games]: the tree that searches slot s this ply */
+    uint64_t *root_me;     /* [n_trees]: roots in tree order (mover-relative; 0, 0 on padding trees) */
+    uint64_t *root_opp;
+    uint8_t *pair_entrant; /* [ceil(n_trees / 56)]: 0 full, 1 fast */
+    uint8_t *hist_full;    /* [n_games * max_plies]: the flag of the slot's history rows */
+    uint8_t *eg_hist_full; /* [eg->cap * max_plies]: the flag of the endgame queue's history blocks; NULL without a handover */
+    uint8_t *rp_full;      /* [replay_cap]: the flag of the replay records */
+    /* device uint64 [2]: 0 full plies laid out, 1 fast plies laid out */
+    unsigned long long *counters;
+} bz_selfplay_cap_state;
+
+/* The tree layout of this ply (one CTA), as above; adds this ply's full and fast slots to counters 0 and 1 (the caller
+ * zeroes them once).  BZ_ERR_ARG: a bad self-play state, a NULL cs or array in it, full_below > 2^32,
+ * n_trees < n_games + 55. */
+int bz_selfplay_cap_layout(const bz_selfplay_state *st, const bz_selfplay_cap_state *cs, bz_stream_t stream);
+/* bz_selfplay_advance (eg and rs NULL), bz_selfplay_advance_endgame (eg given) or bz_selfplay_advance_resign (rs given)
+ * with slot s read from tree tree_of_slot[s] of pools (pools->n_trees == cs->n_trees) and the ply's flag recorded.
+ * BZ_ERR_ARG: what those refuse, what bz_selfplay_cap_layout refuses, a NULL eg_hist_full when eg is given. */
+int bz_selfplay_advance_cap(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                            const bz_selfplay_resign_state *rs, const bz_selfplay_cap_state *cs,
+                            const bz_tree_pools *pools, uint8_t *action_out, bz_stream_t stream);
+/* bz_selfplay_endgame_play (wld = 0) or _wld (wld != 0), with the q rows when rs is given, and the flag rows carried
+ * through: a solver ply's flag is 1.  Same refusals as bz_selfplay_advance_cap with eg given, and those of the solver
+ * phase. */
+int bz_selfplay_endgame_play_cap(const bz_selfplay_state *st, const bz_selfplay_endgame_state *eg,
+                                 const bz_selfplay_resign_state *rs, const bz_selfplay_cap_state *cs, void *workspace,
+                                 int wld, bz_stream_t stream);
+
+/* Root noise on the trees of the CTA pairs whose pair_entrant is `entrant` (bz_mcts_root_noise otherwise): the trees of
+ * other pairs are left as they are.  pair_entrant: device uint8 [ceil(n_trees / 56)].  BZ_ERR_ARG: what
+ * bz_mcts_root_noise refuses, a NULL pair_entrant. */
+int bz_mcts_root_noise_entrant(const bz_tree_pools *pools, const float *noise, float eps, const uint8_t *pair_entrant,
+                               int entrant, bz_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * Batched round-robin tournaments: every pairing of up to BZ_MAX_ENTRANTS entrants (a net and a search budget each) in
  * the same launches; a net-versus-net match is the tournament of two entrants and the one pairing (0, 1).  Game pair i
